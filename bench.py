@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- scattering-order updates/s of the SOS_AER hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--scenarios S] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--scenarios S] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[4], the critical-albedo style batch sweep): S independent
@@ -382,6 +382,26 @@ def emit(obj):
         os.write(_REAL_STDOUT, data)
 
 
+DUMP_SAMPLE = 1 << 20   # elements of the radiance field --dump-outputs writes: 2 x 8 MB (values and their indices)
+
+
+def dump_outputs(dirname, res, S, L, N, torch):
+    """--dump-outputs: what a caller of BatchSolver.solve received from the last timed step, as float64 DIR/<name>.npy, so
+    that two builds can be compared output for output.  The (S, L, N) radiance field (615 MB at the default size) is
+    written as a fixed sample: I_sample at the flat (S, L, N) indices I_sample_index, drawn by a seeded generator.  The
+    per-scenario arrays (orders to convergence, last TOA / surface convergence ratios, status bits, still-active flags) are
+    written whole."""
+    os.makedirs(dirname, exist_ok=True)
+    flat = np.sort(np.random.default_rng(0).choice(S * L * N, size=min(DUMP_SAMPLE, S * L * N), replace=False))
+    ld = res.I.shape[-1]                                     # the device field pads every row of N values to ld
+    padded = torch.from_numpy((flat // N) * ld + flat % N).to(res.I.device)
+    out = {"I_sample": res.I.reshape(-1)[padded].cpu().numpy(), "I_sample_index": flat}
+    for name in ("n_orders", "ratio_toa", "ratio_surf", "status", "active"):
+        out[name] = getattr(res, name)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     # stdout carries exactly one JSON line: anything a library prints on fd 1 (NCCL prints its version there when
     # NCCL_DEBUG is set) goes to stderr instead
@@ -404,7 +424,13 @@ def main():
     ap.add_argument("--thick-chunk-rows", type=int, default=0, help="N > 1, layer blocks: rows per scan chunk of the sharded plan (0: the library's choice, as on one GPU)")
     ap.add_argument("--no-secondary", dest="secondary", action="store_false", help="N > 1: skip the mu-sharded thick-cloud record")
     ap.add_argument("--full-sweep", type=int, default=9984, help="solves of the full configs[4] sweep reported as full_sweep (0: skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="sweep workload: write what the last timed step returned as "
+                    "DIR/<name>.npy (rank 0; a fixed sample of the radiance field, see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "sweep"):
+        ap.error("--dump-outputs covers the sweep workload of --impl ours")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -478,13 +504,15 @@ def main():
     for k in range(args.steps):
         flush.zero_()                                  # L2 flush between timed iterations (untimed)
         ev[2 * k].record()
-        step_resident()
+        res = step_resident()
         ev[2 * k + 1].record()
     barrier()
     t_end = time.perf_counter()
     t_wall = t_end - t_wall
     clocks = sampler.stop(t_begin, t_end)
     launches = eng.launches - l0
+    if args.dump_outputs and rank == 0:               # before the next solve overwrites the field
+        dump_outputs(args.dump_outputs, res, S, L, N, torch)
     # per-kernel times: the SAME K steps once more with CUDA-event spans around every kernel class (on the launching
     # stream).  The spans cost a few percent and switch the order loop from graph replays to single launches, so the
     # headline pass above runs without them; step_ms_spans reports what this pass took.
