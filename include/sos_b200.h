@@ -86,7 +86,11 @@ typedef struct {
   int phase_aer;
   int extrap_width[3];  /* idx of improved_limit_mu_down per region (:342-345,361-364,380-383;
                            single layer SOS_Aer_I1_In.py:124-127) */
-  int reserved;
+  int order_cap;        /* 0: the reference's stopping rule (ratio of :309 against threshold).  > 0: the scenario sums
+                           exactly the orders 1 .. order_cap (active while its order is below the cap; the ratio is not
+                           consulted and a 0/0 ratio is not SOS_STATUS_NONFINITE, a non-finite I_n still is).  What an
+                           azimuthal Fourier mode m >= 1 uses: it sums the orders its mode 0 summed, and its ratio is
+                           meaningless (I_m changes sign; the mu = +-1 columns are exactly 0). */
 } sos_scenario;
 
 /* Per-scenario results of sos_solve / sos_converge (host copy). */
@@ -135,6 +139,28 @@ int sos_build_contraction(sos_plan* plan, const double* P_d, int ldp, double* A_
 int sos_build_phase(sos_plan* plan, int family, double g, double mu0, const double* phi_h, const double* cphi_h,
                     const double* tab_x_d, const double* tab_y_d, int tab_n, double* P_d, int ldp, double* P0_d,
                     void* stream);
+
+/* Azimuthal Fourier modes m = 0 .. n_modes-1 of the same phase functions (family and table arguments as in
+ * sos_build_phase).  Azimuth nodes: phi_h [n_phi] ascending on [0, pi] (2 <= n_phi <= 1024); cphi_h [1 + n_modes][n_phi]:
+ * row 0 = cos(0 - phi_k) (the node cosines, as sos_build_phase takes them), row 1 + m = cos(m phi_k), both computed by
+ * the host.  The phase function is evaluated once per (element, node); with A = f(-(cc - x_k)), B = f(-(cc + x_k)),
+ * x_k = ss cos(phi_k), mode m integrates trapz_k(cos(m phi_k) (A + (-1)^m B)).  Every mode is normalised by the column
+ * integrals of MODE 0: P_m[:, n] = 4 R_m[:, n] / trapz(R_0[:, n], mu), P0_m = 2 P0raw_m / trapz(P0raw_0, mu), so that
+ * sum_m (2 - delta_m0) P0_m cos(m phi) = c p(cos Theta) with one constant c.  With the 25 nodes of sos_build_phase,
+ * mode 0 is bit for bit what sos_build_phase writes.  P_d: mode m at P_d + m*mode_stride ([N][ldp] each, mode_stride >=
+ * N*ldp); P0_d: [n_modes][N]; either may be NULL.  1 <= n_modes <= 64. */
+int sos_build_phase_modes(sos_plan* plan, int family, double g, double mu0, int n_phi, const double* phi_h, const double* cphi_h,
+                          int n_modes, const double* tab_x_d, const double* tab_y_d, int tab_n, double* P_d, int ldp,
+                          size_t mode_stride, double* P0_d, void* stream);
+
+/* Azimuth synthesis of Fourier-mode fields: out[geo][r][p][col] (+)= sum over s with geo_h[s] = geo of
+ * w_h[s][p] * I[s][rows_h[r]][col] (col < N), the sum in ascending s (no atomics: deterministic).  I_d: a field of this plan
+ * ([S*L][ld]); geo_h [S] in [0, n_geo) or -1 (member skipped); w_h [S][n_az] (1 for mode 0, 2 cos(m phi_p) for mode m, as
+ * the host computed them); rows_h [n_rows] in [0, L); out_d [n_geo][n_rows][n_az][N].  accumulate = 0 overwrites, 1 adds
+ * (the mode sub-batches of one geometry solved on several plans add into one output).  Only geometries with at least one
+ * member are written. */
+int sos_azimuth_synthesis(sos_plan* plan, const double* I_d, const int* geo_h, const double* w_h, int n_geo, const int* rows_h,
+                          int n_rows, int n_az, double* out_d, int accumulate, void* stream);
 
 /* Register the contraction matrices (device, [N][lda] each) the scenarios index. */
 int sos_plan_set_phase(sos_plan* plan, const double* const* A_d, int n_matrices, int lda);

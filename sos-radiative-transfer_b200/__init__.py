@@ -11,7 +11,7 @@ the repository root) or with importlib.import_module("sos-radiative-transfer_b20
 from . import _lib
 from ._lib import SosError
 from .grid import mu_grid, tau_profile, extrapolation_width, aerosol_rows
-from .phase import phase_matrices, phase_P, phase_P0, phase_table
+from .phase import phase_matrices, phase_P, phase_P0, phase_table, phase_modes
 from . import mie
 from .mie import EVA_AEROSOL, WILDFIRE_AEROSOL
 from .engine import SosEngine, ScenarioCoefficients, SolveResult
@@ -24,12 +24,14 @@ from .multi_gpu import PeerFields, PeerBuffers, LayerShardedSolver, MuShardedSol
 from .drivers import (Scenario, DriverResult, BatchSolver, solve_scenarios, SOS_Aer_main_specular,
                       SOS_Aer_main_lambertian, SOS_Aer_radiative_forcing, SOS_Aer_critical_albedo,
                       critical_albedo_sweep, EVA, WILDFIRE, clear_caches)
+from .azimuth import AzimuthalResult, solve_azimuthal
 
 __all__ = [
-    "SosError", "mu_grid", "tau_profile", "extrapolation_width", "aerosol_rows", "phase_matrices", "phase_P", "phase_P0", "phase_table", "mie", "EVA_AEROSOL", "WILDFIRE_AEROSOL",
+    "SosError", "mu_grid", "tau_profile", "extrapolation_width", "aerosol_rows", "phase_matrices", "phase_P", "phase_P0", "phase_table", "phase_modes", "mie", "EVA_AEROSOL", "WILDFIRE_AEROSOL",
     "SosEngine", "ScenarioCoefficients", "SolveResult", "I1_NumInt", "Jn_NumInt", "In_NumInt",
     "mu_approx_In", "clear_cache", "Scenario", "DriverResult", "BatchSolver", "solve_scenarios",
     "MuShardedSolver", "LayerShardedSolver", "PeerFields", "PeerBuffers", "mu_blocks", "shard_scenarios", "gather_scenario_results", "allgather_columns", "shard_range",
     "SOS_Aer_main_specular", "SOS_Aer_main_lambertian", "SOS_Aer_radiative_forcing", "SOS_Aer_critical_albedo", "critical_albedo_sweep", "EVA", "WILDFIRE", "clear_caches",
+    "AzimuthalResult", "solve_azimuthal",
     "graphe", "graphe_diffusivity", "graphe_flux", "graphe_heating_rate", "graphe_successive_dif", "graphe_flux_up_down", "successive_diffusivity",
 ]

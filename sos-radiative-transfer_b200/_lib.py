@@ -48,14 +48,14 @@ class sos_scenario(C.Structure):
         ("phase_atm", C.c_int),
         ("phase_aer", C.c_int),
         ("extrap_width", C.c_int * 3),
-        ("reserved", C.c_int),
+        ("order_cap", C.c_int),
     ]
 
 
 # the same 80 bytes as a NumPy record: whole batches are marshalled without a Python loop (engine.scenario_table)
 SCENARIO_DTYPE = np.dtype([("mu0", "f8"), ("grd_alb", "f8"), ("tauStar_tot", "f8"), ("coef_atm", "f8"), ("coef_mix_atm", "f8"),
                            ("coef_mix_aer", "f8"), ("threshold", "f8"), ("phase_atm", "i4"), ("phase_aer", "i4"),
-                           ("extrap_width", "i4", 3), ("reserved", "i4")])
+                           ("extrap_width", "i4", 3), ("order_cap", "i4")])
 assert SCENARIO_DTYPE.itemsize == C.sizeof(sos_scenario)
 
 
@@ -88,6 +88,9 @@ SIGNATURES = {
     "sos_extrap_layout": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "sos_build_contraction": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, _vp]),
     "sos_build_phase": (C.c_int, [_vp, C.c_int, C.c_double, C.c_double, _vp, _vp, _vp, _vp, C.c_int, _vp, C.c_int, _vp, _vp]),
+    "sos_build_phase_modes": (C.c_int, [_vp, C.c_int, C.c_double, C.c_double, C.c_int, _vp, _vp, C.c_int, _vp, _vp, C.c_int, _vp,
+                                        C.c_int, C.c_size_t, _vp, _vp]),
+    "sos_azimuth_synthesis": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, _vp]),
     "sos_plan_set_phase": (C.c_int, [_vp, C.POINTER(_vp), C.c_int, C.c_int]),
     "sos_fold_layout": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "sos_build_folded": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.POINTER(C.c_double), _vp]),

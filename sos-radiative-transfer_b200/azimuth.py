@@ -1,0 +1,148 @@
+"""Azimuth-resolved radiance: Fourier modes of the phase function solved as batch members and summed on the device.
+
+Every field the drivers return is the azimuth average (mode 0) of the radiance.  For a plane-parallel medium each Fourier
+mode m of the radiance obeys the same equation as mode 0 -- the same contraction J = (omega/4) int P I dmu', sweeps and
+specular mirror coupling -- with the operand P_m and the solar vector P0_m of phase.phase_modes instead of P and P0.  So a
+(geometry, mode) pair is one more member of a batch: its own operand index and first-order table row, summing exactly the
+orders its mode 0 summed (sos_scenario.order_cap), and
+
+    I(tau, mu, phi) = I_0 + 2 sum_{m >= 1} I_m cos(m phi)
+
+is summed on the device (sos_azimuth_synthesis).
+
+phi is the azimuth of the PROPAGATION direction of the diffuse light relative to the propagation azimuth of the solar beam:
+with the grid's signs (mu < 0 downward) the beam travels along (-mu0, 0), cos Theta = -mu0 mu + sqrt(1 - mu0^2) sqrt(1 - mu^2)
+cos phi, and phi = 0 is the forward half-plane.  A sensor's relative azimuth (the azimuth of its viewing direction, opposite
+to the propagation of the light it receives) is phi + pi.
+"""
+from __future__ import annotations
+
+from dataclasses import dataclass, replace
+from typing import List, Optional, Sequence
+
+import numpy as np
+import torch
+
+from . import phase as PH
+from .drivers import (DriverResult, MAX_PHASES_PER_PLAN, BatchSolver, Scenario, _MODE_STACKS, grid_groups, solved_batches,
+                      split_for_plan_limits)
+
+# phase functions per plan of the mode members (two per mode: typically 8 modes per plan)
+MODE_PHASES_PER_PLAN = MAX_PHASES_PER_PLAN
+
+
+@dataclass
+class AzimuthalResult:
+    """base: the mode-0 result (what solve_scenarios returns for the scenario); radiance (n_rows, n_phi, N): I(tau_row, mu, phi)
+    at the layers `rows` and azimuths `phi`; modes (n_modes, n_rows, N): the Fourier components I_m at those layers (mode 0 =
+    base.I rows); mode_orders / mode_status (n_modes,): orders summed and status bits of every mode (a mode whose
+    atmosphere and aerosol modes vanish is not solved: 0 orders, I_m = 0)."""
+    base: DriverResult
+    radiance: np.ndarray
+    rows: np.ndarray
+    phi: np.ndarray
+    n_modes: int
+    modes: np.ndarray
+    mode_orders: np.ndarray
+    mode_status: np.ndarray
+
+
+def _mode_spec(spec, m: int, n_quad: int):
+    name, g = PH.resolve(spec[0], spec[1] if len(spec) > 1 else None)
+    return (name, g, m, n_quad)
+
+
+def _vanishes(spec, m: int) -> bool:
+    return PH.mode_vanishes(PH.resolve(spec[0], spec[1] if len(spec) > 1 else None)[0], m)
+
+
+def _validate(scenarios: Sequence[Scenario], n_modes: int, n_quad: int):
+    if n_modes < 1:
+        raise ValueError("solve_azimuthal: n_modes must be >= 1")
+    if n_quad < 2 * n_modes:
+        raise ValueError(f"solve_azimuthal: n_quad = {n_quad} azimuth nodes cannot resolve {n_modes} modes (need >= 2 n_modes)")
+    for sc in scenarios:
+        if sc.surface in ("lambert", "lambert_readme") and sc.grd_alb > 0:
+            # the first order reflects the beam specularly while the n >= 2 coupling is isotropic: no consistent mode split
+            raise ValueError(f"solve_azimuthal: surface {sc.surface!r} with grd_alb > 0 has no Fourier-mode decomposition")
+        for spec in (sc.atm_phase, sc.aer_phase):
+            if not isinstance(spec[0], str):
+                raise ValueError("solve_azimuthal: modes are built from the phase function; (P0, P) arrays cannot be split")
+
+
+def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -1), n_quad: int = 25,
+                    device=None) -> List[AzimuthalResult]:
+    """Radiance as a function of azimuth for every scenario: modes 0 .. n_modes-1, synthesized at the azimuths `phi`
+    (radians, see the module docstring for the convention) on the layers `rows` (negative = from the bottom).
+
+    Mode 0 is solved exactly as solve_scenarios solves it (result.base); modes 1 .. n_modes-1 of all geometries are batched
+    with order_cap = the orders their mode 0 summed, so the azimuth-resolved field is the same truncated series, order for
+    order, as the mode-0 field.  n_quad: azimuth nodes of the mode builder (>= 2 n_modes; 25 = the azimuth-averaged
+    builders' nodes, enough for Rayleigh and moderate HG -- sharp peaks need more).  Lambert surfaces with grd_alb > 0 and
+    caller-supplied (P0, P) arrays raise ValueError before any device work."""
+    scenarios = list(scenarios)
+    K, n_quad = int(n_modes), int(n_quad)
+    _validate(scenarios, K, n_quad)
+    phi = np.atleast_1d(np.asarray(phi, dtype=np.float64))
+    if phi.ndim != 1:
+        raise ValueError("solve_azimuthal: phi must be a 1-D sequence of azimuths")
+    n_az = phi.size
+    for sc in scenarios:
+        if not all(-sc.nb_layers <= int(r) < sc.nb_layers for r in rows) or len(rows) == 0:
+            raise ValueError(f"solve_azimuthal: rows must lie in [-{sc.nb_layers}, {sc.nb_layers})")
+    w_modes = 2.0 * np.cos(np.arange(K)[:, None] * phi[None, :])   # row m >= 1: 2 cos(m phi_p)
+    ones = np.ones(n_az)
+    out: List[Optional[AzimuthalResult]] = [None] * len(scenarios)
+    try:
+        for group in grid_groups(scenarios):
+            rws = np.array([int(r) for r in rows], dtype=np.int64) % scenarios[group[0]].nb_layers
+            pos = {i: k for k, i in enumerate(group)}
+            n0 = {}
+            base = {}
+            modes = {i: np.zeros((K, rws.size, 2 * scenarios[i].nb_angles)) for i in group}
+            orders = {i: np.zeros(K, dtype=np.int64) for i in group}
+            status = {i: np.zeros(K, dtype=np.int64) for i in group}
+            radiance = None
+            for idxs, bs, res, results in solved_batches(scenarios, device=device, groups=[group]):
+                eng = bs.engine
+                if radiance is None:
+                    radiance = torch.empty((len(group), rws.size, n_az, eng.N), dtype=torch.float64, device=eng.device)
+                eng.azimuth_synthesis(res.I, np.array([pos[i] for i in idxs]), np.tile(ones, (len(idxs), 1)), len(group), rws,
+                                      radiance, accumulate=False)
+                for i, r in zip(idxs, results):
+                    base[i], n0[i] = r, int(r.n)
+                    modes[i][0] = r.I[rws]
+                    orders[i][0], status[i][0] = r.n, r.status
+            # modes 1 .. K-1 of every geometry of the group, each summing the orders of its mode 0
+            members, keys = [], []
+            for i in group:
+                sc = scenarios[i]
+                for m in range(1, K):
+                    if _vanishes(sc.atm_phase, m) and _vanishes(sc.aer_phase, m):
+                        continue   # I_m = 0: nothing to solve
+                    members.append(replace(sc, atm_phase=_mode_spec(sc.atm_phase, m, n_quad),
+                                           aer_phase=_mode_spec(sc.aer_phase, m, n_quad)))
+                    keys.append((i, m))
+            for sub in split_for_plan_limits(members, range(len(members)), max_phases=MODE_PHASES_PER_PLAN):
+                caps = [n0[keys[j][0]] for j in sub]
+                bs = BatchSolver([members[j] for j in sub], device=device, order_caps=caps)
+                try:
+                    res = bs.solve(max_orders=max(caps))
+                    eng = bs.engine
+                    geo = np.array([pos[keys[j][0]] for j in sub])
+                    w = np.stack([w_modes[keys[j][1]] for j in sub])
+                    eng.azimuth_synthesis(res.I, geo, w, len(group), rws, radiance, accumulate=True)
+                    fields = res.I.view(eng.S, eng.L, eng.ld)[:, torch.as_tensor(rws, device=eng.device), : eng.N].cpu().numpy()
+                    for s, j in enumerate(sub):
+                        i, m = keys[j]
+                        modes[i][m] = fields[s]
+                        orders[i][m], status[i][m] = res.n_orders[s], res.status[s]
+                finally:
+                    bs.engine.close()
+            rad = radiance.cpu().numpy()
+            for i in group:
+                out[i] = AzimuthalResult(base=base[i], radiance=rad[pos[i]], rows=rws.copy(), phi=phi.copy(), n_modes=K,
+                                         modes=modes[i], mode_orders=orders[i], mode_status=status[i])
+    finally:
+        _MODE_STACKS.clear()   # the device mode stacks serve the sub-batches of one call
+    return out  # type: ignore

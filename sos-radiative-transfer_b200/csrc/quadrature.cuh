@@ -103,4 +103,45 @@ build_contraction_kernel(const double* __restrict__ P, int ldp, double* __restri
   }
 }
 
+
+// Azimuth synthesis (include/sos_b200.h: sos_azimuth_synthesis).  Thread = one mu column of one (geometry, row) and AZ_CHUNK
+// azimuths; the members of the geometry are summed in ascending order (no atomics: deterministic).  HBM bound: every
+// member row is read once per azimuth chunk (the chunks of one row hit L2), every output element written once.
+constexpr int AZ_THREADS = 128;
+constexpr int AZ_CHUNK = 8;
+
+struct SynthTables {
+  const int* geo;       // [n_present] geometry of each present group
+  const int* mem_off;   // [n_present + 1]
+  const int* members;   // member scenarios of the groups, ascending within a group
+  const double* w;      // [S][n_az]
+  const int* rows;      // [n_rows]
+};
+
+__global__ void __launch_bounds__(AZ_THREADS)
+azimuth_synthesis_kernel(const double* __restrict__ I, int L, int ld, int N, const SynthTables t, int n_rows, int n_az,
+                         double* __restrict__ out, int accumulate) {
+  const int col = blockIdx.x * AZ_THREADS + threadIdx.x;
+  if (col >= N) return;
+  const int gi = blockIdx.y / n_rows, r = blockIdx.y % n_rows;
+  const int p0 = blockIdx.z * AZ_CHUNK;
+  const int np = min(AZ_CHUNK, n_az - p0);
+  const int row = t.rows[r];
+  double acc[AZ_CHUNK];
+#pragma unroll
+  for (int q = 0; q < AZ_CHUNK; ++q) acc[q] = 0.0;
+  for (int j = t.mem_off[gi]; j < t.mem_off[gi + 1]; ++j) {
+    const int s = t.members[j];
+    const double v = __ldg(&I[(static_cast<size_t>(s) * L + row) * ld + col]);
+    const double* __restrict__ w = t.w + static_cast<size_t>(s) * n_az + p0;
+#pragma unroll
+    for (int q = 0; q < AZ_CHUNK; ++q)
+      if (q < np) acc[q] = fma(__ldg(&w[q]), v, acc[q]);
+  }
+  double* o = out + ((static_cast<size_t>(t.geo[gi]) * n_rows + r) * n_az + p0) * N + col;
+#pragma unroll
+  for (int q = 0; q < AZ_CHUNK; ++q)
+    if (q < np) o[static_cast<size_t>(q) * N] = accumulate ? o[static_cast<size_t>(q) * N] + acc[q] : acc[q];
+}
+
 }  // namespace sosquad

@@ -1016,6 +1016,121 @@ int sos_build_phase(sos_plan* p, int family, double g, double mu0, const double*
   return SOS_OK;
 }
 
+int sos_build_phase_modes(sos_plan* p, int family, double g, double mu0, int n_phi, const double* phi_h, const double* cphi_h,
+                          int n_modes, const double* tab_x_d, const double* tab_y_d, int tab_n, double* P_d, int ldp,
+                          size_t mode_stride, double* P0_d, void* stream) {
+  if (!p || !phi_h || !cphi_h || (!P_d && !P0_d)) return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  if (family < 0 || family > 2 || (family == 2 && (!tab_x_d || !tab_y_d || tab_n < 2))) return SOS_ERR_INVALID;
+  if (n_phi < 2 || n_phi > sosphase::MAX_NPHI || n_modes < 1 || n_modes > sosphase::MAX_MODES) return SOS_ERR_INVALID;
+  const int N = p->N;
+  if (P_d && (ldp < N || (n_modes > 1 && mode_stride < static_cast<size_t>(N) * ldp))) return SOS_ERR_INVALID;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // node table [phi | cos(0 - phi) | trapezoid weight * cos(m phi)] computed here from what the host passed
+  std::vector<double> tab(static_cast<size_t>(n_phi) * (2 + n_modes), 0.0);
+  double* phi = tab.data();
+  double* cphi = phi + n_phi;
+  double* wcos = cphi + n_phi;
+  for (int k = 0; k < n_phi; ++k) {
+    phi[k] = phi_h[k];
+    cphi[k] = cphi_h[k];
+    const double tw = 0.5 * ((k + 1 < n_phi ? phi_h[k + 1] : phi_h[k]) - (k > 0 ? phi_h[k - 1] : phi_h[k]));
+    for (int m = 1; m < n_modes; ++m) wcos[static_cast<size_t>(k) * n_modes + m] = tw * cphi_h[static_cast<size_t>(1 + m) * n_phi + k];
+  }
+  double* tab_d = nullptr;
+  SOS_CUDA(cudaMallocAsync(&tab_d, tab.size() * sizeof(double), st));
+  SOS_CUDA(cudaMemcpyAsync(tab_d, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  sosphase::ModeArgs a;
+  std::memset(&a, 0, sizeof(a));
+  a.pa.family = family; a.pa.g = g; a.pa.tab_x = tab_x_d; a.pa.tab_y = tab_y_d; a.pa.tab_n = tab_n;
+  a.n_phi = n_phi; a.n_modes = n_modes;
+  a.phi = tab_d; a.cphi = tab_d + n_phi; a.wcos = tab_d + 2 * n_phi;
+  const size_t smem = static_cast<size_t>(n_modes - 1) * sosphase::MODE_THREADS * sizeof(double);
+  int r = SOS_OK;
+  if (P_d) {
+    cudaFuncSetAttribute(sosphase::phase_modes_raw_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    const long long n_el = static_cast<long long>(N) * N;
+    sosphase::phase_modes_raw_kernel<false><<<static_cast<unsigned>((n_el + sosphase::MODE_THREADS - 1) / sosphase::MODE_THREADS),
+                                             sosphase::MODE_THREADS, smem, st>>>(a, p->dev.mu, N, mu0, P_d, ldp, mode_stride);
+    r = launch_check(p, "phase_modes_raw_kernel");
+    if (!r) {
+      // every mode is normalised by the column integrals of mode 0 (the same kernels as sos_build_phase)
+      sosphase::phase_colint_kernel<<<(N + 127) / 128, 128, 0, st>>>(p->dev.mu, N, P_d, ldp, p->d_colint);
+      r = launch_check(p);
+    }
+    const dim3 grid((N + 31) / 32, (N + 7) / 8);
+    for (int m = 0; m < n_modes && !r; ++m) {
+      sosphase::phase_normalise_kernel<<<grid, 256, 0, st>>>(N, P_d + m * mode_stride, ldp, p->d_colint);
+      r = launch_check(p);
+    }
+  }
+  if (P0_d && !r) {
+    cudaFuncSetAttribute(sosphase::phase_modes_raw_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    sosphase::phase_modes_raw_kernel<true><<<(N + sosphase::MODE_THREADS - 1) / sosphase::MODE_THREADS, sosphase::MODE_THREADS, smem,
+                                            st>>>(a, p->dev.mu, N, mu0, P0_d, N, 0);
+    r = launch_check(p, "phase_modes_raw_kernel");
+    if (!r) {
+      sosphase::phase_p0_modes_norm_kernel<<<1, 256, 0, st>>>(p->dev.mu, N, n_modes, P0_d);
+      r = launch_check(p);
+    }
+  }
+  SOS_CUDA(cudaFreeAsync(tab_d, st));
+  return r;
+}
+
+int sos_azimuth_synthesis(sos_plan* p, const double* I_d, const int* geo_h, const double* w_h, int n_geo, const int* rows_h,
+                          int n_rows, int n_az, double* out_d, int accumulate, void* stream) {
+  if (!p || !I_d || !geo_h || !w_h || !rows_h || !out_d || n_geo < 1 || n_rows < 1 || n_az < 1) return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  const GridDev& g = p->dev;
+  const int S = g.S;
+  for (int r = 0; r < n_rows; ++r)
+    if (rows_h[r] < 0 || rows_h[r] >= g.L) return SOS_ERR_INVALID;
+  // members of every present geometry, ascending; one int table [geo | mem_off | members | rows] + the weights
+  std::vector<std::vector<int>> by_geo(n_geo);
+  for (int s = 0; s < S; ++s) {
+    if (geo_h[s] < -1 || geo_h[s] >= n_geo) return SOS_ERR_INVALID;
+    if (geo_h[s] >= 0) by_geo[geo_h[s]].push_back(s);
+  }
+  std::vector<int> geo, off(1, 0), members;
+  for (int k = 0; k < n_geo; ++k) {
+    if (by_geo[k].empty()) continue;
+    geo.push_back(k);
+    members.insert(members.end(), by_geo[k].begin(), by_geo[k].end());
+    off.push_back(static_cast<int>(members.size()));
+  }
+  const int n_present = static_cast<int>(geo.size());
+  if (n_present == 0) return SOS_OK;
+  if (static_cast<long long>(n_present) * n_rows > 65535) return SOS_ERR_UNSUPPORTED;
+  const size_t n_w = static_cast<size_t>(S) * n_az;
+  std::vector<int> itab;
+  itab.reserve(geo.size() + off.size() + members.size() + n_rows);
+  itab.insert(itab.end(), geo.begin(), geo.end());
+  itab.insert(itab.end(), off.begin(), off.end());
+  itab.insert(itab.end(), members.begin(), members.end());
+  itab.insert(itab.end(), rows_h, rows_h + n_rows);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  char* buf = nullptr;
+  const size_t wbytes = n_w * sizeof(double);
+  SOS_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&buf), wbytes + itab.size() * sizeof(int), st));
+  SOS_CUDA(cudaMemcpyAsync(buf, w_h, wbytes, cudaMemcpyHostToDevice, st));
+  SOS_CUDA(cudaMemcpyAsync(buf + wbytes, itab.data(), itab.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  const int* it = reinterpret_cast<const int*>(buf + wbytes);
+  sosquad::SynthTables t;
+  t.w = reinterpret_cast<const double*>(buf);
+  t.geo = it;
+  t.mem_off = t.geo + geo.size();
+  t.members = t.mem_off + off.size();
+  t.rows = t.members + members.size();
+  const dim3 grid((g.N + sosquad::AZ_THREADS - 1) / sosquad::AZ_THREADS, n_present * n_rows,
+                  (n_az + sosquad::AZ_CHUNK - 1) / sosquad::AZ_CHUNK);
+  if (grid.z > 65535) { cudaFreeAsync(buf, st); return SOS_ERR_UNSUPPORTED; }
+  sosquad::azimuth_synthesis_kernel<<<grid, sosquad::AZ_THREADS, 0, st>>>(I_d, g.L, g.ld, g.N, t, n_rows, n_az, out_d, accumulate ? 1 : 0);
+  const int r = launch_check(p, "azimuth_synthesis_kernel");
+  SOS_CUDA(cudaFreeAsync(buf, st));
+  return r;
+}
+
 static int encode_A_maps(sos_plan* p) {
   const int bn = p->gemm_bn + 8;  // rows are loaded 8 columns wider than the tile (bank layout)
   for (size_t i = 0; i < p->A_ptrs.size(); ++i) {

@@ -1468,9 +1468,13 @@ sweep_zone_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ J
     bool nonfinite = false;
     const int a0 = toa ? max(M, c_lo) : c_lo;
     const int a1 = toa ? c_hi : min(M, c_hi);
+    // an order-capped member (an azimuthal mode m >= 1) stops on its cap: its ratio is meaningless (0/0 on the mu = +-1
+    // columns), only a non-finite I_n is an error
+    const bool capped = g.scen[s].order_cap > 0;
     for (int m = a0 + lane; m < a1; m += 32) {
-      const double r = Is[roff + m] / __ldcg(&Ia[roff + m]);
-      if (isnan(r)) nonfinite = true; else rmax = fmax(rmax, r);
+      const double v = Is[roff + m];
+      const double r = v / __ldcg(&Ia[roff + m]);
+      if (capped ? !isfinite(v) : isnan(r)) nonfinite = true; else rmax = fmax(rmax, r);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) rmax = fmax(rmax, __shfl_xor_sync(0xffffffffu, rmax, o));
@@ -1478,7 +1482,7 @@ sweep_zone_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ J
     if (lane == 0) {
       if (toa) g.state[s].ratio_toa = rmax;
       if (surf) g.state[s].ratio_surf = rmax;
-      if (nonfinite || rmax == INFINITY) atomicOr(&g.state[s].status, SOS_STATUS_NONFINITE);  // -inf: no owned column
+      if (nonfinite || (rmax == INFINITY && !capped)) atomicOr(&g.state[s].status, SOS_STATUS_NONFINITE);  // -inf: no owned column
     }
   }
 }
@@ -1516,8 +1520,9 @@ __device__ __forceinline__ void converge_block(const GridDev& g, int order_arg, 
     ScenState& st = g.state[s];
     if (st.active) {
       st.n_orders = order;
+      const int cap = g.scen[s].order_cap;
       const double r = fmax(st.ratio_toa, st.ratio_surf);
-      if (!(r >= g.scen[s].threshold)) st.active = 0;
+      if (cap > 0 ? order >= cap : !(r >= g.scen[s].threshold)) st.active = 0;
     }
   }
   __syncthreads();
@@ -1556,7 +1561,8 @@ __global__ void reset_kernel(const GridDev g, const double* __restrict__ I1, int
     st.n_orders = 1;
     st.status = 0;
     if (s == 0) *order_counter = 1;
-    st.active = (fmax(st.ratio_toa, r) >= g.scen[s].threshold) ? 1 : 0;
+    const int cap = g.scen[s].order_cap;
+    st.active = (cap > 0 ? 1 < cap : fmax(st.ratio_toa, r) >= g.scen[s].threshold) ? 1 : 0;
   }
 }
 

@@ -20,7 +20,9 @@ from . import grid as G
 from . import phase as PH
 from .engine import ScenarioCoefficients, SosEngine
 
-PhaseSpec = Union[Tuple[str, float], Tuple[np.ndarray, np.ndarray]]
+# (name, g), optionally (name, g, m, n_quad): azimuthal Fourier mode m of the family built with n_quad azimuth nodes
+# (phase.phase_modes; the azimuth module builds these), or caller-supplied (P0, P) arrays
+PhaseSpec = Union[Tuple[str, float], Tuple[str, float, int, int], Tuple[np.ndarray, np.ndarray]]
 
 
 @dataclass
@@ -86,17 +88,29 @@ class PhaseCache:
         if isinstance(spec[0], str):
             name, g = PH.resolve(spec[0], spec[1] if len(spec) > 1 else None)   # 'eva' / 'wildfire' -> the log-normal Mie mixture
             g = tuple(float(v) for v in g) if isinstance(g, (tuple, list)) else float(g)
-            kP, k0 = (name, g, M), (name, g, M, float(mu0))
+            mode = tuple(int(v) for v in spec[2:4]) if len(spec) > 2 else ()   # (m, n_quad) of an azimuthal mode
+            kP, k0 = (name, g, M) + mode, (name, g, M, float(mu0)) + mode
             if need_P and kP not in self._P:
-                self._P[kP] = PH.phase_P(name, M, mu, g)
+                self._P[kP] = PH.phase_P(name, M, mu, g) if not mode else _host_mode(name, g, M, mu, mode)[1]
             if k0 not in self._P0:
-                self._P0[k0] = PH.phase_P0(name, M, mu, mu0, g)
+                self._P0[k0] = PH.phase_P0(name, M, mu, mu0, g) if not mode else _host_mode(name, g, M, mu, mode, mu0)[0]
             return self._P0[k0], self._P.get(kP), kP
         P0, P = spec
         return np.asarray(P0, dtype=np.float64), np.asarray(P, dtype=np.float64), ("array", id(P))
 
 
+def _host_mode(name, g, M, mu, mode, mu0=None):
+    """(P0_m or None, P_m or None) of mode (m, n_quad) on the host; exact zeros for a mode that vanishes."""
+    m, nq = mode
+    N = 2 * M
+    if PH.mode_vanishes(name, m):
+        return (np.zeros(N) if mu0 is not None else None), np.zeros((N, N))
+    P0, P = PH.phase_modes(name, M, mu, m + 1, g, mu0=mu0, n_quad=nq, want_P=mu0 is None)
+    return (P0[m] if P0 is not None else None), (P[m] if P is not None else None)
+
+
 _PHASES = PhaseCache()
+_MODE_STACKS = {}   # device-built mode stacks (P_0 .. P_{K-1}) per (family, g, grid, n_quad, device), see _DeviceBuilt
 
 
 def clear_caches(disk: bool = False):
@@ -125,11 +139,23 @@ class _DeviceBuilt:
     """Placeholder for a phase matrix that SosEngine.set_phase builds on the device when (and only
     when) the operand cache misses."""
 
-    def __init__(self, engine, name, g):
-        self.engine, self.name, self.g = engine, name, g
+    def __init__(self, engine, name, g, mode=None):
+        self.engine, self.name, self.g, self.mode = engine, name, g, mode
 
     def build(self):
-        return self.engine.build_phase_matrix(self.name, self.g)[0]
+        if self.mode is None:
+            return self.engine.build_phase_matrix(self.name, self.g)[0]
+        m, nq = self.mode
+        eng = self.engine
+        if PH.mode_vanishes(self.name, m):
+            return torch.zeros((eng.N, eng.N), dtype=torch.float64, device=eng.device)
+        # one launch builds modes 0 .. K-1 together (the phase function is evaluated once per element and node): build in
+        # steps of 8 modes and keep the stack for the other modes of the same family
+        key = (self.name, self.g, eng.N, eng.mu.tobytes(), nq, eng.device.index)
+        stack = _MODE_STACKS.get(key)
+        if stack is None or stack.shape[0] <= m:
+            stack = _MODE_STACKS[key] = eng.build_phase_modes(self.name, self.g, n_modes=min(64, (m // 8 + 1) * 8), n_quad=nq)[0]
+        return stack[m]
 
 
 def _group_key(sc: Scenario):
@@ -141,7 +167,9 @@ class BatchSolver:
     """All scenarios of one group (same L, M, aerosol rows, surface) on one device."""
 
     def __init__(self, scenarios: Sequence[Scenario], device=None, chunk_rows: int = 0, phases: Optional[PhaseCache] = None,
-                 device_phase: bool = True, fold: Optional[bool] = None):
+                 device_phase: bool = True, fold: Optional[bool] = None, order_caps: Optional[Sequence[int]] = None):
+        """order_caps: per scenario, sum exactly orders 1 .. cap instead of stopping on the threshold (0 = the threshold;
+        sos_scenario.order_cap); None = all 0.  update() takes the caps of the next batch the same way."""
         keys = {_group_key(s) for s in scenarios}
         if len(keys) != 1:
             raise ValueError("BatchSolver: scenarios must share nb_layers, nb_angles, aerosol rows and surface")
@@ -153,7 +181,7 @@ class BatchSolver:
         self._device_phase = device_phase
         self.z = G.aerosol_rows(scenarios[0].z0, scenarios[0].z_up, scenarios[0].z_down, L)[0]
         self._mat_index, self._mats, self._mat_keys = {}, [], []
-        coefs = self._prepare(scenarios)
+        coefs = self._prepare(scenarios, order_caps)
         surface = {"specular": _lib.SURFACE_SPECULAR, "lambert": _lib.SURFACE_LAMBERT,
                    "lambert_readme": _lib.SURFACE_LAMBERT_README}[surf]
         self.engine = SosEngine(self.mu, self.tau, coefs, [0, self.idx_up, self.idx_down + 1, L], surface,
@@ -161,7 +189,7 @@ class BatchSolver:
         self._register_phases()
         self.I1 = None
 
-    def _prepare(self, scenarios):
+    def _prepare(self, scenarios, order_caps=None):
         """Host side of a batch: tau profiles, per-scenario scalars, the table of distinct solar phase vectors with the rows
         and weights each scenario's first-order coefficients are made of (assembled on the device); phase functions met for the
         first time are appended to self._mats (the caller registers them)."""
@@ -233,6 +261,8 @@ class BatchSolver:
         coefs["phase_aer"] = mat_idx[:, 1]
         coefs["extrap_width"][:, 0] = G.extrapolation_widths(tau[:, iu - 1], M)
         coefs["extrap_width"][:, 1] = coefs["extrap_width"][:, 2] = G.extrapolation_widths(tau[:, idn], M)
+        if order_caps is not None:
+            coefs["order_cap"] = order_caps
         self.tau = tau
         return coefs
 
@@ -253,16 +283,16 @@ class BatchSolver:
             # contraction operand is already resident; only the cheap P0 vectors were built on the host
             for i, k in enumerate(self._mat_keys):
                 if k is not None and mats[i] is None:
-                    mats[i] = _DeviceBuilt(self.engine, k[0], k[1])
+                    mats[i] = _DeviceBuilt(self.engine, k[0], k[1], tuple(k[3:5]) if len(k) > 3 else None)
         self.engine.set_phase(mats, keys=self._mat_keys)
 
-    def update(self, scenarios: Sequence[Scenario]):
+    def update(self, scenarios: Sequence[Scenario], order_caps: Optional[Sequence[int]] = None):
         """Feed the solver its next batch (same grid group, same number of scenarios): the plan, its device buffers and
         the registered phase operands are kept (sos_plan_update); only tau, the per-scenario scalars and the first-order
         coefficients change.  What a parameter sweep calls between batches instead of building a new BatchSolver."""
         if len(scenarios) != len(self.scenarios) or {_group_key(s) for s in scenarios} != {self._key}:
             raise ValueError("BatchSolver.update: the next batch must keep the grid group and the batch size")
-        coefs = self._prepare(scenarios)
+        coefs = self._prepare(scenarios, order_caps)
         if self._new_mats:
             if len(self._mats) > 16:
                 raise ValueError("BatchSolver.update: more than 16 phase functions in one plan")
@@ -348,17 +378,17 @@ def _phase_id(spec):
     return spec if isinstance(spec[0], str) else ("array", id(spec[1]))
 
 
-def split_for_plan_limits(scenarios: Sequence[Scenario], idxs: Sequence[int]) -> List[List[int]]:
-    """Cut one grid group into sub-batches a plan accepts: at most 16 distinct phase matrices and 48 (atm, aer) operand
-    pairs each (a phase sweep over more than 16 HG asymmetry factors, or per-scenario Mie arrays, would otherwise be
-    refused by sos_plan_create).  Order inside the group is kept."""
+def split_for_plan_limits(scenarios: Sequence[Scenario], idxs: Sequence[int], max_phases: int = MAX_PHASES_PER_PLAN) -> List[List[int]]:
+    """Cut one grid group into sub-batches a plan accepts: at most 16 (max_phases) distinct phase matrices and 48 (atm, aer)
+    operand pairs each (a phase sweep over more than 16 HG asymmetry factors, or per-scenario Mie arrays, would otherwise
+    be refused by sos_plan_create).  Order inside the group is kept."""
     out, cur, phases, pairs = [], [], set(), set()
     for i in idxs:
         sc = scenarios[i]
         pa, pe = _phase_id(sc.atm_phase), _phase_id(sc.aer_phase)
         new_phases = phases | {pa, pe}
         new_pairs = pairs | {(pa, pe), (pa, None)}
-        if cur and (len(new_phases) > MAX_PHASES_PER_PLAN or len(new_pairs) > MAX_GROUPS_PER_PLAN):
+        if cur and (len(new_phases) > max_phases or len(new_pairs) > MAX_GROUPS_PER_PLAN):
             out.append(cur)
             cur, new_phases, new_pairs = [], {pa, pe}, {(pa, pe), (pa, None)}
         cur.append(i)
@@ -371,18 +401,34 @@ def split_for_plan_limits(scenarios: Sequence[Scenario], idxs: Sequence[int]) ->
 def solve_scenarios(scenarios: Sequence[Scenario], device=None, keep_orders: int = 0, quadratures: bool = True,
                     fold: Optional[bool] = None) -> List[DriverResult]:
     """Solve any mix of scenarios; those sharing a grid are batched together.  fold: see SosEngine."""
+    out: List[Optional[DriverResult]] = [None] * len(scenarios)
+    for idxs, _, _, results in solved_batches(scenarios, device=device, keep_orders=keep_orders, quadratures=quadratures,
+                                              fold=fold):
+        for i, r in zip(idxs, results):
+            out[i] = r
+    return out  # type: ignore
+
+
+def grid_groups(scenarios: Sequence[Scenario]) -> List[List[int]]:
+    """Indices of the scenarios that share a grid (layers, angles, aerosol rows, surface), group by group."""
     groups: Dict[tuple, List[int]] = {}
     for i, sc in enumerate(scenarios):
         groups.setdefault(_group_key(sc), []).append(i)
-    out: List[Optional[DriverResult]] = [None] * len(scenarios)
-    batches = [b for idxs in groups.values() for b in split_for_plan_limits(scenarios, idxs)]
-    for idxs in batches:
+    return list(groups.values())
+
+
+def solved_batches(scenarios: Sequence[Scenario], device=None, keep_orders: int = 0, quadratures: bool = True,
+                   fold: Optional[bool] = None, groups: Optional[List[List[int]]] = None):
+    """The batches of solve_scenarios one at a time: yields (indices, BatchSolver, SolveResult, [DriverResult]) while the
+    batch's plan and device fields are still alive (the plan is closed when the caller asks for the next batch)."""
+    groups = grid_groups(scenarios) if groups is None else groups
+    for idxs in [b for g in groups for b in split_for_plan_limits(scenarios, g)]:
         bs = BatchSolver([scenarios[i] for i in idxs], device=device, fold=fold)
-        res = bs.solve(keep_orders=keep_orders)
-        for i, r in zip(idxs, bs.results(res, quadratures=quadratures, keep_orders=keep_orders)):
-            out[i] = r
-        bs.engine.close()
-    return out  # type: ignore
+        try:
+            res = bs.solve(keep_orders=keep_orders)
+            yield idxs, bs, res, bs.results(res, quadratures=quadratures, keep_orders=keep_orders)
+        finally:
+            bs.engine.close()
 
 
 def SOS_Aer_main_specular(keep_orders: int = 0, device=None, **params) -> DriverResult:

@@ -55,6 +55,7 @@ class ScenarioCoefficients:
     phase_atm: int = 0
     phase_aer: int = 0
     extrap_width: Sequence[int] = (0, 0, 0)
+    order_cap: int = 0   # > 0: sum exactly orders 1 .. order_cap, ignoring the threshold (an azimuthal mode m >= 1)
 
 
 class SolveResult:
@@ -127,6 +128,7 @@ class SosEngine:
             sc[i].phase_atm, sc[i].phase_aer = s.phase_atm, s.phase_aer
             for k in range(3):
                 sc[i].extrap_width[k] = int(s.extrap_width[k]) if k < len(s.extrap_width) else 0
+            sc[i].order_cap = int(s.order_cap)
         return sc
 
     def update(self, tau, scenarios: Sequence[ScenarioCoefficients]):
@@ -379,6 +381,57 @@ class SosEngine:
                                                 P.data_ptr(), N, P0.data_ptr() if P0 is not None else None, self._stream),
                        "sos_build_phase")
         return P, P0
+
+    def build_phase_modes(self, name: str, g: float = 0.5, n_modes: int = 1, mu0: Optional[float] = None, n_quad: int = 25,
+                          want_P: bool = True):
+        """Azimuthal Fourier modes m = 0 .. n_modes-1 of a phase function, built ON THE DEVICE (sos_build_phase_modes) with
+        n_quad azimuth nodes on [0, pi]: (P (n_modes, N, N) tensor or None, P0 (n_modes, N) tensor or None).  Families as in
+        build_phase_matrix; every mode is normalised by the column integrals of mode 0 (phase.phase_modes is the NumPy
+        reference).  At n_quad = 25 mode 0 is bit for bit build_phase_matrix."""
+        from . import phase as PH
+        N, K = self.N, int(n_modes)
+        P = torch.empty((K, N, N), dtype=torch.float64, device=self.device) if want_P else None
+        P0 = torch.empty((K, N), dtype=torch.float64, device=self.device) if mu0 is not None else None
+        if name == "iso":
+            for t, v in ((P, 2.0), (P0, 1.0)):
+                if t is not None:
+                    t.zero_()
+                    t[0].fill_(v)
+            return P, P0
+        fam = {"rayleigh": 0, "hg": 1, "fwc": 2, "mie_lognormal": 2}[name]
+        phi, cphi = PH.azimuth_nodes(n_quad, K)
+        tx = ty = None
+        if fam == 2:
+            xs, ys = PH.phase_table(name, g)
+            tx = torch.as_tensor(np.array(xs, dtype=np.float64)).to(self.device)
+            ty = torch.as_tensor(np.array(ys, dtype=np.float64)).to(self.device)
+        gval = float(g) if not isinstance(g, (tuple, list)) else 0.0
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_build_phase_modes(self._plan, fam, gval, float(mu0 if mu0 is not None else 0.5), int(n_quad),
+                                                      phi.ctypes.data, cphi.ctypes.data, K,
+                                                      tx.data_ptr() if tx is not None else None,
+                                                      ty.data_ptr() if ty is not None else None, int(tx.numel()) if tx is not None else 0,
+                                                      P.data_ptr() if P is not None else None, N, N * N,
+                                                      P0.data_ptr() if P0 is not None else None, self._stream),
+                       "sos_build_phase_modes")
+            torch.cuda.current_stream(self.device).synchronize()   # (the table tensors may be freed after this)
+        return P, P0
+
+    def azimuth_synthesis(self, I: torch.Tensor, geo: np.ndarray, weights: np.ndarray, n_geo: int, rows: Sequence[int],
+                          out: torch.Tensor, accumulate: bool):
+        """out[geo][r][p][:] (+)= sum over the members s of geo (ascending) of weights[s, p] * I[s, rows[r], :N]
+        (sos_azimuth_synthesis).  geo (S,) int: geometry of each member, -1 = not summed; out: (n_geo, n_rows, n_az, N)."""
+        ge = np.ascontiguousarray(geo, dtype=np.int32)
+        w = np.ascontiguousarray(weights, dtype=np.float64)
+        rw = np.ascontiguousarray(rows, dtype=np.int32)
+        n_az = w.shape[1]
+        if ge.shape != (self.S,) or w.shape != (self.S, n_az) or out.shape != (n_geo, rw.size, n_az, self.N) or not out.is_contiguous():
+            raise ValueError("azimuth_synthesis: shapes do not match the plan")
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_azimuth_synthesis(self._plan, I.data_ptr(), ge.ctypes.data, w.ctypes.data, int(n_geo),
+                                                      rw.ctypes.data, int(rw.size), int(n_az), out.data_ptr(), int(bool(accumulate)),
+                                                      self._stream), "sos_azimuth_synthesis")
+        return out
 
     # ------------------------------------------------------------------ operators
     def first_order(self, C_coef: np.ndarray, out: Optional[torch.Tensor] = None, also_into: Optional[torch.Tensor] = None) -> torch.Tensor:

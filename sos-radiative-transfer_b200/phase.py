@@ -127,3 +127,77 @@ def phase_P(name: str, nb_angles: int, mu: np.ndarray, g: float = 0.5, block: in
 def phase_matrices(name: str, nb_angles: int, mu: np.ndarray, mu0: float, g: float = 0.5):
     """Return (P0 (N,), P (N, N)) for name in {'iso', 'rayleigh', 'hg', 'fwc', 'mie_lognormal'}."""
     return phase_P0(name, nb_angles, mu, mu0, g), phase_P(name, nb_angles, mu, g)
+
+
+def mode_vanishes(name: str, m: int) -> bool:
+    """True when Fourier mode m of the family is identically zero: isotropic m >= 1, Rayleigh m >= 3 (0.75 (1 + cos^2 Theta)
+    is a polynomial of degree 2 in cos(phi)).  The builders return rounding-level values there; solvers use exact zeros."""
+    return m >= 1 and (name == "iso" or (name == "rayleigh" and m >= 3))
+
+
+def azimuth_nodes(n_quad: int, n_modes: int):
+    """(phi (n_quad,), table (1 + n_modes, n_quad)) of the mode builders: phi = linspace(0, pi, n_quad), table row 0 =
+    cos(0 - phi) (the node cosines of the azimuth-averaged builders), row 1 + m = cos(m phi)."""
+    phi = np.linspace(0, np.pi, int(n_quad))
+    tab = np.empty((1 + int(n_modes), phi.size))
+    tab[0] = np.cos(0 - phi)
+    tab[1:] = np.cos(np.arange(int(n_modes))[:, None] * phi[None, :])
+    return phi, tab
+
+
+def _mode_rings(f, cc, x, cm, phi):
+    """trapz over phi of cos(m phi) [f(-(cc - x)) + (-1)^m f(-(cc + x))] for every m (leading axis); mode 0 in the
+    operation order of phase_P0 / phase_P.  cc: (..., 1), x: (..., n_quad), cm: (K, n_quad)."""
+    fb, fa = f(-(cc + x)), f(-(cc - x))
+    even, odd = fb + fa, fa - fb
+    out = [_trapz(even, phi)]
+    for m in range(1, cm.shape[0]):
+        out.append(_trapz(cm[m] * (odd if m & 1 else even), phi))
+    return np.stack(out)
+
+
+def phase_modes(name: str, nb_angles: int, mu: np.ndarray, n_modes: int, g: float = 0.5, mu0=None, n_quad: int = 25,
+                want_P: bool = True):
+    """Azimuthal Fourier modes m = 0 .. n_modes-1 of a phase function: (P0_m (K, N) or None without mu0, P_m (K, N, N) or
+    None with want_P=False).
+
+    phi is the azimuth of the propagation direction of the scattered light relative to the propagation azimuth of the
+    incident light (the solar beam travels along (-mu0, 0): cos Theta = -mu0 mu + sqrt(1 - mu0^2) sqrt(1 - mu^2) cos phi;
+    phi = 0 is the forward half-plane, a sensor's relative viewing azimuth is phi + pi).  Mode m integrates the builders'
+    integrand over the n_quad nodes of [0, pi] with weight cos(m phi): trapz(cos(m phi) [f(-(cc - x)) + (-1)^m f(-(cc + x))]),
+    and every mode is normalised by the column integrals of MODE 0 (P_m[:, n] = 4 R_m[:, n] / trapz(R_0[:, n], mu),
+    P0_m = 2 P0raw_m / trapz(P0raw_0, mu)), so that sum_m (2 - delta_m0) P0_m cos(m phi) = c p(cos Theta) with one
+    constant c.  Mode 0 is phase_P0 / phase_P at n_quad = 25.  n_quad nodes resolve modes well below n_quad (mode m aliases
+    with harmonics 2 (n_quad - 1) +- m)."""
+    name, g = resolve(name, g)
+    N, K = 2 * nb_angles, int(n_modes)
+    mu = np.asarray(mu, dtype=np.float64)
+    P0 = P = None
+    if name == "iso":
+        if mu0 is not None:
+            P0 = np.zeros((K, N))
+            P0[0] = 1.0
+        if want_P:
+            P = np.zeros((K, N, N))
+            P[0] = 2.0
+        return P0, P
+    f = _kernel(name, g)
+    phi, tab = azimuth_nodes(n_quad, K)
+    cphi, cm = tab[0], tab[1:]
+    s = np.sqrt(1 - mu * mu)
+    if mu0 is not None:
+        cc = (mu * mu0)[:, None]
+        x = (np.sqrt(1 - mu0 * mu0) * s)[:, None] * cphi[None, :]
+        P0 = _mode_rings(f, cc, x, cm, phi) / (4 * np.pi)
+        P0 = P0 / _trapz(P0[0], mu) * 2
+    if want_P:
+        P = np.empty((K, N, N))
+        blk = max(1, (1 << 22) // max(1, N * phi.size))
+        for a in range(0, N, blk):
+            b = min(N, a + blk)
+            cmn = mu[:, None] * mu[None, a:b]
+            smn = s[None, a:b] * s[:, None]
+            x = smn[:, :, None] * cphi[None, None, :]
+            P[:, :, a:b] = _mode_rings(f, cmn[:, :, None], x, cm, phi) / (2 * np.pi)
+        P = 4 * P / _trapz(P[0], mu, axis=0)[None, None, :]
+    return P0, P
