@@ -48,10 +48,17 @@ typedef enum {
   SOS_SURFACE_NONE = 0,      /* single homogeneous layer: In_NumInt (SOS_Aer_I1_In.py:77-130) */
   SOS_SURFACE_SPECULAR = 1,  /* SOS_Aer_main_specular.py:397,399 */
   SOS_SURFACE_LAMBERT = 2,   /* Lambert-as-coded: SOS_Aer_main_lambertian.py:399,401 */
-  SOS_SURFACE_LAMBERT_README = 3  /* the n >= 2 Lambert coupling as the README states it (README.md:215): isotropic upward
+  SOS_SURFACE_LAMBERT_README = 3, /* the n >= 2 Lambert coupling as the README states it (README.md:215): isotropic upward
                                      radiance -2 rho int_{-1}^{0} I_n(tau*, mu') mu' dmu' > 0 over the WHOLE downward half
                                      (the shipped code has the opposite sign and drops [-h, 0]: Q5).  A separate, named
                                      physics mode: validated by invariants, not by parity with the reference. */
+  SOS_SURFACE_LAMBERT_DIFFUSE = 4  /* a Lambertian ground in every order, the direct beam included (three-region plans only;
+                                      SOS_ERR_UNSUPPORTED otherwise).  Order 1: no mirror-reflected beam; every upward column
+                                      starts at the surface row from the isotropic b = rho (e^{-T/mu0} - 2 int_{-1}^{0} I_1 mu dmu),
+                                      the reflection of the direct beam and of order 1's own downward light (a pre-pass of the
+                                      first-order entry points writes b per scenario).  Orders n >= 2: the coupling of
+                                      SOS_SURFACE_LAMBERT_README.  sos_quadratures adds no collimated reflected beam: the
+                                      reflected light is part of the diffuse field. */
 } sos_surface;
 
 /* device-side status bits (OR-ed per scenario) */

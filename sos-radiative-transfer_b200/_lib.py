@@ -70,7 +70,7 @@ class sos_result(C.Structure):
     ]
 
 
-SURFACE_NONE, SURFACE_SPECULAR, SURFACE_LAMBERT, SURFACE_LAMBERT_README = 0, 1, 2, 3
+SURFACE_NONE, SURFACE_SPECULAR, SURFACE_LAMBERT, SURFACE_LAMBERT_README, SURFACE_LAMBERT_DIFFUSE = 0, 1, 2, 3, 4
 QUERY_FUSED_ORDER, QUERY_GENERATED_SOURCE, QUERY_FOLDED, QUERY_DEVICE = 0, 1, 2, 3
 STATUS_BLEND_OVERRUN, STATUS_NONFINITE, STATUS_MAX_ORDERS = 1, 2, 4
 

@@ -2,7 +2,9 @@
 
 Every field the drivers return is the azimuth average (mode 0) of the radiance.  For a plane-parallel medium each Fourier
 mode m of the radiance obeys the same equation as mode 0 -- the same contraction J = (omega/4) int P I dmu', sweeps and
-specular mirror coupling -- with the operand P_m and the solar vector P0_m of phase.phase_modes instead of P and P0.  So a
+specular mirror coupling -- with the operand P_m and the solar vector P0_m of phase.phase_modes instead of P and P0.  A
+diffuse Lambert ground ('lambert_diffuse') is isotropic and enters mode 0 only: modes m >= 1 are solved over a black
+ground.  So a
 (geometry, mode) pair is one more member of a batch: its own operand index and first-order table row, summing exactly the
 orders its mode 0 summed (sos_scenario.order_cap), and
 
@@ -64,7 +66,8 @@ def _validate(scenarios: Sequence[Scenario], n_modes: int, n_quad: int):
     for sc in scenarios:
         if sc.surface in ("lambert", "lambert_readme") and sc.grd_alb > 0:
             # the first order reflects the beam specularly while the n >= 2 coupling is isotropic: no consistent mode split
-            raise ValueError(f"solve_azimuthal: surface {sc.surface!r} with grd_alb > 0 has no Fourier-mode decomposition")
+            raise ValueError(f"solve_azimuthal: surface {sc.surface!r} with grd_alb > 0 has no Fourier-mode decomposition; "
+                             "surface='lambert_diffuse' is a Lambertian ground in every order")
         for spec in (sc.atm_phase, sc.aer_phase):
             if not isinstance(spec[0], str):
                 raise ValueError("solve_azimuthal: modes are built from the phase function; (P0, P) arrays cannot be split")
@@ -78,8 +81,9 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
     Mode 0 is solved exactly as solve_scenarios solves it (result.base); modes 1 .. n_modes-1 of all geometries are batched
     with order_cap = the orders their mode 0 summed, so the azimuth-resolved field is the same truncated series, order for
     order, as the mode-0 field.  n_quad: azimuth nodes of the mode builder (>= 2 n_modes; 25 = the azimuth-averaged
-    builders' nodes, enough for Rayleigh and moderate HG -- sharp peaks need more).  Lambert surfaces with grd_alb > 0 and
-    caller-supplied (P0, P) arrays raise ValueError before any device work."""
+    builders' nodes, enough for Rayleigh and moderate HG -- sharp peaks need more).  A 'lambert_diffuse' ground enters mode 0
+    only (the modes m >= 1 of its geometries are solved over a black ground).  'lambert' / 'lambert_readme' surfaces with
+    grd_alb > 0 and caller-supplied (P0, P) arrays raise ValueError before any device work."""
     scenarios = list(scenarios)
     K, n_quad = int(n_modes), int(n_quad)
     _validate(scenarios, K, n_quad)
@@ -120,8 +124,10 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
                 for m in range(1, K):
                     if _vanishes(sc.atm_phase, m) and _vanishes(sc.aer_phase, m):
                         continue   # I_m = 0: nothing to solve
-                    members.append(replace(sc, atm_phase=_mode_spec(sc.atm_phase, m, n_quad),
-                                           aer_phase=_mode_spec(sc.aer_phase, m, n_quad)))
+                    mode_sc = replace(sc, atm_phase=_mode_spec(sc.atm_phase, m, n_quad), aer_phase=_mode_spec(sc.aer_phase, m, n_quad))
+                    if sc.surface == "lambert_diffuse":
+                        mode_sc = replace(mode_sc, surface="specular", grd_alb=0.0)   # an isotropic ground has no mode m >= 1
+                    members.append(mode_sc)
                     keys.append((i, m))
             for sub in split_for_plan_limits(members, range(len(members)), max_phases=MODE_PHASES_PER_PLAN):
                 caps = [n0[keys[j][0]] for j in sub]

@@ -10,8 +10,12 @@
 // -(tau_b - tau_t)/mu == (tau_t - tau_b)/mu.  The carries are the values of the same closed form at the
 // region boundary rows, so each thread first re-evaluates its column's short carry chain (<= 5 values)
 // and then fills its rows; no inter-thread dependency, one launch.
+//
+// A diffuse Lambert ground (SOS_SURFACE_LAMBERT_DIFFUSE) has no mirror term (S = 0); the carry of every upward column at
+// the surface row is the isotropic b_s of first_order_surface_kernel, a pre-pass with one CTA per scenario.
 #pragma once
 #include "common.cuh"
+#include "sweep.cuh"  // sossweep::block_sum
 
 namespace sosfirst {
 
@@ -92,7 +96,7 @@ __device__ double down_carry(const GridDev& g, const Col& c, const double* __res
 __global__ void __launch_bounds__(128)
 first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][2][N]*/, double* __restrict__ I1,
                            double* __restrict__ I1_copy /*second destination (the accumulator I of the order loop) or nullptr*/,
-                           int rows_per_block) {
+                           int rows_per_block, const double* __restrict__ bs /*[S] diffuse Lambert ground, or nullptr*/) {
   const int s = blockIdx.z;
   const int m = blockIdx.x * blockDim.x + threadIdx.x;
   const int L = g.L, M = g.M, N = g.N, ld = g.ld;
@@ -114,7 +118,7 @@ first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
   const double F0 = PI / mu0;
   const double T = sc.tauStar_tot;
   const double q = 1.0 / (4.0 * PI);
-  const double S = F0 * sc.grd_alb * exp(-T / mu0);
+  const double S = bs ? 0.0 : F0 * sc.grd_alb * exp(-T / mu0);  // the mirror-reflected beam
 
   // row-only exponentials, shared by the 128 columns of the block
   __shared__ double sh_e0[64], sh_es[64];
@@ -158,22 +162,25 @@ first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
     return;
   }
 
-  // ---- upward column: needs the mirror downward column at the surface row first ----
+  // ---- upward column: needs the mirror downward column at the surface row first (a diffuse ground: b_s) ----
   const int mir = N - 1 - m;
-  Col d;
-  d.mu0 = mu0; d.F0q = c.F0q; d.Sq = c.Sq; d.T = T;
-  d.mu = g.mu[mir];
-  d.inv_mu = 1.0 / d.mu;
-  d.down = true;
-  d.special = fabs(d.mu + mu0) < SOS_MU0_TOLERANCE;
-  d.Cm_atm = Catm[mir]; d.Cmir_atm = Catm[m];
-  d.Cm_mix = Cmix[mir]; d.Cmir_mix = Cmix[m];
   const int R = g.nreg;
-  double surf_down;
-  {
+  double surf_carry;
+  if (bs) {
+    surf_carry = bs[s];
+  } else {
+    Col d;
+    d.mu0 = mu0; d.F0q = c.F0q; d.Sq = c.Sq; d.T = T;
+    d.mu = g.mu[mir];
+    d.inv_mu = 1.0 / d.mu;
+    d.down = true;
+    d.special = fabs(d.mu + mu0) < SOS_MU0_TOLERANCE;
+    d.Cm_atm = Catm[mir]; d.Cmir_atm = Catm[m];
+    d.Cm_mix = Cmix[mir]; d.Cmir_mix = Cmix[m];
     const double tt = tau[L - 1];
-    surf_down = i1_value(d, (R - 1) == 1, tt, exp(-tt / mu0), exp(-(T - tt) / mu0), down_carry(g, d, tau, R - 1, T),
-                         down_region(g, tau, R - 1, T, mu0));
+    const double surf_down = i1_value(d, (R - 1) == 1, tt, exp(-tt / mu0), exp(-(T - tt) / mu0), down_carry(g, d, tau, R - 1, T),
+                                      down_region(g, tau, R - 1, T, mu0));
+    surf_carry = sc.grd_alb * surf_down;
   }
 
   c.mu = g.mu[m];
@@ -184,13 +191,13 @@ first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
   c.Cm_mix = Cmix[m]; c.Cmir_mix = Cmix[mir];
 
   // upward regions, bottom first:
-  //   last region : carry = rho * I1[L-1, mirror], tau_d = tau[L-1], tau_s = T                      (:206-216)
+  //   last region : carry = rho * I1[L-1, mirror] (diffuse ground: b_s), tau_d = tau[L-1], tau_s = T  (:206-216)
   //   region k    : carry = I1[rstart[k+1], m],    tau_d = tau[rstart[k+1]], tau_s = tau[rstart[k+1]-1]
   RegionK rks[3];
   double carry_k[3];
   for (int k = 0; k < R; ++k)
     rks[k] = (k == R - 1) ? region_consts(tau[L - 1], T, T, mu0) : region_consts(tau[g.rstart[k + 1]], tau[g.rstart[k + 1] - 1], T, mu0);
-  carry_k[R - 1] = sc.grd_alb * surf_down;
+  carry_k[R - 1] = surf_carry;
   for (int k = R - 2; k >= 0; --k) {
     const double tt = tau[g.rstart[k + 1]];  // first row of the region below = carry row
     carry_k[k] = i1_value(c, (k + 1) == 1, tt, exp(-tt / mu0), exp(-(T - tt) / mu0), carry_k[k + 1], rks[k + 1]);
@@ -199,6 +206,57 @@ first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
     const int k = region_of(g, t);
     put(t, m, i1_value(c, k == 1, tau[t], sh_e0[t - ta], sh_es[t - ta], carry_k[k], rks[k]));
   }
+}
+
+// Diffuse Lambert ground: b_s[s] = rho (e^{-T/mu0} - 2 trapz(I1[L-1, 0..M-1] mu, mu)), the upward radiance the ground
+// reflects of the direct beam (irradiance pi e^{-T/mu0} with F0 = pi/mu0) and of order 1's own downward light.  One CTA
+// per scenario evaluates row L-1 of the downward columns with the calls and row factors of first_order_regions_kernel
+// (S = 0), so these are the values it stores; the trapezoid is the one of the lambert_readme coupling (sweep.cuh: ascending
+// abscissa, the interval next to mu = 0- included) and is summed by the deterministic block sum.
+// Dynamic shared memory: (M + 32) doubles.
+__global__ void __launch_bounds__(128)
+first_order_surface_kernel(const GridDev g, const double* __restrict__ Cs /*[S][2][N]*/, double* __restrict__ bs) {
+  extern __shared__ double fo_row[];  // [M] row L-1 of the downward half, then [32] block_sum scratch
+  const int s = blockIdx.x;
+  const int L = g.L, M = g.M, N = g.N, R = g.nreg;
+  const double* __restrict__ tau = g.tau + static_cast<size_t>(s) * L;
+  const sos_scenario sc = g.scen[s];
+  const double* __restrict__ Catm = Cs + static_cast<size_t>(s) * 2 * N;
+  const double* __restrict__ Cmix = Catm + N;
+  const double PI = 3.14159265358979323846;
+  const double mu0 = sc.mu0;
+  const double F0 = PI / mu0;
+  const double T = sc.tauStar_tot;
+  const double q = 1.0 / (4.0 * PI);
+  const double S = 0.0;
+  const double tt = tau[L - 1];
+  const double e0 = exp(-tt / mu0), es = exp(-(T - tt) / mu0);
+  const int k = R - 1;  // region of the surface row
+  const RegionK rk = down_region(g, tau, k, T, mu0);
+  for (int m = threadIdx.x; m < M; m += blockDim.x) {
+    if (m == M - 1) {
+      const double* C = (k == 1) ? Cmix : Catm;
+      fo_row[m] = (mu0 / (mu0 + g.mu[m])) * C[m] * (F0 * q) * e0 + (mu0 / (mu0 - g.mu[m])) * C[N - 1 - m] * (S * q) * es;
+      continue;
+    }
+    Col c;
+    c.mu0 = mu0; c.F0q = F0 * q; c.Sq = S * q; c.T = T;
+    c.mu = g.mu[m];
+    c.inv_mu = 1.0 / c.mu;
+    c.down = true;
+    c.special = fabs(c.mu + mu0) < SOS_MU0_TOLERANCE;
+    c.Cm_atm = Catm[m]; c.Cmir_atm = Catm[N - 1 - m];
+    c.Cm_mix = Cmix[m]; c.Cmir_mix = Cmix[N - 1 - m];
+    fo_row[m] = i1_value(c, k == 1, tt, e0, es, down_carry(g, c, tau, k, T), rk);
+  }
+  __syncthreads();
+  double part = 0.0;
+  for (int c0 = threadIdx.x; c0 < M - 1; c0 += blockDim.x) {
+    const int c1 = c0 + 1;
+    part += (g.mu[c1] - g.mu[c0]) * (fo_row[c1] * g.mu[c1] + fo_row[c0] * g.mu[c0]) * 0.5;
+  }
+  const double down = -2.0 * sossweep::block_sum(part, fo_row + M);
+  if (threadIdx.x == 0) bs[s] = sc.grd_alb * (exp(-T / mu0) + down);
 }
 
 // I1_NumInt (SOS_Aer_I1_In.py:13-58): one homogeneous layer above a black surface

@@ -55,7 +55,9 @@ quadrature_outputs_kernel(const GridDev g, const double* __restrict__ sums, cons
   const double* q = sums + (static_cast<size_t>(s) * L + t) * 3;
   const size_t o = static_cast<size_t>(s) * L + t;
   const double dn = exp(-tau[t] / sc.mu0);
-  const double up = sc.grd_alb * exp(-(2.0 * tl - tau[t]) / sc.mu0);
+  // the collimated beam reflected by a mirror ground; a diffuse Lambert ground puts it into the field itself
+  const double alb_dir = (g.surface == SOS_SURFACE_LAMBERT_DIFFUSE) ? 0.0 : sc.grd_alb;
+  const double up = alb_dir * exp(-(2.0 * tl - tau[t]) / sc.mu0);
   if (flux_down) flux_down[o] = q[0] - (F0 * direct_scale) * dn;                 // graphe.py:157 / :77
   if (flux_up) flux_up[o] = q[1] + (F0 * direct_scale) * up;                     // graphe.py:158 / :78
   if (net_flux) net_flux[o] = (q[0] + q[1]) - F0 * dn + F0 * up;                 // graphe.py:41
@@ -65,7 +67,7 @@ quadrature_outputs_kernel(const GridDev g, const double* __restrict__ sums, cons
     const double ds = 1.0 / (4.0 * PI);
     auto total = [&](int i) {
       const double* qi = sums + (static_cast<size_t>(s) * L + i) * 3;
-      return (qi[0] - (F0 * ds) * exp(-tau[i] / sc.mu0)) + (qi[1] + (F0 * ds) * sc.grd_alb * exp(-(2.0 * tl - tau[i]) / sc.mu0));
+      return (qi[0] - (F0 * ds) * exp(-tau[i] / sc.mu0)) + (qi[1] + (F0 * ds) * alb_dir * exp(-(2.0 * tl - tau[i]) / sc.mu0));
     };
     auto hr = [&](int i) {  // i in [0, L-2]
       return -(1.0 / (1.225 * 1004.0)) * (total(i + 1) - total(i)) / (z[i + 1] - z[i]);

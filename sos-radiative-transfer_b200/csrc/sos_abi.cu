@@ -114,6 +114,7 @@ struct sos_plan {
   double* d_sums = nullptr;  // [S][L][3]
   double* d_z = nullptr;     // [L]
   double* d_colint = nullptr;  // [N] column integrals of the device phase builder
+  double* d_bs = nullptr;    // [S] upward surface radiance of order 1 over a diffuse Lambert ground (that surface only)
   int* h_poll = nullptr;     // pinned
   double* h_C[2] = {nullptr, nullptr};        // pinned staging of the first-order coefficients (sos_first_order never blocks)
   cudaEvent_t h_C_ev[2] = {nullptr, nullptr};
@@ -516,7 +517,8 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
     if (grid->region_start[k + 1] <= grid->region_start[k]) return SOS_ERR_INVALID;
   if (grid->n_regions == 3 && (grid->region_start[1] < 2 || grid->region_start[2] < grid->region_start[1] + 1))
     return SOS_ERR_INVALID;
-  if (grid->surface < 0 || grid->surface > 3) return SOS_ERR_INVALID;
+  if (grid->surface < 0 || grid->surface > 4) return SOS_ERR_INVALID;
+  if (grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE && grid->n_regions != 3) return SOS_ERR_UNSUPPORTED;
 
   int dev = 0;
   SOS_CUDA(cudaGetDevice(&dev));
@@ -669,6 +671,7 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
   TRY(dev_alloc(p, &p->d_sums, static_cast<size_t>(S) * L * 3));
   TRY(dev_alloc(p, &p->d_z, static_cast<size_t>(L)));
   TRY(dev_alloc(p, &p->d_colint, static_cast<size_t>(N)));
+  if (grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE) TRY(dev_alloc(p, &p->d_bs, static_cast<size_t>(S)));
   {
     cudaError_t e = cudaMemset(p->d_carryD, 0, nagg * sizeof(double));
     if (e == cudaSuccess) e = cudaMemset(p->d_carryU, 0, nagg * sizeof(double));
@@ -756,6 +759,9 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
     int r2 = plan_tiles(p, nullptr);  // all scenarios active
     if (r2) { sos_plan_destroy(p); return r2; }
     cudaDeviceSynchronize();
+  }
+  if (p->d_bs && (M + 32) * sizeof(double) > 48 * 1024) {
+    cudaFuncSetAttribute(sosfirst::first_order_surface_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (M + 32) * sizeof(double));
   }
   if ((N + 32 + 2 * (nch + 1)) * sizeof(double) > 48 * 1024) {
     cudaFuncSetAttribute(sossweep::sweep_carry_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
@@ -1434,8 +1440,14 @@ static int first_order_launch(sos_plan* p, double* I1_d, double* I1_copy_d, cuda
   const GridDev& g = p->dev;
   const int rows_per_block = std::min(64, std::max(8, env_int("SOS_B200_FO_ROWS", 64)));  // (the kernel stages 64 rows at most)
   dim3 grid((g.N + 127) / 128, (g.L + rows_per_block - 1) / rows_per_block, g.S);
+  if (p->d_bs) {
+    // diffuse Lambert ground: the isotropic upward radiance of order 1 at the surface row, read by every upward column
+    sosfirst::first_order_surface_kernel<<<g.S, 128, (g.M + 32) * sizeof(double), st>>>(g, p->d_C, p->d_bs);
+    int r = launch_check(p, "first_order_surface_kernel");
+    if (r) return r;
+  }
   if (g.nreg == 3)
-    sosfirst::first_order_regions_kernel<<<grid, 128, 0, st>>>(g, p->d_C, I1_d, I1_copy_d, rows_per_block);
+    sosfirst::first_order_regions_kernel<<<grid, 128, 0, st>>>(g, p->d_C, I1_d, I1_copy_d, rows_per_block, p->d_bs);
   else
     sosfirst::first_order_single_kernel<<<grid, 128, 0, st>>>(g, p->d_C, I1_d, I1_copy_d, rows_per_block);
   return launch_check(p);

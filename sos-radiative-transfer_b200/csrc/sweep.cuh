@@ -568,7 +568,7 @@ sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ 
       part += (g.mu[c1] - g.mu[c0]) * (row[c1] * g.mu[c1] + row[c0] * g.mu[c0]) * 0.5;
     }
     lambert = -2.0 * sc.grd_alb * block_sum(part, scratch);
-  } else if (g.surface == SOS_SURFACE_LAMBERT_README) {
+  } else if (g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE) {
     // README.md:215: -2 rho int_{-1}^{0} I mu dmu with the abscissa ascending and the interval next to mu = 0 included
     double part = 0.0;
     for (int c0 = threadIdx.x; c0 < M - 1; c0 += blockDim.x) {
@@ -581,7 +581,8 @@ sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ 
   for (int m = M + 1 + threadIdx.x; m < N; m += blockDim.x) {
     double seed = 0.0;
     if (g.surface == SOS_SURFACE_SPECULAR) seed = sc.grd_alb * row[N - 1 - m];
-    else if (g.surface == SOS_SURFACE_LAMBERT || g.surface == SOS_SURFACE_LAMBERT_README) seed = lambert;
+    else if (g.surface == SOS_SURFACE_LAMBERT || g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE)
+      seed = lambert;
     row[m] = seed;
   }
   __syncthreads();

@@ -45,6 +45,8 @@ class Scenario:
     aer_phase: PhaseSpec = ("hg", 0.5)
     # 'specular' | 'lambert' (Lambert-as-coded, SURVEY.md 8c "repair A") | 'lambert_readme' (the n >= 2 coupling with the
     # README's sign and integration range, README.md:215; first order as in the other two: a named physics mode, not parity)
+    # | 'lambert_diffuse' (a Lambertian ground in every order: order 1 reflects the direct beam and its own downward light
+    # isotropically, no mirror beam; n >= 2 as 'lambert_readme'; the fluxes carry no collimated reflected beam)
     surface: str = "specular"
     threshold: float = 1e-4
     max_orders: int = 10000
@@ -183,7 +185,7 @@ class BatchSolver:
         self._mat_index, self._mats, self._mat_keys = {}, [], []
         coefs = self._prepare(scenarios, order_caps)
         surface = {"specular": _lib.SURFACE_SPECULAR, "lambert": _lib.SURFACE_LAMBERT,
-                   "lambert_readme": _lib.SURFACE_LAMBERT_README}[surf]
+                   "lambert_readme": _lib.SURFACE_LAMBERT_README, "lambert_diffuse": _lib.SURFACE_LAMBERT_DIFFUSE}[surf]
         self.engine = SosEngine(self.mu, self.tau, coefs, [0, self.idx_up, self.idx_down + 1, L], surface,
                                 device=device, chunk_rows=chunk_rows, fold=fold)
         self._register_phases()
@@ -338,7 +340,8 @@ class BatchSolver:
             # TOA net flux with the F0/(4 pi) direct scaling (SOS_Aer_critical_albedo.py:377-382): same quadrature sums, direct
             # terms rescaled from F0 to F0/(4 pi) -- for the whole batch at once
             mu0 = np.array([sc.mu0 for sc in self.scenarios], dtype=np.float64)
-            alb = np.array([sc.grd_alb for sc in self.scenarios], dtype=np.float64)
+            # (a diffuse Lambert ground reflects the beam into the field: no collimated reflected term)
+            alb = np.array([0.0 if sc.surface == "lambert_diffuse" else sc.grd_alb for sc in self.scenarios], dtype=np.float64)
             k = (np.pi / mu0) * (1.0 - 1.0 / (4 * np.pi))
             t0, tl = self.tau[:, 0], self.tau[:, -1]
             fd = q["flux_down"][:, 0] + k * np.exp(-t0 / mu0)
