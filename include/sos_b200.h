@@ -58,7 +58,18 @@ typedef enum {
                                       the reflection of the direct beam and of order 1's own downward light (a pre-pass of the
                                       first-order entry points writes b per scenario).  Orders n >= 2: the coupling of
                                       SOS_SURFACE_LAMBERT_README.  sos_quadratures adds no collimated reflected beam: the
-                                      reflected light is part of the diffuse field. */
+                                      reflected light is part of the diffuse field. */,
+  SOS_SURFACE_ROSSLI = 5           /* a Ross-Li bidirectional ground (RossThick + LiSparse-Reciprocal kernels) in every order
+                                      (three-region plans only; SOS_ERR_UNSUPPORTED otherwise):
+                                      rho = f_iso + f_vol K_vol + f_geo K_geo with f_iso = sos_scenario.grd_alb.  The f_iso
+                                      part is SOS_SURFACE_LAMBERT_DIFFUSE unchanged; every upward column i adds
+                                        order 1:  sum_k f_k (e^{-T/mu0} beam_k[i] + sum_c u_c R^k[c][i])
+                                        order n:  sum_k f_k sum_c u_c R^k[c][i]
+                                      with u_c = -2 w_c mu_c I_n(tau*, mu_c) over the downward half (w = trapezoid weights
+                                      of the ascending downward half) and the mode matrices / weights / beam vectors of
+                                      sos_plan_set_brdf and sos_plan_set_brdf_scenarios (both required before a first order
+                                      or a sweep: SOS_ERR_STATE otherwise).  With f_vol = f_geo = 0 every value is bit for bit
+                                      the one of SOS_SURFACE_LAMBERT_DIFFUSE.  No collimated reflected beam in the fluxes. */
 } sos_surface;
 
 /* device-side status bits (OR-ed per scenario) */
@@ -160,6 +171,18 @@ int sos_build_phase_modes(sos_plan* plan, int family, double g, double mu0, int 
                           int n_modes, const double* tab_x_d, const double* tab_y_d, int tab_n, double* P_d, int ldp,
                           size_t mode_stride, double* P0_d, void* stream);
 
+/* Fourier modes m = 0 .. n_modes-1 of the two Ross-Li kernels on the plan's mu grid, for SOS_SURFACE_ROSSLI.
+ * R^k_m(mu, mu') = (1/pi) int_0^pi K_k(max(mu, mu_min), max(mu', mu_min), phi - pi) cos(m phi) dphi, where phi is the engine's
+ * propagation azimuth relative to the incident light's and psi = phi - pi the Ross-Li relative azimuth (hot spot at psi = 0),
+ * so that rho = R_0 + 2 sum_{m >= 1} R_m cos(m phi), the normalisation of the radiance modes.  Kernels of Lucht, Schaaf &
+ * Strahler (2000) with h/b = 2, b/r = 1; both zenith cosines clamped to mu_min (0 < mu_min < 1).  Nodes: phi_h [n_nodes]
+ * ascending on [0, pi] (2 <= n_nodes <= 1024), trapezoid rule; cos_h [1 + n_modes][n_nodes]: row 0 = cos(phi_k - pi),
+ * row 1 + m = cos(m phi_k), both computed by the host.  Writes the TRANSPOSED matrices: element (c, i) = R_m(mu_{M+1+i}, |mu_c|),
+ * c = 0 .. M-1 downward columns, i = 0 .. M-2 upward columns, at Rvol_d / Rgeo_d + m * mode_stride + c * ldr + i
+ * (ldr >= M-1, mode_stride >= M * ldr).  One thread per element evaluates both kernels once per node.  1 <= n_modes <= 64. */
+int sos_build_brdf_modes(sos_plan* plan, int n_nodes, const double* phi_h, const double* cos_h, int n_modes, double mu_min,
+                         double* Rvol_d, double* Rgeo_d, int ldr, size_t mode_stride, void* stream);
+
 /* Azimuth synthesis of Fourier-mode fields: out[geo][r][p][col] (+)= sum over s with geo_h[s] = geo of
  * w_h[s][p] * I[s][rows_h[r]][col] (col < N), the sum in ascending s (no atomics: deterministic).  I_d: a field of this plan
  * ([S*L][ld]); geo_h [S] in [0, n_geo) or -1 (member skipped); w_h [S][n_az] (1 for mode 0, 2 cos(m phi_p) for mode m, as
@@ -171,6 +194,17 @@ int sos_azimuth_synthesis(sos_plan* plan, const double* I_d, const int* geo_h, c
 
 /* Register the contraction matrices (device, [N][lda] each) the scenarios index. */
 int sos_plan_set_phase(sos_plan* plan, const double* const* A_d, int n_matrices, int lda);
+
+/* SOS_SURFACE_ROSSLI plans only (SOS_ERR_UNSUPPORTED otherwise).
+ *   sos_plan_set_brdf            register n_sets (1 .. 64) mode matrix pairs (Rvol_d[j], Rgeo_d[j]): device [M][ldr] each in
+ *                                the transposed layout of sos_build_brdf_modes (ldr >= M-1), kept alive by the caller.  Drops
+ *                                the captured order graphs; the per-scenario data must be given again afterwards.
+ *   sos_plan_set_brdf_scenarios  per scenario: set_h [S] (the pair it uses, 0 .. n_sets-1), f_h [S][2] = (f_vol, f_geo) >= 0
+ *                                and beam_h [S][2][M-1] = (R^vol_m(mu_i, mu0), R^geo_m(mu_i, mu0)) over the upward columns
+ *                                i = M+1 .. N-1 for the scenario's mode m.  Copied on `stream` into plan-owned buffers in place:
+ *                                captured order graphs stay valid, so it follows sos_plan_update for the next batch. */
+int sos_plan_set_brdf(sos_plan* plan, const double* const* Rvol_d, const double* const* Rgeo_d, int n_sets, int ldr);
+int sos_plan_set_brdf_scenarios(sos_plan* plan, const int* set_h, const double* f_h, const double* beam_h, void* stream);
 
 /* Folded contraction (optional, half the multiply-adds).  The operand A[k][m] = w_k/4 P[m][N-1-k] of
  * SOS_Aer_I1_In.py:73 is centrosymmetric (A[N-1-k][N-1-m] = A[k][m]) whenever P(mu, mu') = P(-mu, -mu') --

@@ -4,7 +4,8 @@ Every field the drivers return is the azimuth average (mode 0) of the radiance. 
 mode m of the radiance obeys the same equation as mode 0 -- the same contraction J = (omega/4) int P I dmu', sweeps and
 specular mirror coupling -- with the operand P_m and the solar vector P0_m of phase.phase_modes instead of P and P0.  A
 diffuse Lambert ground ('lambert_diffuse') is isotropic and enters mode 0 only: modes m >= 1 are solved over a black
-ground.  So a
+ground.  A Ross-Li ground ('rossli') couples mode m through its own kernel modes (brdf module): the members of mode m keep
+the surface with grd_alb = 0 (the isotropic part has no mode m >= 1) and the Ross-Li mode m.  So a
 (geometry, mode) pair is one more member of a batch: its own operand index and first-order table row, summing exactly the
 orders its mode 0 summed (sos_scenario.order_cap), and
 
@@ -26,8 +27,8 @@ import numpy as np
 import torch
 
 from . import phase as PH
-from .drivers import (DriverResult, MAX_PHASES_PER_PLAN, BatchSolver, Scenario, _MODE_STACKS, grid_groups, solved_batches,
-                      split_for_plan_limits)
+from .drivers import (DriverResult, MAX_PHASES_PER_PLAN, BatchSolver, Scenario, _BRDF_STACKS, _MODE_STACKS, check_brdf,
+                      grid_groups, solved_batches, split_for_plan_limits)
 
 # phase functions per plan of the mode members (two per mode: typically 8 modes per plan)
 MODE_PHASES_PER_PLAN = MAX_PHASES_PER_PLAN
@@ -59,6 +60,7 @@ def _vanishes(spec, m: int) -> bool:
 
 
 def _validate(scenarios: Sequence[Scenario], n_modes: int, n_quad: int):
+    check_brdf(scenarios)
     if n_modes < 1:
         raise ValueError("solve_azimuthal: n_modes must be >= 1")
     if n_quad < 2 * n_modes:
@@ -82,7 +84,8 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
     with order_cap = the orders their mode 0 summed, so the azimuth-resolved field is the same truncated series, order for
     order, as the mode-0 field.  n_quad: azimuth nodes of the mode builder (>= 2 n_modes; 25 = the azimuth-averaged
     builders' nodes, enough for Rayleigh and moderate HG -- sharp peaks need more).  A 'lambert_diffuse' ground enters mode 0
-    only (the modes m >= 1 of its geometries are solved over a black ground).  'lambert' / 'lambert_readme' surfaces with
+    only (the modes m >= 1 of its geometries are solved over a black ground); a 'rossli' ground enters every mode through
+    its kernel modes, which are integrated on brdf.BRDF_NODES nodes whatever n_quad.  'lambert' / 'lambert_readme' surfaces with
     grd_alb > 0 and caller-supplied (P0, P) arrays raise ValueError before any device work."""
     scenarios = list(scenarios)
     K, n_quad = int(n_modes), int(n_quad)
@@ -122,16 +125,21 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
             for i in group:
                 sc = scenarios[i]
                 for m in range(1, K):
-                    if _vanishes(sc.atm_phase, m) and _vanishes(sc.aer_phase, m):
-                        continue   # I_m = 0: nothing to solve
+                    brdf = sc.surface == "rossli" and (sc.brdf_vol != 0 or sc.brdf_geo != 0)
+                    if _vanishes(sc.atm_phase, m) and _vanishes(sc.aer_phase, m) and not brdf:
+                        continue   # I_m = 0: nothing to solve (a Ross-Li ground reflects mode m of the beam itself)
                     mode_sc = replace(sc, atm_phase=_mode_spec(sc.atm_phase, m, n_quad), aer_phase=_mode_spec(sc.aer_phase, m, n_quad))
                     if sc.surface == "lambert_diffuse":
                         mode_sc = replace(mode_sc, surface="specular", grd_alb=0.0)   # an isotropic ground has no mode m >= 1
+                    elif sc.surface == "rossli":
+                        mode_sc = replace(mode_sc, grd_alb=0.0)   # the kernels' mode m (BatchSolver brdf_modes below)
                     members.append(mode_sc)
                     keys.append((i, m))
             for sub in split_for_plan_limits(members, range(len(members)), max_phases=MODE_PHASES_PER_PLAN):
                 caps = [n0[keys[j][0]] for j in sub]
-                bs = BatchSolver([members[j] for j in sub], device=device, order_caps=caps)
+                rossli = members[sub[0]].surface == "rossli"
+                bs = BatchSolver([members[j] for j in sub], device=device, order_caps=caps,
+                                 brdf_modes=[keys[j][1] for j in sub] if rossli else None)
                 try:
                     res = bs.solve(max_orders=max(caps))
                     eng = bs.engine
@@ -151,4 +159,5 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
                                          modes=modes[i], mode_orders=orders[i], mode_status=status[i])
     finally:
         _MODE_STACKS.clear()   # the device mode stacks serve the sub-batches of one call
+        _BRDF_STACKS.clear()
     return out  # type: ignore

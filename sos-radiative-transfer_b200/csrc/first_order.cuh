@@ -12,7 +12,9 @@
 // and then fills its rows; no inter-thread dependency, one launch.
 //
 // A diffuse Lambert ground (SOS_SURFACE_LAMBERT_DIFFUSE) has no mirror term (S = 0); the carry of every upward column at
-// the surface row is the isotropic b_s of first_order_surface_kernel, a pre-pass with one CTA per scenario.
+// the surface row is the isotropic b_s of first_order_surface_kernel, a pre-pass with one CTA per scenario.  A Ross-Li
+// ground (SOS_SURFACE_ROSSLI) has one such carry per upward column: b_s plus the reflection of the beam and of order 1's
+// downward light by the two kernels (brdf.cuh).
 #pragma once
 #include "common.cuh"
 #include "sweep.cuh"  // sossweep::block_sum
@@ -93,10 +95,13 @@ __device__ double down_carry(const GridDev& g, const Col& c, const double* __res
   return carry;
 }
 
+// PER_COLUMN: bs holds one surface carry per upward column, [S][M-1] (Ross-Li ground); otherwise one per scenario, [S]
+// (diffuse Lambert ground), or bs is nullptr (mirror coupling).  Separate instantiations: the others compile as without it.
+template <bool PER_COLUMN>
 __global__ void __launch_bounds__(128)
 first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][2][N]*/, double* __restrict__ I1,
                            double* __restrict__ I1_copy /*second destination (the accumulator I of the order loop) or nullptr*/,
-                           int rows_per_block, const double* __restrict__ bs /*[S] diffuse Lambert ground, or nullptr*/) {
+                           int rows_per_block, const double* __restrict__ bs /*diffuse ground, or nullptr*/) {
   const int s = blockIdx.z;
   const int m = blockIdx.x * blockDim.x + threadIdx.x;
   const int L = g.L, M = g.M, N = g.N, ld = g.ld;
@@ -167,7 +172,7 @@ first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
   const int R = g.nreg;
   double surf_carry;
   if (bs) {
-    surf_carry = bs[s];
+    surf_carry = PER_COLUMN ? bs[static_cast<size_t>(s) * (M - 1) + (m - M - 1)] : bs[s];
   } else {
     Col d;
     d.mu0 = mu0; d.F0q = c.F0q; d.Sq = c.Sq; d.T = T;
@@ -213,9 +218,12 @@ first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
 // per scenario evaluates row L-1 of the downward columns with the calls and row factors of first_order_regions_kernel
 // (S = 0), so these are the values it stores; the trapezoid is the one of the lambert_readme coupling (sweep.cuh: ascending
 // abscissa, the interval next to mu = 0- included) and is summed by the deterministic block sum.
+// Ross-Li ground (brdf.f != nullptr): bs[s][i] = b_s + sum_k f_k (e^{-T/mu0} beam_k[i] + sum_c u_c R^k[c][i]) for the upward
+// columns i = 0 .. M-2, u_c = -2 w_c mu_c I1[L-1, c] (sosbrdf::coupling_weight); with grd_alb = f_iso, b_s is the term above.
 // Dynamic shared memory: (M + 32) doubles.
 __global__ void __launch_bounds__(128)
-first_order_surface_kernel(const GridDev g, const double* __restrict__ Cs /*[S][2][N]*/, double* __restrict__ bs) {
+first_order_surface_kernel(const GridDev g, const double* __restrict__ Cs /*[S][2][N]*/, double* __restrict__ bs,
+                           const sosbrdf::BrdfDev brdf) {
   extern __shared__ double fo_row[];  // [M] row L-1 of the downward half, then [32] block_sum scratch
   const int s = blockIdx.x;
   const int L = g.L, M = g.M, N = g.N, R = g.nreg;
@@ -256,7 +264,21 @@ first_order_surface_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
     part += (g.mu[c1] - g.mu[c0]) * (fo_row[c1] * g.mu[c1] + fo_row[c0] * g.mu[c0]) * 0.5;
   }
   const double down = -2.0 * sossweep::block_sum(part, fo_row + M);
-  if (threadIdx.x == 0) bs[s] = sc.grd_alb * (exp(-T / mu0) + down);
+  const double b_s = sc.grd_alb * (exp(-T / mu0) + down);
+  if (!brdf.f) {
+    if (threadIdx.x == 0) bs[s] = b_s;
+    return;
+  }
+  for (int c = threadIdx.x; c < M; c += blockDim.x) fo_row[c] *= sosbrdf::coupling_weight(g.mu, M, c);   // (block_sum synced)
+  __syncthreads();
+  const double E = exp(-T / mu0), fv = brdf.f[2 * s], fg = brdf.f[2 * s + 1];
+  const double* __restrict__ bv = brdf.beam + static_cast<size_t>(s) * 2 * (M - 1);
+  const double* __restrict__ bg = bv + (M - 1);
+  for (int i = threadIdx.x; i < M - 1; i += blockDim.x) {
+    double sv, sgeo;
+    sosbrdf::coupling(brdf, s, fo_row, M, i, sv, sgeo);
+    bs[static_cast<size_t>(s) * (M - 1) + i] = b_s + (fv * (E * bv[i] + sv) + fg * (E * bg[i] + sgeo));
+  }
 }
 
 // I1_NumInt (SOS_Aer_I1_In.py:13-58): one homogeneous layer above a black surface

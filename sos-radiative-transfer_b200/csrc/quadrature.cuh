@@ -55,8 +55,8 @@ quadrature_outputs_kernel(const GridDev g, const double* __restrict__ sums, cons
   const double* q = sums + (static_cast<size_t>(s) * L + t) * 3;
   const size_t o = static_cast<size_t>(s) * L + t;
   const double dn = exp(-tau[t] / sc.mu0);
-  // the collimated beam reflected by a mirror ground; a diffuse Lambert ground puts it into the field itself
-  const double alb_dir = (g.surface == SOS_SURFACE_LAMBERT_DIFFUSE) ? 0.0 : sc.grd_alb;
+  // the collimated beam reflected by a mirror ground; a diffuse Lambert or Ross-Li ground puts it into the field itself
+  const double alb_dir = (g.surface == SOS_SURFACE_LAMBERT_DIFFUSE || g.surface == SOS_SURFACE_ROSSLI) ? 0.0 : sc.grd_alb;
   const double up = alb_dir * exp(-(2.0 * tl - tau[t]) / sc.mu0);
   if (flux_down) flux_down[o] = q[0] - (F0 * direct_scale) * dn;                 // graphe.py:157 / :77
   if (flux_up) flux_up[o] = q[1] + (F0 * direct_scale) * up;                     // graphe.py:158 / :78

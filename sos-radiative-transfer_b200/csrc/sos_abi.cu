@@ -114,7 +114,12 @@ struct sos_plan {
   double* d_sums = nullptr;  // [S][L][3]
   double* d_z = nullptr;     // [L]
   double* d_colint = nullptr;  // [N] column integrals of the device phase builder
-  double* d_bs = nullptr;    // [S] upward surface radiance of order 1 over a diffuse Lambert ground (that surface only)
+  double* d_bs = nullptr;    // upward surface radiance of order 1: [S] over a diffuse Lambert ground, [S][M-1] over a Ross-Li one
+  // Ross-Li ground (that surface only): the registered mode matrix pairs and the per-scenario data of sosbrdf::BrdfDev
+  const double** d_brdf_R = nullptr;  // [MAX_SETS][2]
+  char* d_brdf_scen = nullptr;        // [S][2] f | [S][2][M-1] beam | [S] set (int)
+  int brdf_sets = 0, brdf_ldr = 0;
+  bool brdf_scen_ready = false;
   int* h_poll = nullptr;     // pinned
   double* h_C[2] = {nullptr, nullptr};        // pinned staging of the first-order coefficients (sos_first_order never blocks)
   cudaEvent_t h_C_ev[2] = {nullptr, nullptr};
@@ -365,6 +370,28 @@ void drop_graphs(sos_plan* p) {
 // ---------------------------------------------------------------------------------------------
 // generated source (sweep.cuh: SrcGen): plan-side buffers
 // ---------------------------------------------------------------------------------------------
+// Ross-Li ground: layout of the per-scenario buffer and the view the kernels take of it
+size_t brdf_scen_bytes(int S, int M) {
+  return static_cast<size_t>(S) * (2 + 2 * (M - 1)) * sizeof(double) + static_cast<size_t>(S) * sizeof(int);
+}
+
+sosbrdf::BrdfDev brdf_dev(const sos_plan* p) {
+  sosbrdf::BrdfDev b;
+  std::memset(&b, 0, sizeof(b));
+  if (!p->d_brdf_R) return b;
+  const int S = p->dev.S, M = p->dev.M;
+  const double* f = reinterpret_cast<const double*>(p->d_brdf_scen);
+  b.R = p->d_brdf_R;
+  b.f = f;
+  b.beam = f + 2 * static_cast<size_t>(S);
+  b.set = reinterpret_cast<const int*>(f + static_cast<size_t>(S) * (2 + 2 * (M - 1)));
+  b.ldr = p->brdf_ldr;
+  return b;
+}
+
+// a Ross-Li plan needs its mode matrices and per-scenario data before any first order or sweep
+bool brdf_missing(const sos_plan* p) { return p->d_brdf_R && !(p->brdf_sets > 0 && p->brdf_scen_ready); }
+
 int env_int(const char* name, int dflt) {
   const char* e = std::getenv(name);
   return (e && *e) ? std::atoi(e) : dflt;
@@ -517,8 +544,9 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
     if (grid->region_start[k + 1] <= grid->region_start[k]) return SOS_ERR_INVALID;
   if (grid->n_regions == 3 && (grid->region_start[1] < 2 || grid->region_start[2] < grid->region_start[1] + 1))
     return SOS_ERR_INVALID;
-  if (grid->surface < 0 || grid->surface > 4) return SOS_ERR_INVALID;
-  if (grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE && grid->n_regions != 3) return SOS_ERR_UNSUPPORTED;
+  if (grid->surface < 0 || grid->surface > 5) return SOS_ERR_INVALID;
+  if ((grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE || grid->surface == SOS_SURFACE_ROSSLI) && grid->n_regions != 3)
+    return SOS_ERR_UNSUPPORTED;
 
   int dev = 0;
   SOS_CUDA(cudaGetDevice(&dev));
@@ -672,6 +700,11 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
   TRY(dev_alloc(p, &p->d_z, static_cast<size_t>(L)));
   TRY(dev_alloc(p, &p->d_colint, static_cast<size_t>(N)));
   if (grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE) TRY(dev_alloc(p, &p->d_bs, static_cast<size_t>(S)));
+  if (grid->surface == SOS_SURFACE_ROSSLI) {
+    TRY(dev_alloc(p, &p->d_bs, static_cast<size_t>(S) * (M - 1)));
+    TRY(dev_alloc(p, &p->d_brdf_R, static_cast<size_t>(2) * sosbrdf::MAX_SETS));
+    TRY(dev_alloc(p, &p->d_brdf_scen, brdf_scen_bytes(S, M)));
+  }
   {
     cudaError_t e = cudaMemset(p->d_carryD, 0, nagg * sizeof(double));
     if (e == cudaSuccess) e = cudaMemset(p->d_carryU, 0, nagg * sizeof(double));
@@ -764,7 +797,8 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
     cudaFuncSetAttribute(sosfirst::first_order_surface_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (M + 32) * sizeof(double));
   }
   if ((N + 32 + 2 * (nch + 1)) * sizeof(double) > 48 * 1024) {
-    cudaFuncSetAttribute(sossweep::sweep_carry_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
+    cudaFuncSetAttribute(sossweep::sweep_carry_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
+    cudaFuncSetAttribute(sossweep::sweep_carry_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
   }
   {
     int r3 = gen_setup(p, p->scen_h.data());
@@ -1171,6 +1205,80 @@ int sos_plan_set_phase(sos_plan* p, const double* const* A_d, int n, int lda) {
   return SOS_OK;
 }
 
+int sos_build_brdf_modes(sos_plan* p, int n_nodes, const double* phi_h, const double* cos_h, int n_modes, double mu_min,
+                         double* Rvol_d, double* Rgeo_d, int ldr, size_t mode_stride, void* stream) {
+  if (!p || !phi_h || !cos_h || !Rvol_d || !Rgeo_d) return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  const int M = p->dev.M;
+  if (n_nodes < 2 || n_nodes > sosbrdf::MAX_NODES || n_modes < 1 || n_modes > sosbrdf::MAX_MODES) return SOS_ERR_INVALID;
+  if (!(mu_min > 0.0 && mu_min < 1.0) || M < 2 || ldr < M - 1 || (n_modes > 1 && mode_stride < static_cast<size_t>(M) * ldr))
+    return SOS_ERR_INVALID;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // node table [cos(phi_k - pi) | trapezoid weight * cos(m phi_k) / pi] computed here from what the host passed
+  const double PI = 3.14159265358979323846;
+  std::vector<double> tab(static_cast<size_t>(n_nodes) * (1 + n_modes), 0.0);
+  double* cpsi = tab.data();
+  double* wcos = cpsi + n_nodes;
+  for (int k = 0; k < n_nodes; ++k) {
+    cpsi[k] = cos_h[k];
+    const double tw = 0.5 * ((k + 1 < n_nodes ? phi_h[k + 1] : phi_h[k]) - (k > 0 ? phi_h[k - 1] : phi_h[k]));
+    for (int m = 0; m < n_modes; ++m) wcos[static_cast<size_t>(k) * n_modes + m] = tw * cos_h[static_cast<size_t>(1 + m) * n_nodes + k] / PI;
+  }
+  double* tab_d = nullptr;
+  SOS_CUDA(cudaMallocAsync(&tab_d, tab.size() * sizeof(double), st));
+  SOS_CUDA(cudaMemcpyAsync(tab_d, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  const size_t smem = static_cast<size_t>(2 * n_modes) * sosbrdf::BUILD_THREADS * sizeof(double);
+  cudaFuncSetAttribute(sosbrdf::brdf_modes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+  const long long n_el = static_cast<long long>(M) * (M - 1);
+  sosbrdf::brdf_modes_kernel<<<static_cast<unsigned>((n_el + sosbrdf::BUILD_THREADS - 1) / sosbrdf::BUILD_THREADS), sosbrdf::BUILD_THREADS,
+                               smem, st>>>(p->dev.mu, M, mu_min, tab_d, tab_d + n_nodes, n_nodes, n_modes, Rvol_d, Rgeo_d, ldr, mode_stride);
+  const int r = launch_check(p, "brdf_modes_kernel");
+  SOS_CUDA(cudaFreeAsync(tab_d, st));
+  return r;
+}
+
+int sos_plan_set_brdf(sos_plan* p, const double* const* Rvol_d, const double* const* Rgeo_d, int n_sets, int ldr) {
+  if (!p || !Rvol_d || !Rgeo_d) return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  if (!p->d_brdf_R) return SOS_ERR_UNSUPPORTED;
+  if (n_sets < 1 || n_sets > sosbrdf::MAX_SETS || ldr < p->dev.M - 1) return SOS_ERR_INVALID;
+  std::vector<const double*> ptrs(2 * static_cast<size_t>(n_sets));
+  for (int j = 0; j < n_sets; ++j) {
+    if (!Rvol_d[j] || !Rgeo_d[j]) return SOS_ERR_INVALID;
+    ptrs[2 * j] = Rvol_d[j];
+    ptrs[2 * j + 1] = Rgeo_d[j];
+  }
+  drop_graphs(p);
+  SOS_CUDA(cudaMemcpy(p->d_brdf_R, ptrs.data(), ptrs.size() * sizeof(const double*), cudaMemcpyHostToDevice));
+  p->brdf_sets = n_sets;
+  p->brdf_ldr = ldr;
+  p->brdf_scen_ready = false;   // the set indices refer to the previous registration
+  return SOS_OK;
+}
+
+int sos_plan_set_brdf_scenarios(sos_plan* p, const int* set_h, const double* f_h, const double* beam_h, void* stream) {
+  if (!p || !set_h || !f_h || !beam_h) return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  if (!p->d_brdf_R) return SOS_ERR_UNSUPPORTED;
+  if (p->brdf_sets < 1) return SOS_ERR_STATE;
+  const int S = p->dev.S, M = p->dev.M;
+  for (int s = 0; s < S; ++s) {
+    if (set_h[s] < 0 || set_h[s] >= p->brdf_sets) return SOS_ERR_INVALID;
+    if (!(f_h[2 * s] >= 0.0 && f_h[2 * s + 1] >= 0.0) || !std::isfinite(f_h[2 * s]) || !std::isfinite(f_h[2 * s + 1])) return SOS_ERR_INVALID;
+  }
+  const size_t nf = 2 * static_cast<size_t>(S), nb = nf * (M - 1);
+  for (size_t k = 0; k < nb; ++k)
+    if (!std::isfinite(beam_h[k])) return SOS_ERR_INVALID;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  double* d = reinterpret_cast<double*>(p->d_brdf_scen);
+  SOS_CUDA(cudaMemcpyAsync(d, f_h, nf * sizeof(double), cudaMemcpyHostToDevice, st));
+  SOS_CUDA(cudaMemcpyAsync(d + nf, beam_h, nb * sizeof(double), cudaMemcpyHostToDevice, st));
+  SOS_CUDA(cudaMemcpyAsync(d + nf + nb, set_h, S * sizeof(int), cudaMemcpyHostToDevice, st));
+  SOS_CUDA(cudaStreamSynchronize(st));   // (the host arrays may be pageable and are the caller's after this call)
+  p->brdf_scen_ready = true;
+  return SOS_OK;
+}
+
 int sos_fold_layout(int nb_angles, int* rows, int* ld) {
   const int Mh = (nb_angles + 15) / 16 * 16;
   if (rows) *rows = Mh;       // k rows, padded to the k-step
@@ -1438,16 +1546,19 @@ static int first_order_stage(sos_plan* p, double** buf, cudaEvent_t* ev) {
 
 static int first_order_launch(sos_plan* p, double* I1_d, double* I1_copy_d, cudaStream_t st) {
   const GridDev& g = p->dev;
+  if (brdf_missing(p)) return SOS_ERR_STATE;
   const int rows_per_block = std::min(64, std::max(8, env_int("SOS_B200_FO_ROWS", 64)));  // (the kernel stages 64 rows at most)
   dim3 grid((g.N + 127) / 128, (g.L + rows_per_block - 1) / rows_per_block, g.S);
   if (p->d_bs) {
-    // diffuse Lambert ground: the isotropic upward radiance of order 1 at the surface row, read by every upward column
-    sosfirst::first_order_surface_kernel<<<g.S, 128, (g.M + 32) * sizeof(double), st>>>(g, p->d_C, p->d_bs);
+    // diffuse Lambert / Ross-Li ground: the upward radiance of order 1 at the surface row, read by the upward columns
+    sosfirst::first_order_surface_kernel<<<g.S, 128, (g.M + 32) * sizeof(double), st>>>(g, p->d_C, p->d_bs, brdf_dev(p));
     int r = launch_check(p, "first_order_surface_kernel");
     if (r) return r;
   }
-  if (g.nreg == 3)
-    sosfirst::first_order_regions_kernel<<<grid, 128, 0, st>>>(g, p->d_C, I1_d, I1_copy_d, rows_per_block, p->d_bs);
+  if (g.nreg == 3 && p->d_brdf_R)
+    sosfirst::first_order_regions_kernel<true><<<grid, 128, 0, st>>>(g, p->d_C, I1_d, I1_copy_d, rows_per_block, p->d_bs);
+  else if (g.nreg == 3)
+    sosfirst::first_order_regions_kernel<false><<<grid, 128, 0, st>>>(g, p->d_C, I1_d, I1_copy_d, rows_per_block, p->d_bs);
   else
     sosfirst::first_order_single_kernel<<<grid, 128, 0, st>>>(g, p->d_C, I1_d, I1_copy_d, rows_per_block);
   return launch_check(p);
@@ -1759,6 +1870,7 @@ static int sweeps_impl(sos_plan* p, const double* J_d, double* In_d, double* I_d
   const int T = sossweep::LOCAL_THREADS;
   dim3 cgrid((g.M - 1 + T - 1) / T + (g.N - g.M - 1 + T - 1) / T, g.c_hi - g.c_lo, g.S);
   const bool layered = p->layers.n > 1;
+  if (brdf_missing(p)) return SOS_ERR_STATE;
   if (layered && !in_order_loop) return SOS_ERR_UNSUPPORTED;  // sharded plans run whole orders only (sos_solve): the exchange ends in order_end_kernel
   if (layered && In_d != p->layers.In[p->layers.rank]) return SOS_ERR_INVALID;  // the neighbours write their halo rows into the registered field
   {
@@ -1778,7 +1890,12 @@ static int sweeps_impl(sos_plan* p, const double* J_d, double* In_d, double* I_d
     if (r) return r;
   } else {
     const size_t smem = (g.N + 32 + 2 * (g.nchunks + 1)) * sizeof(double);
-    sossweep::sweep_carry_kernel<<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD, p->d_carryU);
+    if (p->d_brdf_R)
+      sossweep::sweep_carry_kernel<true><<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD,
+                                                                                     p->d_carryU, brdf_dev(p));
+    else
+      sossweep::sweep_carry_kernel<false><<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD,
+                                                                                      p->d_carryU, sosbrdf::BrdfDev{});
     int r = launch_check(p, "sweep_carry_kernel");
     if (r) return r;
   }
@@ -1935,7 +2052,7 @@ int sos_solve(sos_plan* p, double* I_d, double* In_d, double* J_d, double* order
   if (!p || !I_d || !In_d || !J_d) return SOS_ERR_INVALID;
   SOS_GUARD(p);
   NvtxRange nvtx("sos:solve");
-  if (!p->maps_A_ready) return SOS_ERR_STATE;
+  if (!p->maps_A_ready || brdf_missing(p)) return SOS_ERR_STATE;
   if (poll_every < 1) poll_every = 1;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const GridDev& g = p->dev;

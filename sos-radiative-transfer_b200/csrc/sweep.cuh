@@ -33,6 +33,7 @@
 // local pass of those rows reads nothing at all.
 #pragma once
 #include <type_traits>
+#include "brdf.cuh"
 #include "common.cuh"
 #include "layer_shard.cuh"
 
@@ -494,9 +495,13 @@ __device__ __forceinline__ double block_sum(double v, double* scratch /*[32]*/) 
 // ------------------------------------------------------------------------------------------
 // 2. carry chain (one CTA per scenario)
 // ------------------------------------------------------------------------------------------
+// BRDF = true: the Ross-Li ground (SOS_SURFACE_ROSSLI, brdf.cuh), the lambert_readme term with grd_alb = f_iso plus the two
+// kernel mat-vecs; a separate instantiation, so that the kernel of the other surfaces is compiled as without it.
+template <bool BRDF>
 __global__ void __launch_bounds__(CARRY_THREADS)
 sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ J, const double* __restrict__ aggD,
-                   const double* __restrict__ aggU, double* __restrict__ carryD, double* __restrict__ carryU) {
+                   const double* __restrict__ aggU, double* __restrict__ carryD, double* __restrict__ carryU,
+                   const sosbrdf::BrdfDev brdf) {
   extern __shared__ double sm_row[];  // [N] + scratch[32] + tau at the chunk boundaries: [nch + 1] (down), [nch + 1] (up)
   __shared__ int found;
   const int s = blockIdx.x;
@@ -568,7 +573,7 @@ sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ 
       part += (g.mu[c1] - g.mu[c0]) * (row[c1] * g.mu[c1] + row[c0] * g.mu[c0]) * 0.5;
     }
     lambert = -2.0 * sc.grd_alb * block_sum(part, scratch);
-  } else if (g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE) {
+  } else if (BRDF || g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE) {
     // README.md:215: -2 rho int_{-1}^{0} I mu dmu with the abscissa ascending and the interval next to mu = 0 included
     double part = 0.0;
     for (int c0 = threadIdx.x; c0 < M - 1; c0 += blockDim.x) {
@@ -578,12 +583,25 @@ sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ 
     lambert = -2.0 * sc.grd_alb * block_sum(part, scratch);
   }
   // seeds into the upper half of the row buffer
-  for (int m = M + 1 + threadIdx.x; m < N; m += blockDim.x) {
-    double seed = 0.0;
-    if (g.surface == SOS_SURFACE_SPECULAR) seed = sc.grd_alb * row[N - 1 - m];
-    else if (g.surface == SOS_SURFACE_LAMBERT || g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE)
-      seed = lambert;
-    row[m] = seed;
+  if constexpr (BRDF) {
+    // the downward half becomes u_c = -2 w_c mu_c I[L-1, c] in place (the up chain reads row[M ..] only); every upward
+    // column adds f_vol sum_c u_c R^vol[c][i] + f_geo sum_c u_c R^geo[c][i] to the isotropic term
+    for (int c = threadIdx.x; c < M; c += blockDim.x) row[c] *= sosbrdf::coupling_weight(g.mu, M, c);
+    __syncthreads();
+    const double fv = brdf.f[2 * s], fg = brdf.f[2 * s + 1];
+    for (int m = M + 1 + threadIdx.x; m < N; m += blockDim.x) {
+      double sv, sgeo;
+      sosbrdf::coupling(brdf, s, row, M, m - M - 1, sv, sgeo);
+      row[m] = lambert + (fv * sv + fg * sgeo);
+    }
+  } else {
+    for (int m = M + 1 + threadIdx.x; m < N; m += blockDim.x) {
+      double seed = 0.0;
+      if (g.surface == SOS_SURFACE_SPECULAR) seed = sc.grd_alb * row[N - 1 - m];
+      else if (g.surface == SOS_SURFACE_LAMBERT || g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE)
+        seed = lambert;
+      row[m] = seed;
+    }
   }
   __syncthreads();
 

@@ -16,6 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from . import brdf as BR
 from . import grid as G
 from . import phase as PH
 from .engine import ScenarioCoefficients, SosEngine
@@ -47,9 +48,13 @@ class Scenario:
     # README's sign and integration range, README.md:215; first order as in the other two: a named physics mode, not parity)
     # | 'lambert_diffuse' (a Lambertian ground in every order: order 1 reflects the direct beam and its own downward light
     # isotropically, no mirror beam; n >= 2 as 'lambert_readme'; the fluxes carry no collimated reflected beam)
+    # | 'rossli' (a Ross-Li bidirectional ground in every order, brdf module: grd_alb is f_iso and the 'lambert_diffuse'
+    # coupling, brdf_vol / brdf_geo weight the RossThick / LiSparse-R kernels; no collimated reflected beam)
     surface: str = "specular"
     threshold: float = 1e-4
     max_orders: int = 10000
+    brdf_vol: float = 0.0   # Ross-Li kernel weights f_vol, f_geo (>= 0; surface='rossli' only)
+    brdf_geo: float = 0.0
 
 
 # README scenarios (README.md:95-111) -- tau_atm 0.124, omega_aer 0.97, R_s 0.15
@@ -113,6 +118,21 @@ def _host_mode(name, g, M, mu, mode, mu0=None):
 
 _PHASES = PhaseCache()
 _MODE_STACKS = {}   # device-built mode stacks (P_0 .. P_{K-1}) per (family, g, grid, n_quad, device), see _DeviceBuilt
+_BRDF_STACKS = {}   # device-built Ross-Li mode matrices (2, K, M, ldr) per (grid, device), see BatchSolver._send_brdf
+_BRDF_BEAMS = {}    # host beam vectors (2, K, M-1) per (grid, mu0, K)
+# surfaces that reflect the direct beam into the diffuse field: the fluxes carry no collimated reflected beam
+DIFFUSE_GROUNDS = ("lambert_diffuse", "rossli")
+
+
+def check_brdf(scenarios: Sequence[Scenario]):
+    """ValueError for Ross-Li weights that are negative (or not finite) or given on a surface other than 'rossli'."""
+    for sc in scenarios:
+        fv, fg = float(sc.brdf_vol), float(sc.brdf_geo)
+        if not (np.isfinite(fv) and np.isfinite(fg) and fv >= 0 and fg >= 0):
+            raise ValueError(f"Ross-Li kernel weights must be finite and >= 0 (brdf_vol={fv}, brdf_geo={fg})")
+        if sc.surface != "rossli" and (fv != 0 or fg != 0):
+            raise ValueError(f"brdf_vol / brdf_geo weight the Ross-Li kernels: surface={sc.surface!r} takes none "
+                             "(use surface='rossli')")
 
 
 def clear_caches(disk: bool = False):
@@ -124,7 +144,7 @@ def clear_caches(disk: bool = False):
     _PHASES._P.clear()
     _PHASES._P0.clear()
     api.clear_cache()
-    for d in (E._OPERANDS, E._FOLDED, E._LOWRANK):
+    for d in (E._OPERANDS, E._FOLDED, E._LOWRANK, _BRDF_STACKS, _BRDF_BEAMS):
         d.clear()
     mie.lognormal_table.cache_clear()
     if disk:
@@ -169,9 +189,12 @@ class BatchSolver:
     """All scenarios of one group (same L, M, aerosol rows, surface) on one device."""
 
     def __init__(self, scenarios: Sequence[Scenario], device=None, chunk_rows: int = 0, phases: Optional[PhaseCache] = None,
-                 device_phase: bool = True, fold: Optional[bool] = None, order_caps: Optional[Sequence[int]] = None):
+                 device_phase: bool = True, fold: Optional[bool] = None, order_caps: Optional[Sequence[int]] = None,
+                 brdf_modes: Optional[Sequence[int]] = None):
         """order_caps: per scenario, sum exactly orders 1 .. cap instead of stopping on the threshold (0 = the threshold;
-        sos_scenario.order_cap); None = all 0.  update() takes the caps of the next batch the same way."""
+        sos_scenario.order_cap); None = all 0.  brdf_modes (surface 'rossli'): per scenario, the azimuthal Fourier mode of
+        the Ross-Li ground it is coupled with (0 .. 63; None = all 0, the azimuth average).  update() takes both for the
+        next batch the same way."""
         keys = {_group_key(s) for s in scenarios}
         if len(keys) != 1:
             raise ValueError("BatchSolver: scenarios must share nb_layers, nb_angles, aerosol rows and surface")
@@ -185,16 +208,53 @@ class BatchSolver:
         self._mat_index, self._mats, self._mat_keys = {}, [], []
         coefs = self._prepare(scenarios, order_caps)
         surface = {"specular": _lib.SURFACE_SPECULAR, "lambert": _lib.SURFACE_LAMBERT,
-                   "lambert_readme": _lib.SURFACE_LAMBERT_README, "lambert_diffuse": _lib.SURFACE_LAMBERT_DIFFUSE}[surf]
+                   "lambert_readme": _lib.SURFACE_LAMBERT_README, "lambert_diffuse": _lib.SURFACE_LAMBERT_DIFFUSE,
+                   "rossli": _lib.SURFACE_ROSSLI}[surf]
         self.engine = SosEngine(self.mu, self.tau, coefs, [0, self.idx_up, self.idx_down + 1, L], surface,
                                 device=device, chunk_rows=chunk_rows, fold=fold)
         self._register_phases()
+        self._brdf_sets = None
+        if surf == "rossli":
+            self._send_brdf(brdf_modes)
         self.I1 = None
+
+    def _send_brdf(self, brdf_modes):
+        """Ross-Li plan: register the mode matrix pairs the batch uses (when they change) and send every scenario's pair
+        index, weights and beam vectors."""
+        S, M = len(self.scenarios), self.M
+        modes = np.zeros(S, dtype=np.int64) if brdf_modes is None else np.asarray(brdf_modes, dtype=np.int64)
+        if modes.shape != (S,) or np.any(modes < 0) or np.any(modes >= 64):
+            raise ValueError("BatchSolver: brdf_modes must give one mode in [0, 64) per scenario")
+        wanted = sorted(set(modes.tolist()))
+        K = wanted[-1] + 1
+        eng = self.engine
+        if self._brdf_sets is None or not set(wanted) <= set(self._brdf_sets):
+            key = (eng.mu.tobytes(), eng.device.index)
+            stack = _BRDF_STACKS.get(key)
+            if stack is None or stack.shape[1] < K:
+                if len(_BRDF_STACKS) >= 4:
+                    _BRDF_STACKS.pop(next(iter(_BRDF_STACKS)))
+                stack = _BRDF_STACKS[key] = eng.build_brdf_modes(n_modes=K if K == 1 else min(64, (K + 7) // 8 * 8))
+            eng.set_brdf([(stack[0, m], stack[1, m]) for m in wanted])
+            self._brdf_sets = wanted
+        index = {m: j for j, m in enumerate(self._brdf_sets)}
+        beams = np.empty((S, 2, M - 1))
+        for s, sc in enumerate(self.scenarios):
+            bkey = (M, float(sc.mu0), K)
+            b = _BRDF_BEAMS.get(bkey)
+            if b is None:
+                if len(_BRDF_BEAMS) >= 4096:
+                    _BRDF_BEAMS.clear()
+                b = _BRDF_BEAMS[bkey] = np.stack([BR.brdf_beam(k, M, self.mu, sc.mu0, K) for k in BR.KERNELS])
+            beams[s] = b[:, modes[s]]
+        eng.set_brdf_scenarios(np.array([index[m] for m in modes.tolist()]),
+                               np.array([[sc.brdf_vol, sc.brdf_geo] for sc in self.scenarios], dtype=np.float64), beams)
 
     def _prepare(self, scenarios, order_caps=None):
         """Host side of a batch: tau profiles, per-scenario scalars, the table of distinct solar phase vectors with the rows
         and weights each scenario's first-order coefficients are made of (assembled on the device); phase functions met for the
         first time are appended to self._mats (the caller registers them)."""
+        check_brdf(scenarios)
         self.scenarios = list(scenarios)
         L, M = self.L, self.M
         S = len(scenarios)
@@ -288,7 +348,8 @@ class BatchSolver:
                     mats[i] = _DeviceBuilt(self.engine, k[0], k[1], tuple(k[3:5]) if len(k) > 3 else None)
         self.engine.set_phase(mats, keys=self._mat_keys)
 
-    def update(self, scenarios: Sequence[Scenario], order_caps: Optional[Sequence[int]] = None):
+    def update(self, scenarios: Sequence[Scenario], order_caps: Optional[Sequence[int]] = None,
+               brdf_modes: Optional[Sequence[int]] = None):
         """Feed the solver its next batch (same grid group, same number of scenarios): the plan, its device buffers and
         the registered phase operands are kept (sos_plan_update); only tau, the per-scenario scalars and the first-order
         coefficients change.  What a parameter sweep calls between batches instead of building a new BatchSolver."""
@@ -300,6 +361,8 @@ class BatchSolver:
                 raise ValueError("BatchSolver.update: more than 16 phase functions in one plan")
             self._register_phases()          # a phase function met for the first time: register the larger operand set
         self.engine.update(self.tau, coefs)
+        if self._key[4] == "rossli":
+            self._send_brdf(brdf_modes)
 
     def first_order(self, also_into=None):
         if SosEngine.table_fits(self.P0tab.shape[0], len(self.scenarios), self.N):
@@ -340,8 +403,8 @@ class BatchSolver:
             # TOA net flux with the F0/(4 pi) direct scaling (SOS_Aer_critical_albedo.py:377-382): same quadrature sums, direct
             # terms rescaled from F0 to F0/(4 pi) -- for the whole batch at once
             mu0 = np.array([sc.mu0 for sc in self.scenarios], dtype=np.float64)
-            # (a diffuse Lambert ground reflects the beam into the field: no collimated reflected term)
-            alb = np.array([0.0 if sc.surface == "lambert_diffuse" else sc.grd_alb for sc in self.scenarios], dtype=np.float64)
+            # (a diffuse Lambert or Ross-Li ground reflects the beam into the field: no collimated reflected term)
+            alb = np.array([0.0 if sc.surface in DIFFUSE_GROUNDS else sc.grd_alb for sc in self.scenarios], dtype=np.float64)
             k = (np.pi / mu0) * (1.0 - 1.0 / (4 * np.pi))
             t0, tl = self.tau[:, 0], self.tau[:, -1]
             fd = q["flux_down"][:, 0] + k * np.exp(-t0 / mu0)
@@ -424,6 +487,7 @@ def solved_batches(scenarios: Sequence[Scenario], device=None, keep_orders: int 
                    fold: Optional[bool] = None, groups: Optional[List[List[int]]] = None):
     """The batches of solve_scenarios one at a time: yields (indices, BatchSolver, SolveResult, [DriverResult]) while the
     batch's plan and device fields are still alive (the plan is closed when the caller asks for the next batch)."""
+    check_brdf(scenarios)   # (before the first batch touches the device)
     groups = grid_groups(scenarios) if groups is None else groups
     for idxs in [b for g in groups for b in split_for_plan_limits(scenarios, g)]:
         bs = BatchSolver([scenarios[i] for i in idxs], device=device, fold=fold)

@@ -417,6 +417,51 @@ class SosEngine:
             torch.cuda.current_stream(self.device).synchronize()   # (the table tensors may be freed after this)
         return P, P0
 
+    # ------------------------------------------------------------------ Ross-Li ground
+    def build_brdf_modes(self, n_modes: int = 1, n_quad: Optional[int] = None) -> torch.Tensor:
+        """Fourier modes 0 .. n_modes-1 of the two Ross-Li kernels on this grid, built ON THE DEVICE (sos_build_brdf_modes):
+        a (2, n_modes, M, ldr) tensor, [k][m][c][i] = rho_{k,m}(mu[M+1+i], |mu[c]|) for k = vol, geo (the transposed
+        layout the coupling reads; ldr = M-1 rounded up to even).  brdf.brdf_modes is the NumPy reference ([m][i][c])."""
+        from . import brdf as BR
+        K, nq = int(n_modes), int(n_quad if n_quad is not None else BR.BRDF_NODES)
+        M = self.M
+        ldr = _align(M - 1, 2)
+        R = torch.zeros((2, K, M, ldr), dtype=torch.float64, device=self.device)
+        phi, tab = BR.node_table(nq, K)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_build_brdf_modes(self._plan, nq, phi.ctypes.data, tab.ctypes.data, K, BR.BRDF_MU_MIN,
+                                                     R[0].data_ptr(), R[1].data_ptr(), ldr, M * ldr, self._stream),
+                       "sos_build_brdf_modes")
+            torch.cuda.current_stream(self.device).synchronize()   # (phi / tab are host temporaries)
+        return R
+
+    def set_brdf(self, pairs: Sequence):
+        """Register the mode matrix pairs of a Ross-Li plan (sos_plan_set_brdf): pairs[j] = (vol, geo), two (M, ldr) device
+        tensors in the layout of build_brdf_modes (e.g. R[0, m], R[1, m]); the engine keeps them alive."""
+        if not pairs:
+            raise ValueError("set_brdf: at least one mode matrix pair")
+        ldr = pairs[0][0].shape[-1]
+        for P in (t for pair in pairs for t in pair):
+            if P.shape != (self.M, ldr) or P.dtype != torch.float64 or not P.is_contiguous() or P.device != self.device:
+                raise ValueError("set_brdf: every matrix must be a contiguous float64 (M, ldr) tensor on the plan's device")
+        self._brdf = [tuple(pair) for pair in pairs]
+        vol = (C.c_void_p * len(pairs))(*[pair[0].data_ptr() for pair in pairs])
+        geo = (C.c_void_p * len(pairs))(*[pair[1].data_ptr() for pair in pairs])
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_plan_set_brdf(self._plan, vol, geo, len(pairs), int(ldr)), "sos_plan_set_brdf")
+
+    def set_brdf_scenarios(self, sets: np.ndarray, weights: np.ndarray, beams: np.ndarray):
+        """Per-scenario Ross-Li data (sos_plan_set_brdf_scenarios): sets (S,) pair index, weights (S, 2) = (f_vol, f_geo),
+        beams (S, 2, M-1) = the beam vectors of the scenario's mode.  Rewritten in place: captured graphs stay valid."""
+        st = np.ascontiguousarray(sets, dtype=np.int32)
+        f = np.ascontiguousarray(weights, dtype=np.float64)
+        b = np.ascontiguousarray(beams, dtype=np.float64)
+        if st.shape != (self.S,) or f.shape != (self.S, 2) or b.shape != (self.S, 2, self.M - 1):
+            raise ValueError("set_brdf_scenarios: shapes do not match the plan")
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_plan_set_brdf_scenarios(self._plan, st.ctypes.data, f.ctypes.data, b.ctypes.data, self._stream),
+                       "sos_plan_set_brdf_scenarios")
+
     def azimuth_synthesis(self, I: torch.Tensor, geo: np.ndarray, weights: np.ndarray, n_geo: int, rows: Sequence[int],
                           out: torch.Tensor, accumulate: bool):
         """out[geo][r][p][:] (+)= sum over the members s of geo (ascending) of weights[s, p] * I[s, rows[r], :N]
