@@ -69,7 +69,17 @@ typedef enum {
                                       of the ascending downward half) and the mode matrices / weights / beam vectors of
                                       sos_plan_set_brdf and sos_plan_set_brdf_scenarios (both required before a first order
                                       or a sweep: SOS_ERR_STATE otherwise).  With f_vol = f_geo = 0 every value is bit for bit
-                                      the one of SOS_SURFACE_LAMBERT_DIFFUSE.  No collimated reflected beam in the fluxes. */
+                                      the one of SOS_SURFACE_LAMBERT_DIFFUSE.  No collimated reflected beam in the fluxes. */,
+  SOS_SURFACE_OCEAN = 6            /* a wind-roughened ocean (Cox-Munk glint) in every order (three-region plans only;
+                                      SOS_ERR_UNSUPPORTED otherwise): rho = grd_alb + rho_glint(mu_i, mu_v, phi; W, n), both
+                                      in reflectance-factor units.  grd_alb (whitecaps and water-leaving light) is
+                                      SOS_SURFACE_LAMBERT_DIFFUSE unchanged; every upward column i adds
+                                        order 1:  f_glint (e^{-T/mu0} beam[i] + sum_c u_c R[c][i])
+                                        order n:  f_glint sum_c u_c R[c][i]
+                                      with one glint mode matrix R per set (sos_build_glint_modes) and the first weight and
+                                      beam vector of sos_plan_set_brdf_scenarios (u as for SOS_SURFACE_ROSSLI; both calls
+                                      required: SOS_ERR_STATE otherwise).  With f_glint = 0 every value is bit for bit the one
+                                      of SOS_SURFACE_LAMBERT_DIFFUSE.  No collimated reflected beam in the fluxes. */
 } sos_surface;
 
 /* device-side status bits (OR-ed per scenario) */
@@ -183,6 +193,17 @@ int sos_build_phase_modes(sos_plan* plan, int family, double g, double mu0, int 
 int sos_build_brdf_modes(sos_plan* plan, int n_nodes, const double* phi_h, const double* cos_h, int n_modes, double mu_min,
                          double* Rvol_d, double* Rgeo_d, int ldr, size_t mode_stride, void* stream);
 
+/* Fourier modes m = 0 .. n_modes-1 of the Cox-Munk glint on the plan's mu grid, for SOS_SURFACE_OCEAN.
+ * R_m(mu, mu') = (1/pi) int_0^pi rho_glint(mu, mu', phi) cos(m phi) dphi with phi the engine's propagation azimuth (glint at
+ * phi = 0), rho_glint = r(omega) exp(-tan^2 theta_n / sigma2) S / (4 sigma2 mu mu' mu_n^4): isotropic slope variance sigma2 > 0
+ * (Cox & Munk: 0.003 + 0.00512 W), unpolarised Fresnel reflectance r for the relative refractive index n_ref > 1, Smith
+ * shadowing S (DESIGN §12).  Nodes: phi_h [n_nodes] ascending on [0, pi] (2 <= n_nodes <= 1024), trapezoid rule;
+ * cos_h [1 + n_modes][n_nodes]: row 0 = cos(phi_k), row 1 + m = cos(m phi_k).  Writes the transposed layout of
+ * sos_build_brdf_modes: element (c, i) = R_m(mu_{M+1+i}, |mu_c|) at R_d + m * mode_stride + c * ldr + i; the entries of the
+ * column mu = 0- are 0.  1 <= n_modes <= 64. */
+int sos_build_glint_modes(sos_plan* plan, int n_nodes, const double* phi_h, const double* cos_h, int n_modes, double sigma2,
+                          double n_ref, double* R_d, int ldr, size_t mode_stride, void* stream);
+
 /* Azimuth synthesis of Fourier-mode fields: out[geo][r][p][col] (+)= sum over s with geo_h[s] = geo of
  * w_h[s][p] * I[s][rows_h[r]][col] (col < N), the sum in ascending s (no atomics: deterministic).  I_d: a field of this plan
  * ([S*L][ld]); geo_h [S] in [0, n_geo) or -1 (member skipped); w_h [S][n_az] (1 for mode 0, 2 cos(m phi_p) for mode m, as
@@ -192,17 +213,35 @@ int sos_build_brdf_modes(sos_plan* plan, int n_nodes, const double* phi_h, const
 int sos_azimuth_synthesis(sos_plan* plan, const double* I_d, const int* geo_h, const double* w_h, int n_geo, const int* rows_h,
                           int n_rows, int n_az, double* out_d, int accumulate, void* stream);
 
+/* Exact direct glint of azimuth-resolved radiance over SOS_SURFACE_OCEAN: for entries k = 0 .. n-1, rows r, azimuths
+ * p and upward columns i = M+1 .. N-1 of the plan's grid,
+ *   out[geo_h[k]][r][p][i] += e^{-T/mu0} (rho_glint(mu_i, mu0, phi_p) - sum_{m < n_modes} (2 - delta_m0) beam[k][m][i] cos(m phi_p))
+ *                             * e^{-(T - tau[k][r]) / mu_i}
+ * (out as written by sos_azimuth_synthesis, [n_geo][n_rows][n_az][N]; geo_h [n] in [0, n_geo)): the once-reflected direct
+ * beam, transmitted without scattering to the row, with its truncated Fourier series replaced by the exact reflectance.
+ * par_h [n][4] = (mu0, tauStar_tot, sigma2, n_ref); tau_h [n][n_rows] = tau at the rows; beam_h [n][n_modes][M-1] = the
+ * glint beam vectors of modes 0 .. n_modes-1 (the ones given to sos_plan_set_brdf_scenarios); phi_h [n_az].  One thread
+ * per output element, no atomics: deterministic.  1 <= n_modes <= 64. */
+int sos_glint_correction(sos_plan* plan, int n, const int* geo_h, const double* par_h, const double* tau_h, int n_rows,
+                         const double* beam_h, int n_modes, const double* phi_h, int n_az, int n_geo, double* out_d,
+                         void* stream);
+
 /* Register the contraction matrices (device, [N][lda] each) the scenarios index. */
 int sos_plan_set_phase(sos_plan* plan, const double* const* A_d, int n_matrices, int lda);
 
-/* SOS_SURFACE_ROSSLI plans only (SOS_ERR_UNSUPPORTED otherwise).
+/* SOS_SURFACE_ROSSLI and SOS_SURFACE_OCEAN plans only (SOS_ERR_UNSUPPORTED otherwise).
  *   sos_plan_set_brdf            register n_sets (1 .. 64) mode matrix pairs (Rvol_d[j], Rgeo_d[j]): device [M][ldr] each in
  *                                the transposed layout of sos_build_brdf_modes (ldr >= M-1), kept alive by the caller.  Drops
- *                                the captured order graphs; the per-scenario data must be given again afterwards.
+ *                                the captured order graphs; the per-scenario data must be given again afterwards.  An ocean
+ *                                plan takes one matrix per set (the glint of one (W, n, mode), sos_build_glint_modes) in
+ *                                Rvol_d and Rgeo_d = NULL; NULL for a Ross-Li plan, or not NULL for an ocean plan, is
+ *                                SOS_ERR_INVALID.
  *   sos_plan_set_brdf_scenarios  per scenario: set_h [S] (the pair it uses, 0 .. n_sets-1), f_h [S][2] = (f_vol, f_geo) >= 0
  *                                and beam_h [S][2][M-1] = (R^vol_m(mu_i, mu0), R^geo_m(mu_i, mu0)) over the upward columns
  *                                i = M+1 .. N-1 for the scenario's mode m.  Copied on `stream` into plan-owned buffers in place:
- *                                captured order graphs stay valid, so it follows sos_plan_update for the next batch. */
+ *                                captured order graphs stay valid, so it follows sos_plan_update for the next batch.  Ocean:
+ *                                f_h[s] = (f_glint >= 0, 0) (a second weight != 0 is SOS_ERR_INVALID), beam_h[s][0] = the
+ *                                glint mode R_m(mu_i, mu0); beam_h[s][1] is not read. */
 int sos_plan_set_brdf(sos_plan* plan, const double* const* Rvol_d, const double* const* Rgeo_d, int n_sets, int ldr);
 int sos_plan_set_brdf_scenarios(sos_plan* plan, const int* set_h, const double* f_h, const double* beam_h, void* stream);
 

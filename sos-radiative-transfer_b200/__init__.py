@@ -14,6 +14,8 @@ from .grid import mu_grid, tau_profile, extrapolation_width, aerosol_rows
 from .phase import phase_matrices, phase_P, phase_P0, phase_table, phase_modes
 from . import brdf
 from .brdf import BRDF_NODES, BRDF_MU_MIN, rossli_kernels, brdf_modes, brdf_beam
+from . import ocean
+from .ocean import cox_munk, glint_modes, glint_beam
 from . import mie
 from .mie import EVA_AEROSOL, WILDFIRE_AEROSOL
 from .engine import SosEngine, ScenarioCoefficients, SolveResult
@@ -30,7 +32,7 @@ from .azimuth import AzimuthalResult, solve_azimuthal
 
 __all__ = [
     "SosError", "mu_grid", "tau_profile", "extrapolation_width", "aerosol_rows", "phase_matrices", "phase_P", "phase_P0", "phase_table", "phase_modes",
-    "brdf", "BRDF_NODES", "BRDF_MU_MIN", "rossli_kernels", "brdf_modes", "brdf_beam", "mie", "EVA_AEROSOL", "WILDFIRE_AEROSOL",
+    "brdf", "BRDF_NODES", "BRDF_MU_MIN", "rossli_kernels", "brdf_modes", "brdf_beam", "ocean", "cox_munk", "glint_modes", "glint_beam", "mie", "EVA_AEROSOL", "WILDFIRE_AEROSOL",
     "SosEngine", "ScenarioCoefficients", "SolveResult", "I1_NumInt", "Jn_NumInt", "In_NumInt",
     "mu_approx_In", "clear_cache", "Scenario", "DriverResult", "BatchSolver", "solve_scenarios",
     "MuShardedSolver", "LayerShardedSolver", "PeerFields", "PeerBuffers", "mu_blocks", "shard_scenarios", "gather_scenario_results", "allgather_columns", "shard_range",

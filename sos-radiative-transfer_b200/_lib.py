@@ -71,7 +71,7 @@ class sos_result(C.Structure):
 
 
 SURFACE_NONE, SURFACE_SPECULAR, SURFACE_LAMBERT, SURFACE_LAMBERT_README, SURFACE_LAMBERT_DIFFUSE = 0, 1, 2, 3, 4
-SURFACE_ROSSLI = 5
+SURFACE_ROSSLI, SURFACE_OCEAN = 5, 6
 QUERY_FUSED_ORDER, QUERY_GENERATED_SOURCE, QUERY_FOLDED, QUERY_DEVICE = 0, 1, 2, 3
 STATUS_BLEND_OVERRUN, STATUS_NONFINITE, STATUS_MAX_ORDERS = 1, 2, 4
 
@@ -94,6 +94,8 @@ SIGNATURES = {
     "sos_build_brdf_modes": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, _vp, C.c_int, C.c_size_t, _vp]),
     "sos_plan_set_brdf": (C.c_int, [_vp, C.POINTER(_vp), C.POINTER(_vp), C.c_int, C.c_int]),
     "sos_plan_set_brdf_scenarios": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
+    "sos_build_glint_modes": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_double, C.c_double, _vp, C.c_int, C.c_size_t, _vp]),
+    "sos_glint_correction": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_int, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp]),
     "sos_azimuth_synthesis": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, _vp]),
     "sos_plan_set_phase": (C.c_int, [_vp, C.POINTER(_vp), C.c_int, C.c_int]),
     "sos_fold_layout": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),

@@ -5,13 +5,16 @@ mode m of the radiance obeys the same equation as mode 0 -- the same contraction
 specular mirror coupling -- with the operand P_m and the solar vector P0_m of phase.phase_modes instead of P and P0.  A
 diffuse Lambert ground ('lambert_diffuse') is isotropic and enters mode 0 only: modes m >= 1 are solved over a black
 ground.  A Ross-Li ground ('rossli') couples mode m through its own kernel modes (brdf module): the members of mode m keep
-the surface with grd_alb = 0 (the isotropic part has no mode m >= 1) and the Ross-Li mode m.  So a
+the surface with grd_alb = 0 (the isotropic part has no mode m >= 1) and the Ross-Li mode m; so do those of an ocean
+('ocean') with the glint mode m.  So a
 (geometry, mode) pair is one more member of a batch: its own operand index and first-order table row, summing exactly the
 orders its mode 0 summed (sos_scenario.order_cap), and
 
     I(tau, mu, phi) = I_0 + 2 sum_{m >= 1} I_m cos(m phi)
 
-is summed on the device (sos_azimuth_synthesis).
+is summed on the device (sos_azimuth_synthesis).  Over an ocean the radiance also gets the once-reflected direct beam in
+closed form (sos_glint_correction): the glint lobe is too narrow in azimuth for 64 modes at low wind, so its truncated
+series is replaced by the exact reflectance on every upward column.
 
 phi is the azimuth of the PROPAGATION direction of the diffuse light relative to the propagation azimuth of the solar beam:
 with the grid's signs (mu < 0 downward) the beam travels along (-mu0, 0), cos Theta = -mu0 mu + sqrt(1 - mu0^2) sqrt(1 - mu^2)
@@ -27,8 +30,9 @@ import numpy as np
 import torch
 
 from . import phase as PH
-from .drivers import (DriverResult, MAX_PHASES_PER_PLAN, BatchSolver, Scenario, _BRDF_STACKS, _MODE_STACKS, check_brdf,
-                      grid_groups, solved_batches, split_for_plan_limits)
+from . import ocean as OC
+from .drivers import (DriverResult, MAX_PHASES_PER_PLAN, BatchSolver, Scenario, _BRDF_STACKS, _GLINT_STACKS, _MODE_STACKS,
+                      check_brdf, glint_beam, grid_groups, solved_batches, split_for_plan_limits)
 
 # phase functions per plan of the mode members (two per mode: typically 8 modes per plan)
 MODE_PHASES_PER_PLAN = MAX_PHASES_PER_PLAN
@@ -37,9 +41,10 @@ MODE_PHASES_PER_PLAN = MAX_PHASES_PER_PLAN
 @dataclass
 class AzimuthalResult:
     """base: the mode-0 result (what solve_scenarios returns for the scenario); radiance (n_rows, n_phi, N): I(tau_row, mu, phi)
-    at the layers `rows` and azimuths `phi`; modes (n_modes, n_rows, N): the Fourier components I_m at those layers (mode 0 =
-    base.I rows); mode_orders / mode_status (n_modes,): orders summed and status bits of every mode (a mode whose
-    atmosphere and aerosol modes vanish is not solved: 0 orders, I_m = 0)."""
+    at the layers `rows` and azimuths `phi` (over an ocean with the exact direct glint: the once-reflected, unscattered beam
+    in closed form instead of its truncated series); modes (n_modes, n_rows, N): the Fourier components I_m at those layers
+    (the truncated series, order for order; mode 0 = base.I rows); mode_orders / mode_status (n_modes,): orders summed and
+    status bits of every mode (a mode whose atmosphere and aerosol modes vanish is not solved: 0 orders, I_m = 0)."""
     base: DriverResult
     radiance: np.ndarray
     rows: np.ndarray
@@ -85,8 +90,10 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
     order, as the mode-0 field.  n_quad: azimuth nodes of the mode builder (>= 2 n_modes; 25 = the azimuth-averaged
     builders' nodes, enough for Rayleigh and moderate HG -- sharp peaks need more).  A 'lambert_diffuse' ground enters mode 0
     only (the modes m >= 1 of its geometries are solved over a black ground); a 'rossli' ground enters every mode through
-    its kernel modes, which are integrated on brdf.BRDF_NODES nodes whatever n_quad.  'lambert' / 'lambert_readme' surfaces with
-    grd_alb > 0 and caller-supplied (P0, P) arrays raise ValueError before any device work."""
+    its kernel modes, which are integrated on brdf.BRDF_NODES nodes whatever n_quad; so does an 'ocean' through its glint
+    modes, and its radiance includes the exact direct glint (the once-reflected beam transmitted without scattering, in closed
+    form instead of its n_modes-term series; `modes` and `base` stay the truncated series).  'lambert' / 'lambert_readme'
+    surfaces with grd_alb > 0 and caller-supplied (P0, P) arrays raise ValueError before any device work."""
     scenarios = list(scenarios)
     K, n_quad = int(n_modes), int(n_quad)
     _validate(scenarios, K, n_quad)
@@ -116,6 +123,8 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
                     radiance = torch.empty((len(group), rws.size, n_az, eng.N), dtype=torch.float64, device=eng.device)
                 eng.azimuth_synthesis(res.I, np.array([pos[i] for i in idxs]), np.tile(ones, (len(idxs), 1)), len(group), rws,
                                       radiance, accumulate=False)
+                if scenarios[idxs[0]].surface == "ocean":
+                    _glint_correction(eng, bs, [scenarios[i] for i in idxs], [pos[i] for i in idxs], rws, K, phi, radiance)
                 for i, r in zip(idxs, results):
                     base[i], n0[i] = r, int(r.n)
                     modes[i][0] = r.I[rws]
@@ -125,21 +134,22 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
             for i in group:
                 sc = scenarios[i]
                 for m in range(1, K):
-                    brdf = sc.surface == "rossli" and (sc.brdf_vol != 0 or sc.brdf_geo != 0)
+                    brdf = (sc.surface == "rossli" and (sc.brdf_vol != 0 or sc.brdf_geo != 0)) or sc.surface == "ocean"
                     if _vanishes(sc.atm_phase, m) and _vanishes(sc.aer_phase, m) and not brdf:
-                        continue   # I_m = 0: nothing to solve (a Ross-Li ground reflects mode m of the beam itself)
+                        continue   # I_m = 0: nothing to solve (a Ross-Li or ocean ground reflects mode m of the beam itself)
                     mode_sc = replace(sc, atm_phase=_mode_spec(sc.atm_phase, m, n_quad), aer_phase=_mode_spec(sc.aer_phase, m, n_quad))
                     if sc.surface == "lambert_diffuse":
                         mode_sc = replace(mode_sc, surface="specular", grd_alb=0.0)   # an isotropic ground has no mode m >= 1
-                    elif sc.surface == "rossli":
-                        mode_sc = replace(mode_sc, grd_alb=0.0)   # the kernels' mode m (BatchSolver brdf_modes below)
+                    elif sc.surface in ("rossli", "ocean"):
+                        mode_sc = replace(mode_sc, grd_alb=0.0)   # the kernels' / glint's mode m (BatchSolver brdf_modes below)
                     members.append(mode_sc)
                     keys.append((i, m))
-            for sub in split_for_plan_limits(members, range(len(members)), max_phases=MODE_PHASES_PER_PLAN):
+            for sub in split_for_plan_limits(members, range(len(members)), max_phases=MODE_PHASES_PER_PLAN,
+                                             brdf_modes=[k[1] for k in keys]):
                 caps = [n0[keys[j][0]] for j in sub]
-                rossli = members[sub[0]].surface == "rossli"
+                brdf = members[sub[0]].surface in ("rossli", "ocean")
                 bs = BatchSolver([members[j] for j in sub], device=device, order_caps=caps,
-                                 brdf_modes=[keys[j][1] for j in sub] if rossli else None)
+                                 brdf_modes=[keys[j][1] for j in sub] if brdf else None)
                 try:
                     res = bs.solve(max_orders=max(caps))
                     eng = bs.engine
@@ -160,4 +170,16 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
     finally:
         _MODE_STACKS.clear()   # the device mode stacks serve the sub-batches of one call
         _BRDF_STACKS.clear()
+        _GLINT_STACKS.clear()
     return out  # type: ignore
+
+
+def _glint_correction(eng, bs: BatchSolver, scs: Sequence[Scenario], geo: Sequence[int], rws: np.ndarray, K: int, phi: np.ndarray,
+                      radiance: torch.Tensor):
+    """Replace the K-term series of the once-reflected, unscattered direct beam in `radiance` by the exact glint for the
+    ocean geometries `scs` of one mode-0 batch (sos_glint_correction); the modes m >= 1 of those geometries are all solved."""
+    M = bs.M
+    par = np.array([[sc.mu0, sc.tauStar_atm + sc.tauStar_aer, float(OC.slope_variance(sc.wind_speed)), sc.ocean_index]
+                    for sc in scs], dtype=np.float64)
+    beams = np.stack([glint_beam(M, bs.mu, sc, K) for sc in scs])
+    eng.glint_correction(radiance, np.asarray(geo), par, bs.tau[:, rws], beams, phi)

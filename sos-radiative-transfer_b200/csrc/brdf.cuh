@@ -21,7 +21,8 @@ constexpr int MAX_NODES = 1024;
 constexpr int MAX_SETS = 64;      // mode matrix pairs one plan can index (sos_plan_set_brdf)
 constexpr int BUILD_THREADS = 64;
 
-// What the coupling kernels read (plan-owned buffers; all nullptr on other surfaces).
+// What the coupling kernels read (plan-owned buffers; all nullptr on other surfaces).  The Cox-Munk ocean (glint.cuh) uses
+// the same buffers with one matrix per set: R[2 j] = glint, R[2 j + 1] = nullptr, f = (f_glint, 0), the second beam unread.
 struct BrdfDev {
   const double* const* R;  // [n_sets][2] device pointers: R[2 j] = vol, R[2 j + 1] = geo, [M][ldr] each (transposed, above)
   const int* set;          // [S] mode matrix pair of each scenario
@@ -91,6 +92,16 @@ __device__ __forceinline__ void coupling(const BrdfDev& b, int s, const double* 
   }
   sv = av;
   sg = ag;
+}
+
+// The one-matrix form (the ocean's glint): sum_c u_c R[c][i] in ascending c.
+__device__ __forceinline__ double coupling(const BrdfDev& b, int s, const double* __restrict__ u, int M, int i) {
+  const double* __restrict__ R = b.R[2 * b.set[s]] + i;
+  const size_t ld = static_cast<size_t>(b.ldr);
+  double a = 0.0;
+#pragma unroll 4
+  for (int c = 0; c < M; ++c) a += u[c] * R[c * ld];
+  return a;
 }
 
 // u_c = -2 w_c mu_c I[L-1, c], c = 0 .. M-1, with w the trapezoid weights of the ascending downward half (the abscissae of

@@ -14,7 +14,7 @@
 // A diffuse Lambert ground (SOS_SURFACE_LAMBERT_DIFFUSE) has no mirror term (S = 0); the carry of every upward column at
 // the surface row is the isotropic b_s of first_order_surface_kernel, a pre-pass with one CTA per scenario.  A Ross-Li
 // ground (SOS_SURFACE_ROSSLI) has one such carry per upward column: b_s plus the reflection of the beam and of order 1's
-// downward light by the two kernels (brdf.cuh).
+// downward light by the two kernels (brdf.cuh); so has the ocean (SOS_SURFACE_OCEAN), with the one glint matrix (glint.cuh).
 #pragma once
 #include "common.cuh"
 #include "sweep.cuh"  // sossweep::block_sum
@@ -218,9 +218,11 @@ first_order_regions_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
 // per scenario evaluates row L-1 of the downward columns with the calls and row factors of first_order_regions_kernel
 // (S = 0), so these are the values it stores; the trapezoid is the one of the lambert_readme coupling (sweep.cuh: ascending
 // abscissa, the interval next to mu = 0- included) and is summed by the deterministic block sum.
-// Ross-Li ground (brdf.f != nullptr): bs[s][i] = b_s + sum_k f_k (e^{-T/mu0} beam_k[i] + sum_c u_c R^k[c][i]) for the upward
-// columns i = 0 .. M-2, u_c = -2 w_c mu_c I1[L-1, c] (sosbrdf::coupling_weight); with grd_alb = f_iso, b_s is the term above.
+// NK kernel matrices (Ross-Li ground: 2, ocean: 1; 0 = the diffuse Lambert ground above): bs[s][i] = b_s + sum_k f_k
+// (e^{-T/mu0} beam_k[i] + sum_c u_c R^k[c][i]) for the upward columns i = 0 .. M-2, u_c = -2 w_c mu_c I1[L-1, c]
+// (sosbrdf::coupling_weight); with grd_alb = the isotropic part, b_s is the term above.
 // Dynamic shared memory: (M + 32) doubles.
+template <int NK>
 __global__ void __launch_bounds__(128)
 first_order_surface_kernel(const GridDev g, const double* __restrict__ Cs /*[S][2][N]*/, double* __restrict__ bs,
                            const sosbrdf::BrdfDev brdf) {
@@ -265,19 +267,23 @@ first_order_surface_kernel(const GridDev g, const double* __restrict__ Cs /*[S][
   }
   const double down = -2.0 * sossweep::block_sum(part, fo_row + M);
   const double b_s = sc.grd_alb * (exp(-T / mu0) + down);
-  if (!brdf.f) {
+  if constexpr (NK == 0) {
     if (threadIdx.x == 0) bs[s] = b_s;
-    return;
-  }
-  for (int c = threadIdx.x; c < M; c += blockDim.x) fo_row[c] *= sosbrdf::coupling_weight(g.mu, M, c);   // (block_sum synced)
-  __syncthreads();
-  const double E = exp(-T / mu0), fv = brdf.f[2 * s], fg = brdf.f[2 * s + 1];
-  const double* __restrict__ bv = brdf.beam + static_cast<size_t>(s) * 2 * (M - 1);
-  const double* __restrict__ bg = bv + (M - 1);
-  for (int i = threadIdx.x; i < M - 1; i += blockDim.x) {
-    double sv, sgeo;
-    sosbrdf::coupling(brdf, s, fo_row, M, i, sv, sgeo);
-    bs[static_cast<size_t>(s) * (M - 1) + i] = b_s + (fv * (E * bv[i] + sv) + fg * (E * bg[i] + sgeo));
+  } else {
+    for (int c = threadIdx.x; c < M; c += blockDim.x) fo_row[c] *= sosbrdf::coupling_weight(g.mu, M, c);   // (block_sum synced)
+    __syncthreads();
+    const double E = exp(-T / mu0), fv = brdf.f[2 * s], fg = brdf.f[2 * s + 1];
+    const double* __restrict__ bv = brdf.beam + static_cast<size_t>(s) * 2 * (M - 1);
+    const double* __restrict__ bg = bv + (M - 1);
+    for (int i = threadIdx.x; i < M - 1; i += blockDim.x) {
+      if constexpr (NK == 2) {
+        double sv, sgeo;
+        sosbrdf::coupling(brdf, s, fo_row, M, i, sv, sgeo);
+        bs[static_cast<size_t>(s) * (M - 1) + i] = b_s + (fv * (E * bv[i] + sv) + fg * (E * bg[i] + sgeo));
+      } else {
+        bs[static_cast<size_t>(s) * (M - 1) + i] = b_s + fv * (E * bv[i] + sosbrdf::coupling(brdf, s, fo_row, M, i));
+      }
+    }
   }
 }
 

@@ -2,6 +2,7 @@
 // SOS_Aer_critical_albedo.py:377-382) and the contraction-operand builder.
 #pragma once
 #include "common.cuh"
+#include "glint.cuh"
 
 namespace sosquad {
 
@@ -55,8 +56,9 @@ quadrature_outputs_kernel(const GridDev g, const double* __restrict__ sums, cons
   const double* q = sums + (static_cast<size_t>(s) * L + t) * 3;
   const size_t o = static_cast<size_t>(s) * L + t;
   const double dn = exp(-tau[t] / sc.mu0);
-  // the collimated beam reflected by a mirror ground; a diffuse Lambert or Ross-Li ground puts it into the field itself
-  const double alb_dir = (g.surface == SOS_SURFACE_LAMBERT_DIFFUSE || g.surface == SOS_SURFACE_ROSSLI) ? 0.0 : sc.grd_alb;
+  // the collimated beam reflected by a mirror ground; a diffuse Lambert, Ross-Li or ocean ground puts it into the field itself
+  const double alb_dir =
+      (g.surface == SOS_SURFACE_LAMBERT_DIFFUSE || g.surface == SOS_SURFACE_ROSSLI || g.surface == SOS_SURFACE_OCEAN) ? 0.0 : sc.grd_alb;
   const double up = alb_dir * exp(-(2.0 * tl - tau[t]) / sc.mu0);
   if (flux_down) flux_down[o] = q[0] - (F0 * direct_scale) * dn;                 // graphe.py:157 / :77
   if (flux_up) flux_up[o] = q[1] + (F0 * direct_scale) * up;                     // graphe.py:158 / :78
@@ -144,6 +146,43 @@ azimuth_synthesis_kernel(const double* __restrict__ I, int L, int ld, int N, con
 #pragma unroll
   for (int q = 0; q < AZ_CHUNK; ++q)
     if (q < np) o[static_cast<size_t>(q) * N] = accumulate ? o[static_cast<size_t>(q) * N] + acc[q] : acc[q];
+}
+
+// Exact direct glint of azimuth-resolved radiance (sos_glint_correction).  One thread per output element (entry k,
+// requested row r, azimuth p, upward column i): out[geo[k]][r][p][M+1+i] += E (rho_glint(mu_i, mu0, phi_p) - sum_{m<K} w[p][m]
+// beam[k][m][i]) e^{-(T - tau[k][r]) / mu_i}, E = e^{-T/mu0}, w[p][m] = 1 (m = 0) or 2 cos(m phi_p): the once-reflected direct
+// beam, transmitted without scattering to the row, with its truncated Fourier series replaced by the exact value.
+struct GlintCorrection {
+  const int* geo;       // [n] geometry (first index of out) of each entry
+  const double* par;    // [n][4] mu0, tauStar_tot, sigma^2, n_ref
+  const double* tau;    // [n][n_rows] tau at the requested rows
+  const double* beam;   // [n][K][M-1]
+  const double* w;      // [n_az][K]
+  const double* cphi;   // [n_az]
+};
+
+__global__ void __launch_bounds__(128)
+glint_correction_kernel(const double* __restrict__ mu, int M, int N, const GlintCorrection t, int n, int K, int n_rows,
+                        int n_az, double* __restrict__ out) {
+  const long long e = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const long long per_k = static_cast<long long>(n_rows) * n_az * (M - 1);
+  if (e >= per_k * n) return;
+  const int k = static_cast<int>(e / per_k);
+  long long rest = e % per_k;
+  const int i = static_cast<int>(rest % (M - 1));
+  rest /= (M - 1);
+  const int p = static_cast<int>(rest % n_az), r = static_cast<int>(rest / n_az);
+  const double* __restrict__ par = t.par + 4 * static_cast<size_t>(k);
+  const double mu0 = par[0], T = par[1], sigma2 = par[2], nref = par[3];
+  const double mi = mu[M + 1 + i];
+  const double rho = sosglint::glint(mi, mu0, t.cphi[p], sigma2, nref, sosglint::shadowing(mi, mu0, sqrt(sigma2)));
+  const double* __restrict__ b = t.beam + static_cast<size_t>(k) * K * (M - 1) + i;
+  const double* __restrict__ w = t.w + static_cast<size_t>(p) * K;
+  double series = 0.0;
+  for (int m = 0; m < K; ++m) series += w[m] * b[static_cast<size_t>(m) * (M - 1)];
+  const double tr = exp(-(T - t.tau[static_cast<size_t>(k) * n_rows + r]) / mi);
+  double* o = out + ((static_cast<size_t>(t.geo[k]) * n_rows + r) * n_az + p) * N + (M + 1 + i);
+  *o += exp(-T / mu0) * (rho - series) * tr;
 }
 
 }  // namespace sosquad

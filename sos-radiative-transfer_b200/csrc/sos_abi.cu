@@ -115,10 +115,11 @@ struct sos_plan {
   double* d_z = nullptr;     // [L]
   double* d_colint = nullptr;  // [N] column integrals of the device phase builder
   double* d_bs = nullptr;    // upward surface radiance of order 1: [S] over a diffuse Lambert ground, [S][M-1] over a Ross-Li one
-  // Ross-Li ground (that surface only): the registered mode matrix pairs and the per-scenario data of sosbrdf::BrdfDev
+  // Ross-Li / ocean ground (those surfaces only): the registered mode matrix pairs and the per-scenario data of
+  // sosbrdf::BrdfDev; brdf_nk = matrices per set (Ross-Li 2, ocean 1, other surfaces 0)
   const double** d_brdf_R = nullptr;  // [MAX_SETS][2]
   char* d_brdf_scen = nullptr;        // [S][2] f | [S][2][M-1] beam | [S] set (int)
-  int brdf_sets = 0, brdf_ldr = 0;
+  int brdf_sets = 0, brdf_ldr = 0, brdf_nk = 0;
   bool brdf_scen_ready = false;
   int* h_poll = nullptr;     // pinned
   double* h_C[2] = {nullptr, nullptr};        // pinned staging of the first-order coefficients (sos_first_order never blocks)
@@ -544,8 +545,9 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
     if (grid->region_start[k + 1] <= grid->region_start[k]) return SOS_ERR_INVALID;
   if (grid->n_regions == 3 && (grid->region_start[1] < 2 || grid->region_start[2] < grid->region_start[1] + 1))
     return SOS_ERR_INVALID;
-  if (grid->surface < 0 || grid->surface > 5) return SOS_ERR_INVALID;
-  if ((grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE || grid->surface == SOS_SURFACE_ROSSLI) && grid->n_regions != 3)
+  if (grid->surface < 0 || grid->surface > 6) return SOS_ERR_INVALID;
+  if ((grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE || grid->surface == SOS_SURFACE_ROSSLI || grid->surface == SOS_SURFACE_OCEAN) &&
+      grid->n_regions != 3)
     return SOS_ERR_UNSUPPORTED;
 
   int dev = 0;
@@ -700,7 +702,8 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
   TRY(dev_alloc(p, &p->d_z, static_cast<size_t>(L)));
   TRY(dev_alloc(p, &p->d_colint, static_cast<size_t>(N)));
   if (grid->surface == SOS_SURFACE_LAMBERT_DIFFUSE) TRY(dev_alloc(p, &p->d_bs, static_cast<size_t>(S)));
-  if (grid->surface == SOS_SURFACE_ROSSLI) {
+  if (grid->surface == SOS_SURFACE_ROSSLI || grid->surface == SOS_SURFACE_OCEAN) {
+    p->brdf_nk = (grid->surface == SOS_SURFACE_ROSSLI) ? 2 : 1;
     TRY(dev_alloc(p, &p->d_bs, static_cast<size_t>(S) * (M - 1)));
     TRY(dev_alloc(p, &p->d_brdf_R, static_cast<size_t>(2) * sosbrdf::MAX_SETS));
     TRY(dev_alloc(p, &p->d_brdf_scen, brdf_scen_bytes(S, M)));
@@ -794,11 +797,14 @@ int sos_plan_create(sos_plan** out, const sos_grid* grid, const double* mu_h, co
     cudaDeviceSynchronize();
   }
   if (p->d_bs && (M + 32) * sizeof(double) > 48 * 1024) {
-    cudaFuncSetAttribute(sosfirst::first_order_surface_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (M + 32) * sizeof(double));
+    cudaFuncSetAttribute(sosfirst::first_order_surface_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (M + 32) * sizeof(double));
+    cudaFuncSetAttribute(sosfirst::first_order_surface_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (M + 32) * sizeof(double));
+    cudaFuncSetAttribute(sosfirst::first_order_surface_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (M + 32) * sizeof(double));
   }
   if ((N + 32 + 2 * (nch + 1)) * sizeof(double) > 48 * 1024) {
-    cudaFuncSetAttribute(sossweep::sweep_carry_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
-    cudaFuncSetAttribute(sossweep::sweep_carry_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
+    cudaFuncSetAttribute(sossweep::sweep_carry_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
+    cudaFuncSetAttribute(sossweep::sweep_carry_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
+    cudaFuncSetAttribute(sossweep::sweep_carry_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (N + 32 + 2 * (nch + 1)) * sizeof(double));
   }
   {
     int r3 = gen_setup(p, p->scen_h.data());
@@ -1237,16 +1243,100 @@ int sos_build_brdf_modes(sos_plan* p, int n_nodes, const double* phi_h, const do
   return r;
 }
 
+int sos_build_glint_modes(sos_plan* p, int n_nodes, const double* phi_h, const double* cos_h, int n_modes, double sigma2,
+                          double n_ref, double* R_d, int ldr, size_t mode_stride, void* stream) {
+  if (!p || !phi_h || !cos_h || !R_d) return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  const int M = p->dev.M;
+  if (n_nodes < 2 || n_nodes > sosbrdf::MAX_NODES || n_modes < 1 || n_modes > sosbrdf::MAX_MODES) return SOS_ERR_INVALID;
+  if (!(sigma2 > 0.0 && std::isfinite(sigma2)) || !(n_ref > 1.0 && std::isfinite(n_ref))) return SOS_ERR_INVALID;
+  if (M < 2 || ldr < M - 1 || (n_modes > 1 && mode_stride < static_cast<size_t>(M) * ldr)) return SOS_ERR_INVALID;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // node table [cos(phi_k) | trapezoid weight * cos(m phi_k) / pi], as for sos_build_brdf_modes
+  const double PI = 3.14159265358979323846;
+  std::vector<double> tab(static_cast<size_t>(n_nodes) * (1 + n_modes), 0.0);
+  double* cphi = tab.data();
+  double* wcos = cphi + n_nodes;
+  for (int k = 0; k < n_nodes; ++k) {
+    cphi[k] = cos_h[k];
+    const double tw = 0.5 * ((k + 1 < n_nodes ? phi_h[k + 1] : phi_h[k]) - (k > 0 ? phi_h[k - 1] : phi_h[k]));
+    for (int m = 0; m < n_modes; ++m) wcos[static_cast<size_t>(k) * n_modes + m] = tw * cos_h[static_cast<size_t>(1 + m) * n_nodes + k] / PI;
+  }
+  double* tab_d = nullptr;
+  SOS_CUDA(cudaMallocAsync(&tab_d, tab.size() * sizeof(double), st));
+  SOS_CUDA(cudaMemcpyAsync(tab_d, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  const size_t smem = static_cast<size_t>(n_modes) * sosbrdf::BUILD_THREADS * sizeof(double);
+  cudaFuncSetAttribute(sosglint::glint_modes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+  const long long n_el = static_cast<long long>(M) * (M - 1);
+  sosglint::glint_modes_kernel<<<static_cast<unsigned>((n_el + sosbrdf::BUILD_THREADS - 1) / sosbrdf::BUILD_THREADS), sosbrdf::BUILD_THREADS,
+                                 smem, st>>>(p->dev.mu, M, sigma2, n_ref, tab_d, tab_d + n_nodes, n_nodes, n_modes, R_d, ldr, mode_stride);
+  const int r = launch_check(p, "glint_modes_kernel");
+  SOS_CUDA(cudaFreeAsync(tab_d, st));
+  return r;
+}
+
+int sos_glint_correction(sos_plan* p, int n, const int* geo_h, const double* par_h, const double* tau_h, int n_rows,
+                         const double* beam_h, int n_modes, const double* phi_h, int n_az, int n_geo, double* out_d,
+                         void* stream) {
+  if (!p || !geo_h || !par_h || !tau_h || !beam_h || !phi_h || !out_d || n < 1 || n_rows < 1 || n_az < 1 || n_geo < 1)
+    return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  const int M = p->dev.M, N = p->dev.N;
+  if (n_modes < 1 || n_modes > sosbrdf::MAX_MODES || M < 2) return SOS_ERR_INVALID;
+  for (int k = 0; k < n; ++k) {
+    const double* q = par_h + 4 * static_cast<size_t>(k);
+    if (geo_h[k] < 0 || geo_h[k] >= n_geo) return SOS_ERR_INVALID;
+    if (!(q[0] > 0.0 && q[0] <= 1.0) || !std::isfinite(q[1]) || !(q[2] > 0.0 && std::isfinite(q[2])) ||
+        !(q[3] > 1.0 && std::isfinite(q[3])))
+      return SOS_ERR_INVALID;
+  }
+  // one table: par [n][4] | tau [n][n_rows] | beam [n][K][M-1] | w [n_az][K] | cos(phi) [n_az] | geo [n] (int)
+  const size_t n_par = 4 * static_cast<size_t>(n), n_tau = static_cast<size_t>(n) * n_rows,
+               n_beam = static_cast<size_t>(n) * n_modes * (M - 1), n_w = static_cast<size_t>(n_az) * n_modes;
+  std::vector<double> tab(n_par + n_tau + n_beam + n_w + n_az);
+  std::copy(par_h, par_h + n_par, tab.begin());
+  std::copy(tau_h, tau_h + n_tau, tab.begin() + n_par);
+  std::copy(beam_h, beam_h + n_beam, tab.begin() + n_par + n_tau);
+  double* w = tab.data() + n_par + n_tau + n_beam;
+  double* cphi = w + n_w;
+  for (int q = 0; q < n_az; ++q) {
+    cphi[q] = std::cos(phi_h[q]);
+    for (int m = 0; m < n_modes; ++m) w[static_cast<size_t>(q) * n_modes + m] = m == 0 ? 1.0 : 2.0 * std::cos(m * phi_h[q]);
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  char* buf = nullptr;
+  const size_t dbytes = tab.size() * sizeof(double);
+  SOS_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&buf), dbytes + n * sizeof(int), st));
+  SOS_CUDA(cudaMemcpyAsync(buf, tab.data(), dbytes, cudaMemcpyHostToDevice, st));
+  SOS_CUDA(cudaMemcpyAsync(buf + dbytes, geo_h, n * sizeof(int), cudaMemcpyHostToDevice, st));
+  const double* d = reinterpret_cast<const double*>(buf);
+  sosquad::GlintCorrection t;
+  t.par = d;
+  t.tau = d + n_par;
+  t.beam = t.tau + n_tau;
+  t.w = t.beam + n_beam;
+  t.cphi = t.w + n_w;
+  t.geo = reinterpret_cast<const int*>(buf + dbytes);
+  const long long n_el = static_cast<long long>(n) * n_rows * n_az * (M - 1);
+  sosquad::glint_correction_kernel<<<static_cast<unsigned>((n_el + 127) / 128), 128, 0, st>>>(p->dev.mu, M, N, t, n, n_modes,
+                                                                                           n_rows, n_az, out_d);
+  const int r = launch_check(p, "glint_correction_kernel");
+  SOS_CUDA(cudaFreeAsync(buf, st));
+  return r;
+}
+
 int sos_plan_set_brdf(sos_plan* p, const double* const* Rvol_d, const double* const* Rgeo_d, int n_sets, int ldr) {
-  if (!p || !Rvol_d || !Rgeo_d) return SOS_ERR_INVALID;
+  if (!p || !Rvol_d) return SOS_ERR_INVALID;
   SOS_GUARD(p);
   if (!p->d_brdf_R) return SOS_ERR_UNSUPPORTED;
+  // one matrix per set (ocean) exactly when the second array is absent
+  if ((p->brdf_nk == 1) != (Rgeo_d == nullptr)) return SOS_ERR_INVALID;
   if (n_sets < 1 || n_sets > sosbrdf::MAX_SETS || ldr < p->dev.M - 1) return SOS_ERR_INVALID;
-  std::vector<const double*> ptrs(2 * static_cast<size_t>(n_sets));
+  std::vector<const double*> ptrs(2 * static_cast<size_t>(n_sets), nullptr);
   for (int j = 0; j < n_sets; ++j) {
-    if (!Rvol_d[j] || !Rgeo_d[j]) return SOS_ERR_INVALID;
+    if (!Rvol_d[j] || (Rgeo_d && !Rgeo_d[j])) return SOS_ERR_INVALID;
     ptrs[2 * j] = Rvol_d[j];
-    ptrs[2 * j + 1] = Rgeo_d[j];
+    if (Rgeo_d) ptrs[2 * j + 1] = Rgeo_d[j];
   }
   drop_graphs(p);
   SOS_CUDA(cudaMemcpy(p->d_brdf_R, ptrs.data(), ptrs.size() * sizeof(const double*), cudaMemcpyHostToDevice));
@@ -1262,13 +1352,15 @@ int sos_plan_set_brdf_scenarios(sos_plan* p, const int* set_h, const double* f_h
   if (!p->d_brdf_R) return SOS_ERR_UNSUPPORTED;
   if (p->brdf_sets < 1) return SOS_ERR_STATE;
   const int S = p->dev.S, M = p->dev.M;
+  const bool one = p->brdf_nk == 1;   // ocean: (f_glint, 0), the second beam vector is not read
   for (int s = 0; s < S; ++s) {
     if (set_h[s] < 0 || set_h[s] >= p->brdf_sets) return SOS_ERR_INVALID;
     if (!(f_h[2 * s] >= 0.0 && f_h[2 * s + 1] >= 0.0) || !std::isfinite(f_h[2 * s]) || !std::isfinite(f_h[2 * s + 1])) return SOS_ERR_INVALID;
+    if (one && f_h[2 * s + 1] != 0.0) return SOS_ERR_INVALID;
   }
   const size_t nf = 2 * static_cast<size_t>(S), nb = nf * (M - 1);
   for (size_t k = 0; k < nb; ++k)
-    if (!std::isfinite(beam_h[k])) return SOS_ERR_INVALID;
+    if (!(one && (k / (M - 1)) % 2 == 1) && !std::isfinite(beam_h[k])) return SOS_ERR_INVALID;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   double* d = reinterpret_cast<double*>(p->d_brdf_scen);
   SOS_CUDA(cudaMemcpyAsync(d, f_h, nf * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -1550,8 +1642,14 @@ static int first_order_launch(sos_plan* p, double* I1_d, double* I1_copy_d, cuda
   const int rows_per_block = std::min(64, std::max(8, env_int("SOS_B200_FO_ROWS", 64)));  // (the kernel stages 64 rows at most)
   dim3 grid((g.N + 127) / 128, (g.L + rows_per_block - 1) / rows_per_block, g.S);
   if (p->d_bs) {
-    // diffuse Lambert / Ross-Li ground: the upward radiance of order 1 at the surface row, read by the upward columns
-    sosfirst::first_order_surface_kernel<<<g.S, 128, (g.M + 32) * sizeof(double), st>>>(g, p->d_C, p->d_bs, brdf_dev(p));
+    // diffuse Lambert / Ross-Li / ocean ground: the upward radiance of order 1 at the surface row, read by the upward columns
+    const size_t smem = (g.M + 32) * sizeof(double);
+    if (p->brdf_nk == 2)
+      sosfirst::first_order_surface_kernel<2><<<g.S, 128, smem, st>>>(g, p->d_C, p->d_bs, brdf_dev(p));
+    else if (p->brdf_nk == 1)
+      sosfirst::first_order_surface_kernel<1><<<g.S, 128, smem, st>>>(g, p->d_C, p->d_bs, brdf_dev(p));
+    else
+      sosfirst::first_order_surface_kernel<0><<<g.S, 128, smem, st>>>(g, p->d_C, p->d_bs, brdf_dev(p));
     int r = launch_check(p, "first_order_surface_kernel");
     if (r) return r;
   }
@@ -1890,12 +1988,15 @@ static int sweeps_impl(sos_plan* p, const double* J_d, double* In_d, double* I_d
     if (r) return r;
   } else {
     const size_t smem = (g.N + 32 + 2 * (g.nchunks + 1)) * sizeof(double);
-    if (p->d_brdf_R)
-      sossweep::sweep_carry_kernel<true><<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD,
-                                                                                     p->d_carryU, brdf_dev(p));
+    if (p->brdf_nk == 2)
+      sossweep::sweep_carry_kernel<2><<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD,
+                                                                                  p->d_carryU, brdf_dev(p));
+    else if (p->brdf_nk == 1)
+      sossweep::sweep_carry_kernel<1><<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD,
+                                                                                  p->d_carryU, brdf_dev(p));
     else
-      sossweep::sweep_carry_kernel<false><<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD,
-                                                                                      p->d_carryU, sosbrdf::BrdfDev{});
+      sossweep::sweep_carry_kernel<0><<<g.S, sossweep::CARRY_THREADS, smem, st>>>(g, sg, J_d, p->d_aggD, p->d_aggU, p->d_carryD,
+                                                                                  p->d_carryU, sosbrdf::BrdfDev{});
     int r = launch_check(p, "sweep_carry_kernel");
     if (r) return r;
   }

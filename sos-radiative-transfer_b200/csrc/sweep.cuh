@@ -495,9 +495,10 @@ __device__ __forceinline__ double block_sum(double v, double* scratch /*[32]*/) 
 // ------------------------------------------------------------------------------------------
 // 2. carry chain (one CTA per scenario)
 // ------------------------------------------------------------------------------------------
-// BRDF = true: the Ross-Li ground (SOS_SURFACE_ROSSLI, brdf.cuh), the lambert_readme term with grd_alb = f_iso plus the two
-// kernel mat-vecs; a separate instantiation, so that the kernel of the other surfaces is compiled as without it.
-template <bool BRDF>
+// NK = number of kernel matrices of a bidirectional ground (brdf.cuh): 2 for the Ross-Li ground (SOS_SURFACE_ROSSLI), 1 for
+// the ocean's glint (SOS_SURFACE_OCEAN), each the lambert_readme term with grd_alb as the isotropic part plus NK mat-vecs;
+// 0 for every other surface.  Separate instantiations, so that the kernel of the other surfaces is compiled as without them.
+template <int NK>
 __global__ void __launch_bounds__(CARRY_THREADS)
 sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ J, const double* __restrict__ aggD,
                    const double* __restrict__ aggU, double* __restrict__ carryD, double* __restrict__ carryU,
@@ -573,7 +574,7 @@ sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ 
       part += (g.mu[c1] - g.mu[c0]) * (row[c1] * g.mu[c1] + row[c0] * g.mu[c0]) * 0.5;
     }
     lambert = -2.0 * sc.grd_alb * block_sum(part, scratch);
-  } else if (BRDF || g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE) {
+  } else if (NK > 0 || g.surface == SOS_SURFACE_LAMBERT_README || g.surface == SOS_SURFACE_LAMBERT_DIFFUSE) {
     // README.md:215: -2 rho int_{-1}^{0} I mu dmu with the abscissa ascending and the interval next to mu = 0 included
     double part = 0.0;
     for (int c0 = threadIdx.x; c0 < M - 1; c0 += blockDim.x) {
@@ -583,16 +584,21 @@ sweep_carry_kernel(const GridDev g, const SrcGen sg, const double* __restrict__ 
     lambert = -2.0 * sc.grd_alb * block_sum(part, scratch);
   }
   // seeds into the upper half of the row buffer
-  if constexpr (BRDF) {
+  if constexpr (NK > 0) {
     // the downward half becomes u_c = -2 w_c mu_c I[L-1, c] in place (the up chain reads row[M ..] only); every upward
-    // column adds f_vol sum_c u_c R^vol[c][i] + f_geo sum_c u_c R^geo[c][i] to the isotropic term
+    // column adds f_vol sum_c u_c R^vol[c][i] + f_geo sum_c u_c R^geo[c][i] (Ross-Li) or f_glint sum_c u_c R[c][i] (ocean)
+    // to the isotropic term
     for (int c = threadIdx.x; c < M; c += blockDim.x) row[c] *= sosbrdf::coupling_weight(g.mu, M, c);
     __syncthreads();
     const double fv = brdf.f[2 * s], fg = brdf.f[2 * s + 1];
     for (int m = M + 1 + threadIdx.x; m < N; m += blockDim.x) {
-      double sv, sgeo;
-      sosbrdf::coupling(brdf, s, row, M, m - M - 1, sv, sgeo);
-      row[m] = lambert + (fv * sv + fg * sgeo);
+      if constexpr (NK == 2) {
+        double sv, sgeo;
+        sosbrdf::coupling(brdf, s, row, M, m - M - 1, sv, sgeo);
+        row[m] = lambert + (fv * sv + fg * sgeo);
+      } else {
+        row[m] = lambert + fv * sosbrdf::coupling(brdf, s, row, M, m - M - 1);
+      }
     }
   } else {
     for (int m = M + 1 + threadIdx.x; m < N; m += blockDim.x) {

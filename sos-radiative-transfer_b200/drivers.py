@@ -17,6 +17,7 @@ import torch
 
 from . import _lib
 from . import brdf as BR
+from . import ocean as OC
 from . import grid as G
 from . import phase as PH
 from .engine import ScenarioCoefficients, SosEngine
@@ -50,11 +51,15 @@ class Scenario:
     # isotropically, no mirror beam; n >= 2 as 'lambert_readme'; the fluxes carry no collimated reflected beam)
     # | 'rossli' (a Ross-Li bidirectional ground in every order, brdf module: grd_alb is f_iso and the 'lambert_diffuse'
     # coupling, brdf_vol / brdf_geo weight the RossThick / LiSparse-R kernels; no collimated reflected beam)
+    # | 'ocean' (a wind-roughened sea in every order, ocean module: grd_alb is the isotropic part and the 'lambert_diffuse'
+    # coupling, plus the Cox-Munk glint of wind_speed / ocean_index; no collimated reflected beam)
     surface: str = "specular"
     threshold: float = 1e-4
     max_orders: int = 10000
     brdf_vol: float = 0.0   # Ross-Li kernel weights f_vol, f_geo (>= 0; surface='rossli' only)
     brdf_geo: float = 0.0
+    wind_speed: Optional[float] = None   # m/s, >= 0 (surface='ocean' only, where it is required)
+    ocean_index: float = 1.34            # relative refractive index of the sea (> 1; surface='ocean')
 
 
 # README scenarios (README.md:95-111) -- tau_atm 0.124, omega_aer 0.97, R_s 0.15
@@ -120,12 +125,17 @@ _PHASES = PhaseCache()
 _MODE_STACKS = {}   # device-built mode stacks (P_0 .. P_{K-1}) per (family, g, grid, n_quad, device), see _DeviceBuilt
 _BRDF_STACKS = {}   # device-built Ross-Li mode matrices (2, K, M, ldr) per (grid, device), see BatchSolver._send_brdf
 _BRDF_BEAMS = {}    # host beam vectors (2, K, M-1) per (grid, mu0, K)
+_GLINT_STACKS = {}  # device-built glint mode matrices (K, M, ldr) per (grid, device, W, n), see BatchSolver._send_brdf
+_GLINT_BEAMS = {}   # host glint beam vectors (K, M-1) per (grid, mu0, W, n, K)
+_GLINT_STACKS_MAX = 8   # at M = 501 a 64-mode stack is about 130 MB
 # surfaces that reflect the direct beam into the diffuse field: the fluxes carry no collimated reflected beam
-DIFFUSE_GROUNDS = ("lambert_diffuse", "rossli")
+DIFFUSE_GROUNDS = ("lambert_diffuse", "rossli", "ocean")
+MAX_BRDF_SETS_PER_PLAN = 64   # mode matrix sets one plan registers (sosbrdf::MAX_SETS, sos_plan_set_brdf)
 
 
 def check_brdf(scenarios: Sequence[Scenario]):
-    """ValueError for Ross-Li weights that are negative (or not finite) or given on a surface other than 'rossli'."""
+    """ValueError for Ross-Li weights that are negative (or not finite) or given on a surface other than 'rossli', and for
+    an ocean without a finite wind_speed >= 0 and a finite ocean_index > 1, or a wind_speed on another surface."""
     for sc in scenarios:
         fv, fg = float(sc.brdf_vol), float(sc.brdf_geo)
         if not (np.isfinite(fv) and np.isfinite(fg) and fv >= 0 and fg >= 0):
@@ -133,6 +143,30 @@ def check_brdf(scenarios: Sequence[Scenario]):
         if sc.surface != "rossli" and (fv != 0 or fg != 0):
             raise ValueError(f"brdf_vol / brdf_geo weight the Ross-Li kernels: surface={sc.surface!r} takes none "
                              "(use surface='rossli')")
+        if sc.surface == "ocean":
+            W, n = sc.wind_speed, float(sc.ocean_index)
+            if W is None or not (np.isfinite(float(W)) and float(W) >= 0):
+                raise ValueError(f"surface='ocean' needs a finite wind_speed >= 0 in m/s (wind_speed={W})")
+            if not (np.isfinite(n) and n > 1):
+                raise ValueError(f"surface='ocean' needs a finite ocean_index > 1 (ocean_index={n})")
+        elif sc.wind_speed is not None:
+            raise ValueError(f"wind_speed drives the ocean glint: surface={sc.surface!r} takes none (use surface='ocean')")
+
+
+def _glint_key(sc: Scenario, m: int = 0):
+    """The glint mode matrix set of an ocean scenario coupled in azimuthal mode m: (W, n, m)."""
+    return (float(sc.wind_speed), float(sc.ocean_index), int(m))
+
+
+def glint_beam(M: int, mu: np.ndarray, sc: Scenario, n_modes: int) -> np.ndarray:
+    """The scenario's glint beam vectors of modes 0 .. n_modes-1, (n_modes, M-1) (ocean.glint_beam, cached)."""
+    key = (M, float(sc.mu0), float(sc.wind_speed), float(sc.ocean_index), int(n_modes))
+    b = _GLINT_BEAMS.get(key)
+    if b is None:
+        if len(_GLINT_BEAMS) >= 4096:
+            _GLINT_BEAMS.clear()
+        b = _GLINT_BEAMS[key] = OC.glint_beam(M, mu, sc.mu0, sc.wind_speed, sc.ocean_index, n_modes)
+    return b
 
 
 def clear_caches(disk: bool = False):
@@ -144,7 +178,7 @@ def clear_caches(disk: bool = False):
     _PHASES._P.clear()
     _PHASES._P0.clear()
     api.clear_cache()
-    for d in (E._OPERANDS, E._FOLDED, E._LOWRANK, _BRDF_STACKS, _BRDF_BEAMS):
+    for d in (E._OPERANDS, E._FOLDED, E._LOWRANK, _BRDF_STACKS, _BRDF_BEAMS, _GLINT_STACKS, _GLINT_BEAMS):
         d.clear()
     mie.lognormal_table.cache_clear()
     if disk:
@@ -192,9 +226,10 @@ class BatchSolver:
                  device_phase: bool = True, fold: Optional[bool] = None, order_caps: Optional[Sequence[int]] = None,
                  brdf_modes: Optional[Sequence[int]] = None):
         """order_caps: per scenario, sum exactly orders 1 .. cap instead of stopping on the threshold (0 = the threshold;
-        sos_scenario.order_cap); None = all 0.  brdf_modes (surface 'rossli'): per scenario, the azimuthal Fourier mode of
-        the Ross-Li ground it is coupled with (0 .. 63; None = all 0, the azimuth average).  update() takes both for the
-        next batch the same way."""
+        sos_scenario.order_cap); None = all 0.  brdf_modes (surface 'rossli' or 'ocean'): per scenario, the azimuthal Fourier
+        mode of the Ross-Li kernels or of the glint it is coupled with (0 .. 63; None = all 0, the azimuth average).  An ocean
+        batch registers one glint matrix set per distinct (wind_speed, ocean_index, mode): at most 64
+        (split_for_plan_limits cuts larger groups).  update() takes both for the next batch the same way."""
         keys = {_group_key(s) for s in scenarios}
         if len(keys) != 1:
             raise ValueError("BatchSolver: scenarios must share nb_layers, nb_angles, aerosol rows and surface")
@@ -209,22 +244,24 @@ class BatchSolver:
         coefs = self._prepare(scenarios, order_caps)
         surface = {"specular": _lib.SURFACE_SPECULAR, "lambert": _lib.SURFACE_LAMBERT,
                    "lambert_readme": _lib.SURFACE_LAMBERT_README, "lambert_diffuse": _lib.SURFACE_LAMBERT_DIFFUSE,
-                   "rossli": _lib.SURFACE_ROSSLI}[surf]
+                   "rossli": _lib.SURFACE_ROSSLI, "ocean": _lib.SURFACE_OCEAN}[surf]
         self.engine = SosEngine(self.mu, self.tau, coefs, [0, self.idx_up, self.idx_down + 1, L], surface,
                                 device=device, chunk_rows=chunk_rows, fold=fold)
         self._register_phases()
         self._brdf_sets = None
-        if surf == "rossli":
+        if surf in ("rossli", "ocean"):
             self._send_brdf(brdf_modes)
         self.I1 = None
 
     def _send_brdf(self, brdf_modes):
-        """Ross-Li plan: register the mode matrix pairs the batch uses (when they change) and send every scenario's pair
-        index, weights and beam vectors."""
+        """Ross-Li / ocean plan: register the mode matrix sets the batch uses (when they change) and send every scenario's
+        set index, weights and beam vectors."""
         S, M = len(self.scenarios), self.M
         modes = np.zeros(S, dtype=np.int64) if brdf_modes is None else np.asarray(brdf_modes, dtype=np.int64)
         if modes.shape != (S,) or np.any(modes < 0) or np.any(modes >= 64):
             raise ValueError("BatchSolver: brdf_modes must give one mode in [0, 64) per scenario")
+        if self._key[4] == "ocean":
+            return self._send_glint(modes)
         wanted = sorted(set(modes.tolist()))
         K = wanted[-1] + 1
         eng = self.engine
@@ -249,6 +286,39 @@ class BatchSolver:
             beams[s] = b[:, modes[s]]
         eng.set_brdf_scenarios(np.array([index[m] for m in modes.tolist()]),
                                np.array([[sc.brdf_vol, sc.brdf_geo] for sc in self.scenarios], dtype=np.float64), beams)
+
+    def _send_glint(self, modes):
+        """Ocean plan: one glint matrix per distinct (W, n, mode) of the batch, weights (1, 0) and the glint beam vectors."""
+        S, M = len(self.scenarios), self.M
+        keys = [_glint_key(sc, m) for sc, m in zip(self.scenarios, modes.tolist())]
+        wanted = sorted(set(keys))
+        if len(wanted) > MAX_BRDF_SETS_PER_PLAN:
+            raise ValueError(f"BatchSolver: {len(wanted)} distinct (wind_speed, ocean_index, mode) glint sets; one plan "
+                             f"takes {MAX_BRDF_SETS_PER_PLAN} (split_for_plan_limits cuts the batch)")
+        eng = self.engine
+        if self._brdf_sets is None or not set(wanted) <= set(self._brdf_sets):
+            need = {}
+            for W, n, m in wanted:
+                need[(W, n)] = max(need.get((W, n), 0), m + 1)
+            stacks = {}
+            for (W, n), K in need.items():
+                key = (eng.mu.tobytes(), eng.device.index, W, n)
+                stack = _GLINT_STACKS.get(key)
+                if stack is None or stack.shape[0] < K:
+                    if len(_GLINT_STACKS) >= _GLINT_STACKS_MAX:
+                        _GLINT_STACKS.pop(next(iter(_GLINT_STACKS)))   # (a registered set keeps its stack alive in the engine)
+                    stack = _GLINT_STACKS[key] = eng.build_glint_modes(W, n, n_modes=K if K == 1 else min(64, (K + 7) // 8 * 8))
+                stacks[(W, n)] = stack
+            eng.set_brdf([stacks[(W, n)][m] for W, n, m in wanted])
+            self._brdf_sets = wanted
+        index = {k: j for j, k in enumerate(self._brdf_sets)}
+        K = int(modes.max()) + 1
+        beams = np.zeros((S, 2, M - 1))
+        for s, sc in enumerate(self.scenarios):
+            beams[s, 0] = glint_beam(M, self.mu, sc, K)[modes[s]]
+        weights = np.zeros((S, 2))
+        weights[:, 0] = 1.0
+        eng.set_brdf_scenarios(np.array([index[k] for k in keys]), weights, beams)
 
     def _prepare(self, scenarios, order_caps=None):
         """Host side of a batch: tau profiles, per-scenario scalars, the table of distinct solar phase vectors with the rows
@@ -361,7 +431,7 @@ class BatchSolver:
                 raise ValueError("BatchSolver.update: more than 16 phase functions in one plan")
             self._register_phases()          # a phase function met for the first time: register the larger operand set
         self.engine.update(self.tau, coefs)
-        if self._key[4] == "rossli":
+        if self._key[4] in ("rossli", "ocean"):
             self._send_brdf(brdf_modes)
 
     def first_order(self, also_into=None):
@@ -403,7 +473,7 @@ class BatchSolver:
             # TOA net flux with the F0/(4 pi) direct scaling (SOS_Aer_critical_albedo.py:377-382): same quadrature sums, direct
             # terms rescaled from F0 to F0/(4 pi) -- for the whole batch at once
             mu0 = np.array([sc.mu0 for sc in self.scenarios], dtype=np.float64)
-            # (a diffuse Lambert or Ross-Li ground reflects the beam into the field: no collimated reflected term)
+            # (a diffuse Lambert, Ross-Li or ocean ground reflects the beam into the field: no collimated reflected term)
             alb = np.array([0.0 if sc.surface in DIFFUSE_GROUNDS else sc.grd_alb for sc in self.scenarios], dtype=np.float64)
             k = (np.pi / mu0) * (1.0 - 1.0 / (4 * np.pi))
             t0, tl = self.tau[:, 0], self.tau[:, -1]
@@ -444,21 +514,25 @@ def _phase_id(spec):
     return spec if isinstance(spec[0], str) else ("array", id(spec[1]))
 
 
-def split_for_plan_limits(scenarios: Sequence[Scenario], idxs: Sequence[int], max_phases: int = MAX_PHASES_PER_PLAN) -> List[List[int]]:
-    """Cut one grid group into sub-batches a plan accepts: at most 16 (max_phases) distinct phase matrices and 48 (atm, aer)
-    operand pairs each (a phase sweep over more than 16 HG asymmetry factors, or per-scenario Mie arrays, would otherwise
-    be refused by sos_plan_create).  Order inside the group is kept."""
-    out, cur, phases, pairs = [], [], set(), set()
+def split_for_plan_limits(scenarios: Sequence[Scenario], idxs: Sequence[int], max_phases: int = MAX_PHASES_PER_PLAN,
+                          brdf_modes: Optional[Sequence[int]] = None) -> List[List[int]]:
+    """Cut one grid group into sub-batches a plan accepts: at most 16 (max_phases) distinct phase matrices, 48 (atm, aer)
+    operand pairs and 64 ocean glint sets (distinct (wind_speed, ocean_index, mode); brdf_modes: the mode of every scenario,
+    None = 0) each (a phase sweep over more than 16 HG asymmetry factors, per-scenario Mie arrays or a wind-speed sweep would
+    otherwise be refused by the plan).  Order inside the group is kept."""
+    out, cur, phases, pairs, sets = [], [], set(), set(), set()
     for i in idxs:
         sc = scenarios[i]
         pa, pe = _phase_id(sc.atm_phase), _phase_id(sc.aer_phase)
+        gs = {_glint_key(sc, brdf_modes[i] if brdf_modes is not None else 0)} if sc.surface == "ocean" else set()
         new_phases = phases | {pa, pe}
         new_pairs = pairs | {(pa, pe), (pa, None)}
-        if cur and (len(new_phases) > max_phases or len(new_pairs) > MAX_GROUPS_PER_PLAN):
+        new_sets = sets | gs
+        if cur and (len(new_phases) > max_phases or len(new_pairs) > MAX_GROUPS_PER_PLAN or len(new_sets) > MAX_BRDF_SETS_PER_PLAN):
             out.append(cur)
-            cur, new_phases, new_pairs = [], {pa, pe}, {(pa, pe), (pa, None)}
+            cur, new_phases, new_pairs, new_sets = [], {pa, pe}, {(pa, pe), (pa, None)}, gs
         cur.append(i)
-        phases, pairs = new_phases, new_pairs
+        phases, pairs, sets = new_phases, new_pairs, new_sets
     if cur:
         out.append(cur)
     return out

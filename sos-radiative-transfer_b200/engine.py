@@ -436,23 +436,28 @@ class SosEngine:
         return R
 
     def set_brdf(self, pairs: Sequence):
-        """Register the mode matrix pairs of a Ross-Li plan (sos_plan_set_brdf): pairs[j] = (vol, geo), two (M, ldr) device
-        tensors in the layout of build_brdf_modes (e.g. R[0, m], R[1, m]); the engine keeps them alive."""
-        if not pairs:
-            raise ValueError("set_brdf: at least one mode matrix pair")
-        ldr = pairs[0][0].shape[-1]
-        for P in (t for pair in pairs for t in pair):
+        """Register the mode matrix sets of a Ross-Li or ocean plan (sos_plan_set_brdf): for Ross-Li pairs[j] = (vol, geo),
+        two (M, ldr) device tensors in the layout of build_brdf_modes (e.g. R[0, m], R[1, m]); for the ocean pairs[j] = one
+        (M, ldr) glint matrix of build_glint_modes (e.g. R[m]).  The engine keeps them alive."""
+        if not len(pairs):
+            raise ValueError("set_brdf: at least one mode matrix set")
+        sets = [(p,) if isinstance(p, torch.Tensor) else tuple(p) for p in pairs]
+        ldr = sets[0][0].shape[-1]
+        for P in (t for st in sets for t in st):
             if P.shape != (self.M, ldr) or P.dtype != torch.float64 or not P.is_contiguous() or P.device != self.device:
                 raise ValueError("set_brdf: every matrix must be a contiguous float64 (M, ldr) tensor on the plan's device")
-        self._brdf = [tuple(pair) for pair in pairs]
-        vol = (C.c_void_p * len(pairs))(*[pair[0].data_ptr() for pair in pairs])
-        geo = (C.c_void_p * len(pairs))(*[pair[1].data_ptr() for pair in pairs])
+        if len({len(st) for st in sets}) != 1:
+            raise ValueError("set_brdf: every set has the same number of matrices")
+        self._brdf = sets
+        vol = (C.c_void_p * len(sets))(*[st[0].data_ptr() for st in sets])
+        geo = (C.c_void_p * len(sets))(*[st[1].data_ptr() for st in sets]) if len(sets[0]) > 1 else None
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.sos_plan_set_brdf(self._plan, vol, geo, len(pairs), int(ldr)), "sos_plan_set_brdf")
+            _lib.check(self.lib.sos_plan_set_brdf(self._plan, vol, geo, len(sets), int(ldr)), "sos_plan_set_brdf")
 
     def set_brdf_scenarios(self, sets: np.ndarray, weights: np.ndarray, beams: np.ndarray):
-        """Per-scenario Ross-Li data (sos_plan_set_brdf_scenarios): sets (S,) pair index, weights (S, 2) = (f_vol, f_geo),
-        beams (S, 2, M-1) = the beam vectors of the scenario's mode.  Rewritten in place: captured graphs stay valid."""
+        """Per-scenario Ross-Li / ocean data (sos_plan_set_brdf_scenarios): sets (S,) set index, weights (S, 2) = (f_vol, f_geo)
+        or (f_glint, 0), beams (S, 2, M-1) = the beam vectors of the scenario's mode (the ocean's second is not read).
+        Rewritten in place: captured graphs stay valid."""
         st = np.ascontiguousarray(sets, dtype=np.int32)
         f = np.ascontiguousarray(weights, dtype=np.float64)
         b = np.ascontiguousarray(beams, dtype=np.float64)
@@ -461,6 +466,49 @@ class SosEngine:
         with torch.cuda.device(self.device):
             _lib.check(self.lib.sos_plan_set_brdf_scenarios(self._plan, st.ctypes.data, f.ctypes.data, b.ctypes.data, self._stream),
                        "sos_plan_set_brdf_scenarios")
+
+    # ------------------------------------------------------------------ ocean
+    def build_glint_modes(self, wind_speed: float, n_ref: float = 1.34, n_modes: int = 1,
+                          n_quad: Optional[int] = None) -> torch.Tensor:
+        """Fourier modes 0 .. n_modes-1 of the Cox-Munk glint at wind speed W (m/s) and relative refractive index n_ref on
+        this grid, built ON THE DEVICE (sos_build_glint_modes): a (n_modes, M, ldr) tensor, [m][c][i] =
+        rho_m(mu[M+1+i], |mu[c]|) (the transposed layout the coupling reads; ldr = M-1 rounded up to even).
+        ocean.glint_modes is the NumPy reference ([m][i][c])."""
+        from . import brdf as BR, ocean as OC
+        K, nq = int(n_modes), int(n_quad if n_quad is not None else BR.BRDF_NODES)
+        M = self.M
+        ldr = _align(M - 1, 2)
+        R = torch.zeros((K, M, ldr), dtype=torch.float64, device=self.device)
+        phi, tab = BR.node_table(nq, K)
+        tab[0] = np.cos(phi)   # (the glint takes cos phi itself: it sits at phi = 0)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_build_glint_modes(self._plan, nq, phi.ctypes.data, tab.ctypes.data, K,
+                                                      float(OC.slope_variance(wind_speed)), float(n_ref), R.data_ptr(), ldr,
+                                                      M * ldr, self._stream), "sos_build_glint_modes")
+            torch.cuda.current_stream(self.device).synchronize()   # (phi / tab are host temporaries)
+        return R
+
+    def glint_correction(self, out: torch.Tensor, geo: np.ndarray, params: np.ndarray, tau_rows: np.ndarray, beams: np.ndarray,
+                         phi: np.ndarray):
+        """Exact direct glint of azimuth-resolved radiance (sos_glint_correction): out (n_geo, n_rows, n_az, N) as written by
+        azimuth_synthesis; per entry k: geo[k] its geometry, params[k] = (mu0, tauStar_tot, sigma^2, n_ref), tau_rows[k] tau at
+        the rows, beams[k] (n_modes, M-1) the glint beam vectors of the modes summed into out."""
+        ge = np.ascontiguousarray(geo, dtype=np.int32)
+        par = np.ascontiguousarray(params, dtype=np.float64)
+        tr = np.ascontiguousarray(tau_rows, dtype=np.float64)
+        b = np.ascontiguousarray(beams, dtype=np.float64)
+        ph = np.ascontiguousarray(phi, dtype=np.float64)
+        n = ge.size
+        n_geo, n_rows, n_az = out.shape[:3]
+        if (par.shape != (n, 4) or tr.shape != (n, n_rows) or b.ndim != 3 or b.shape[0] != n or b.shape[2] != self.M - 1
+                or ph.shape != (n_az,) or out.shape[3] != self.N or not out.is_contiguous()):
+            raise ValueError("glint_correction: shapes do not match the plan")
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_glint_correction(self._plan, n, ge.ctypes.data, par.ctypes.data, tr.ctypes.data, n_rows,
+                                                     b.ctypes.data, b.shape[1], ph.ctypes.data, n_az, n_geo, out.data_ptr(),
+                                                     self._stream), "sos_glint_correction")
+            torch.cuda.current_stream(self.device).synchronize()   # (the host tables are temporaries)
+        return out
 
     def azimuth_synthesis(self, I: torch.Tensor, geo: np.ndarray, weights: np.ndarray, n_geo: int, rows: Sequence[int],
                           out: torch.Tensor, accumulate: bool):
