@@ -226,6 +226,35 @@ int sos_glint_correction(sos_plan* plan, int n, const int* geo_h, const double* 
                          const double* beam_h, int n_modes, const double* phi_h, int n_az, int n_geo, double* out_d,
                          void* stream);
 
+/* Exact single scattering of azimuth-resolved radiance (three-region plans; SOS_ERR_UNSUPPORTED otherwise).  The first order
+ * of sos_first_order is linear in its coefficient planes; for entries k = 0 .. n-1 (a plan scenario and the geometry it was
+ * synthesized into), requested rows r (rows_h [n_rows] in [0, L)), azimuths p and every column of the plan's grid it adds
+ *   out[geo][r][p][col] += I1[dC](tau[scenario][rows_h[r]], mu_col)
+ * (out as written by sos_azimuth_synthesis, [n_geo][n_rows][n_az][N]): the closed-form first order of the plan's scenario with
+ * the coefficient planes dC_atm = alb_atm dP0_atm, dC_mix = dC_atm f_atm + (dP0_aer alb_aer) f_aer built from
+ *   dP0(mu, phi_p) = p(cos Theta) / norm - sum_{m < n_modes} (2 - delta_m0) P0m[series][m](mu) cos(m phi_p),
+ *   cos Theta = -mu0 mu + sqrt(1 - mu0^2) sqrt(1 - mu^2) cos phi_p,
+ * i.e. the truncated Fourier series of the singly scattered radiance replaced by its exact value.  Over a specular ground
+ * (and the Lambert kinds) the mirror-reflected beam and the upward carry rho I1[L-1, mirror] are kept; over
+ * SOS_SURFACE_LAMBERT_DIFFUSE, SOS_SURFACE_ROSSLI and SOS_SURFACE_OCEAN both are 0 (their order-1 surface terms stay the
+ * series).  P0m_h [n_vec][n_modes][N]: the solar mode vectors the radiance was summed with (1 <= n_modes <= 64);
+ * tab_h [n_tab]: the tabulated phase functions, abscissae (ascending) at tab_off and values at tab_off + tab_n; phi_h [n_az].
+ * One thread per (entry, azimuth, column), no atomics: deterministic. */
+typedef struct {
+  int scenario;         /* plan scenario (tau, mu0, tauStar_tot, grd_alb) */
+  int geo;              /* first index of out */
+  int family[2];        /* atmosphere, aerosol: -1 isotropic (dP0 = 0), 0 Rayleigh, 1 Henyey-Greenstein, 2 tabulated */
+  int series[2];        /* row of P0m_h */
+  int tab_off[2];       /* tabulated: offset of the abscissae in tab_h */
+  int tab_n[2];         /* tabulated: number of abscissae */
+  double g[2];          /* Henyey-Greenstein asymmetry */
+  double norm[2];       /* T > 0: the mode-0 normalisation, trapz_mu of the azimuth ring integral / (4 pi) */
+  double w[4];          /* alb_atm, f_atm, alb_aer, f_aer */
+} sos_ss_entry;
+int sos_single_scatter_correction(sos_plan* plan, int n, const sos_ss_entry* ent_h, const double* P0m_h, int n_vec, int n_modes,
+                                  const double* tab_h, int n_tab, const int* rows_h, int n_rows, const double* phi_h, int n_az,
+                                  int n_geo, double* out_d, void* stream);
+
 /* Register the contraction matrices (device, [N][lda] each) the scenarios index. */
 int sos_plan_set_phase(sos_plan* plan, const double* const* A_d, int n_matrices, int lda);
 

@@ -11,7 +11,7 @@ the repository root) or with importlib.import_module("sos-radiative-transfer_b20
 from . import _lib
 from ._lib import SosError
 from .grid import mu_grid, tau_profile, extrapolation_width, aerosol_rows
-from .phase import phase_matrices, phase_P, phase_P0, phase_table, phase_modes
+from .phase import phase_matrices, phase_P, phase_P0, phase_table, phase_modes, phase_exact
 from . import brdf
 from .brdf import BRDF_NODES, BRDF_MU_MIN, rossli_kernels, brdf_modes, brdf_beam
 from . import ocean
@@ -31,7 +31,7 @@ from .drivers import (Scenario, DriverResult, BatchSolver, solve_scenarios, SOS_
 from .azimuth import AzimuthalResult, solve_azimuthal
 
 __all__ = [
-    "SosError", "mu_grid", "tau_profile", "extrapolation_width", "aerosol_rows", "phase_matrices", "phase_P", "phase_P0", "phase_table", "phase_modes",
+    "SosError", "mu_grid", "tau_profile", "extrapolation_width", "aerosol_rows", "phase_matrices", "phase_P", "phase_P0", "phase_table", "phase_modes", "phase_exact",
     "brdf", "BRDF_NODES", "BRDF_MU_MIN", "rossli_kernels", "brdf_modes", "brdf_beam", "ocean", "cox_munk", "glint_modes", "glint_beam", "mie", "EVA_AEROSOL", "WILDFIRE_AEROSOL",
     "SosEngine", "ScenarioCoefficients", "SolveResult", "I1_NumInt", "Jn_NumInt", "In_NumInt",
     "mu_approx_In", "clear_cache", "Scenario", "DriverResult", "BatchSolver", "solve_scenarios",

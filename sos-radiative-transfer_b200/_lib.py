@@ -59,6 +59,12 @@ SCENARIO_DTYPE = np.dtype([("mu0", "f8"), ("grd_alb", "f8"), ("tauStar_tot", "f8
 assert SCENARIO_DTYPE.itemsize == C.sizeof(sos_scenario)
 
 
+# one entry of sos_single_scatter_correction (sos_ss_entry): 104 bytes, marshalled as a NumPy record array
+SS_ENTRY_DTYPE = np.dtype([("scenario", "i4"), ("geo", "i4"), ("family", "i4", 2), ("series", "i4", 2), ("tab_off", "i4", 2),
+                           ("tab_n", "i4", 2), ("g", "f8", 2), ("norm", "f8", 2), ("w", "f8", 4)])
+assert SS_ENTRY_DTYPE.itemsize == 104
+
+
 class sos_result(C.Structure):
     _fields_ = [
         ("ratio_toa", C.c_double),
@@ -96,6 +102,8 @@ SIGNATURES = {
     "sos_plan_set_brdf_scenarios": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "sos_build_glint_modes": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_double, C.c_double, _vp, C.c_int, C.c_size_t, _vp]),
     "sos_glint_correction": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_int, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp]),
+    "sos_single_scatter_correction": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_int, _vp, C.c_int, _vp, C.c_int, _vp, C.c_int,
+                                                C.c_int, _vp, _vp]),
     "sos_azimuth_synthesis": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, _vp]),
     "sos_plan_set_phase": (C.c_int, [_vp, C.POINTER(_vp), C.c_int, C.c_int]),
     "sos_fold_layout": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),

@@ -14,7 +14,10 @@ orders its mode 0 summed (sos_scenario.order_cap), and
 
 is summed on the device (sos_azimuth_synthesis).  Over an ocean the radiance also gets the once-reflected direct beam in
 closed form (sos_glint_correction): the glint lobe is too narrow in azimuth for 64 modes at low wind, so its truncated
-series is replaced by the exact reflectance on every upward column.
+series is replaced by the exact reflectance on every upward column.  With single_scatter='exact' the radiance also gets the
+singly scattered light in closed form (sos_single_scatter_correction): a K-term series cannot follow a sharply peaked phase
+function, and the first order's angular shape is the phase function, so its truncated series is replaced by the closed-form
+first order of p(cos Theta) / T at every azimuth (DESIGN section 13).
 
 phi is the azimuth of the PROPAGATION direction of the diffuse light relative to the propagation azimuth of the solar beam:
 with the grid's signs (mu < 0 downward) the beam travels along (-mu0, 0), cos Theta = -mu0 mu + sqrt(1 - mu0^2) sqrt(1 - mu^2)
@@ -29,9 +32,10 @@ from typing import List, Optional, Sequence
 import numpy as np
 import torch
 
+from . import _lib
 from . import phase as PH
 from . import ocean as OC
-from .drivers import (DriverResult, MAX_PHASES_PER_PLAN, BatchSolver, Scenario, _BRDF_STACKS, _GLINT_STACKS, _MODE_STACKS,
+from .drivers import (DriverResult, MAX_PHASES_PER_PLAN, BatchSolver, Scenario, _BRDF_STACKS, _GLINT_STACKS, _MODE_STACKS, _PHASES,
                       check_brdf, glint_beam, grid_groups, solved_batches, split_for_plan_limits)
 
 # phase functions per plan of the mode members (two per mode: typically 8 modes per plan)
@@ -44,7 +48,8 @@ class AzimuthalResult:
     at the layers `rows` and azimuths `phi` (over an ocean with the exact direct glint: the once-reflected, unscattered beam
     in closed form instead of its truncated series); modes (n_modes, n_rows, N): the Fourier components I_m at those layers
     (the truncated series, order for order; mode 0 = base.I rows); mode_orders / mode_status (n_modes,): orders summed and
-    status bits of every mode (a mode whose atmosphere and aerosol modes vanish is not solved: 0 orders, I_m = 0)."""
+    status bits of every mode (a mode whose atmosphere and aerosol modes vanish is not solved: 0 orders, I_m = 0);
+    single_scatter: 'series' (radiance is the truncated series) or 'exact' (its first order by the phase function is exact)."""
     base: DriverResult
     radiance: np.ndarray
     rows: np.ndarray
@@ -53,6 +58,7 @@ class AzimuthalResult:
     modes: np.ndarray
     mode_orders: np.ndarray
     mode_status: np.ndarray
+    single_scatter: str = "series"
 
 
 def _mode_spec(spec, m: int, n_quad: int):
@@ -64,8 +70,13 @@ def _vanishes(spec, m: int) -> bool:
     return PH.mode_vanishes(PH.resolve(spec[0], spec[1] if len(spec) > 1 else None)[0], m)
 
 
-def _validate(scenarios: Sequence[Scenario], n_modes: int, n_quad: int):
+SINGLE_SCATTER = ("series", "exact")
+
+
+def _validate(scenarios: Sequence[Scenario], n_modes: int, n_quad: int, single_scatter: str = "series"):
     check_brdf(scenarios)
+    if single_scatter not in SINGLE_SCATTER:
+        raise ValueError(f"solve_azimuthal: single_scatter must be one of {SINGLE_SCATTER}, not {single_scatter!r}")
     if n_modes < 1:
         raise ValueError("solve_azimuthal: n_modes must be >= 1")
     if n_quad < 2 * n_modes:
@@ -81,7 +92,7 @@ def _validate(scenarios: Sequence[Scenario], n_modes: int, n_quad: int):
 
 
 def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -1), n_quad: int = 25,
-                    device=None) -> List[AzimuthalResult]:
+                    device=None, single_scatter: str = "series") -> List[AzimuthalResult]:
     """Radiance as a function of azimuth for every scenario: modes 0 .. n_modes-1, synthesized at the azimuths `phi`
     (radians, see the module docstring for the convention) on the layers `rows` (negative = from the bottom).
 
@@ -93,10 +104,16 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
     its kernel modes, which are integrated on brdf.BRDF_NODES nodes whatever n_quad; so does an 'ocean' through its glint
     modes, and its radiance includes the exact direct glint (the once-reflected beam transmitted without scattering, in closed
     form instead of its n_modes-term series; `modes` and `base` stay the truncated series).  'lambert' / 'lambert_readme'
-    surfaces with grd_alb > 0 and caller-supplied (P0, P) arrays raise ValueError before any device work."""
+    surfaces with grd_alb > 0 and caller-supplied (P0, P) arrays raise ValueError before any device work.
+
+    single_scatter='exact' replaces the n_modes-term series of the singly scattered radiance (the first order by the phase
+    function: the direct beam and, over a specular ground, the mirror-reflected beam) by its closed form with the exact
+    p(cos Theta) / T at every azimuth, T the mode-0 normalisation at n_quad nodes (phase.phase_exact).  The surface terms of
+    the first order over 'lambert_diffuse', 'rossli' and 'ocean' grounds stay the series; `modes` and `base` do too.  The
+    default 'series' returns the truncated series; any other value raises ValueError before any device work."""
     scenarios = list(scenarios)
     K, n_quad = int(n_modes), int(n_quad)
-    _validate(scenarios, K, n_quad)
+    _validate(scenarios, K, n_quad, single_scatter)
     phi = np.atleast_1d(np.asarray(phi, dtype=np.float64))
     if phi.ndim != 1:
         raise ValueError("solve_azimuthal: phi must be a 1-D sequence of azimuths")
@@ -125,6 +142,8 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
                                       radiance, accumulate=False)
                 if scenarios[idxs[0]].surface == "ocean":
                     _glint_correction(eng, bs, [scenarios[i] for i in idxs], [pos[i] for i in idxs], rws, K, phi, radiance)
+                if single_scatter == "exact":
+                    _single_scatter_correction(eng, bs, [pos[i] for i in idxs], rws, K, n_quad, phi, radiance)
                 for i, r in zip(idxs, results):
                     base[i], n0[i] = r, int(r.n)
                     modes[i][0] = r.I[rws]
@@ -166,7 +185,8 @@ def solve_azimuthal(scenarios: Sequence[Scenario], phi, n_modes: int, rows=(0, -
             rad = radiance.cpu().numpy()
             for i in group:
                 out[i] = AzimuthalResult(base=base[i], radiance=rad[pos[i]], rows=rws.copy(), phi=phi.copy(), n_modes=K,
-                                         modes=modes[i], mode_orders=orders[i], mode_status=status[i])
+                                         modes=modes[i], mode_orders=orders[i], mode_status=status[i],
+                                         single_scatter=single_scatter)
     finally:
         _MODE_STACKS.clear()   # the device mode stacks serve the sub-batches of one call
         _BRDF_STACKS.clear()
@@ -183,3 +203,47 @@ def _glint_correction(eng, bs: BatchSolver, scs: Sequence[Scenario], geo: Sequen
                     for sc in scs], dtype=np.float64)
     beams = np.stack([glint_beam(M, bs.mu, sc, K) for sc in scs])
     eng.glint_correction(radiance, np.asarray(geo), par, bs.tau[:, rws], beams, phi)
+
+
+def _single_scatter_correction(eng, bs: BatchSolver, geo: Sequence[int], rws: np.ndarray, K: int, n_quad: int, phi: np.ndarray,
+                               radiance: torch.Tensor):
+    """Replace the K-term series of the singly scattered radiance in `radiance` by its closed form for the geometries of one
+    mode-0 batch (sos_single_scatter_correction).  The subtracted series is made of the vectors the radiance was summed with:
+    mode 0 the batch's own P0 table row, modes m >= 1 the mode members' (the host-built _PHASES entries, exact zeros for a
+    vanishing mode); an isotropic phase function has no correction."""
+    M, mu = bs.M, bs.mu
+    ents, vecs, vec_row, tabs, tab_off = [], [], {}, [], {}
+    n_tab = 0
+    for s, sc in enumerate(bs.scenarios):
+        e = np.zeros((), dtype=_lib.SS_ENTRY_DTYPE)
+        e["scenario"], e["geo"], e["w"] = s, geo[s], bs.P0w[s]
+        for j, spec in enumerate((sc.atm_phase, sc.aer_phase)):
+            name, g = PH.resolve(spec[0], spec[1] if len(spec) > 1 else None)
+            if name == "iso":
+                e["family"][j] = -1
+                continue
+            e["family"][j] = PH.FAMILY_CODE[name]
+            key = (name, tuple(g) if isinstance(g, (tuple, list)) else float(g), float(sc.mu0))
+            if key not in vec_row:
+                v = np.empty((K, bs.N))
+                v[0] = bs.P0tab[bs.P0idx[s, j]]
+                for m in range(1, K):
+                    v[m] = 0.0 if PH.mode_vanishes(name, m) else _PHASES.get(_mode_spec(spec, m, n_quad), M, mu, sc.mu0, need_P=False)[0]
+                vec_row[key] = (len(vecs), PH.exact_norm(name, mu, sc.mu0, g, n_quad))
+                vecs.append(v)
+            e["series"][j], e["norm"][j] = vec_row[key]
+            if name in PH.TABULATED:
+                if key[:2] not in tab_off:
+                    xs, ys = PH.phase_table(name, g)
+                    tab_off[key[:2]] = (n_tab, len(xs))
+                    tabs += [np.asarray(xs, dtype=np.float64), np.asarray(ys, dtype=np.float64)]
+                    n_tab += 2 * len(xs)
+                e["tab_off"][j], e["tab_n"][j] = tab_off[key[:2]]
+            else:
+                e["g"][j] = float(g)
+        if not np.all(e["family"] < 0):
+            ents.append(e)
+    if not ents:
+        return   # isotropic media: the series is exact
+    eng.single_scatter_correction(radiance, np.array(ents, dtype=_lib.SS_ENTRY_DTYPE), np.stack(vecs),
+                                  np.concatenate(tabs) if tabs else np.zeros(0), rws, phi)

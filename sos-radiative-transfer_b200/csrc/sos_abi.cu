@@ -19,6 +19,7 @@
 #include "layer_shard.cuh"
 #include "phase.cuh"
 #include "quadrature.cuh"
+#include "single_scatter.cuh"
 #include "sweep.cuh"
 
 namespace {
@@ -1321,6 +1322,68 @@ int sos_glint_correction(sos_plan* p, int n, const int* geo_h, const double* par
   sosquad::glint_correction_kernel<<<static_cast<unsigned>((n_el + 127) / 128), 128, 0, st>>>(p->dev.mu, M, N, t, n, n_modes,
                                                                                            n_rows, n_az, out_d);
   const int r = launch_check(p, "glint_correction_kernel");
+  SOS_CUDA(cudaFreeAsync(buf, st));
+  return r;
+}
+
+int sos_single_scatter_correction(sos_plan* p, int n, const sos_ss_entry* ent_h, const double* P0m_h, int n_vec, int n_modes,
+                                  const double* tab_h, int n_tab, const int* rows_h, int n_rows, const double* phi_h, int n_az,
+                                  int n_geo, double* out_d, void* stream) {
+  if (!p || !ent_h || !P0m_h || !rows_h || !phi_h || !out_d || n < 1 || n_vec < 1 || n_rows < 1 || n_az < 1 || n_geo < 1 ||
+      n_tab < 0 || (n_tab > 0 && !tab_h))
+    return SOS_ERR_INVALID;
+  SOS_GUARD(p);
+  const GridDev& g = p->dev;
+  if (g.nreg != 3) return SOS_ERR_UNSUPPORTED;
+  if (n_modes < 1 || n_modes > sosphase::MAX_MODES) return SOS_ERR_INVALID;
+  for (int r = 0; r < n_rows; ++r)
+    if (rows_h[r] < 0 || rows_h[r] >= g.L) return SOS_ERR_INVALID;
+  for (int k = 0; k < n; ++k) {
+    const sos_ss_entry& e = ent_h[k];
+    if (e.scenario < 0 || e.scenario >= g.S || e.geo < 0 || e.geo >= n_geo) return SOS_ERR_INVALID;
+    for (int j = 0; j < 4; ++j)
+      if (!std::isfinite(e.w[j])) return SOS_ERR_INVALID;
+    for (int j = 0; j < 2; ++j) {
+      if (e.family[j] < -1 || e.family[j] > 2) return SOS_ERR_INVALID;
+      if (e.family[j] < 0) continue;
+      if (e.series[j] < 0 || e.series[j] >= n_vec || !(e.norm[j] > 0.0 && std::isfinite(e.norm[j])) || !std::isfinite(e.g[j]))
+        return SOS_ERR_INVALID;
+      if (e.family[j] == 2 && (e.tab_n[j] < 2 || e.tab_off[j] < 0 || static_cast<long long>(e.tab_off[j]) + 2LL * e.tab_n[j] > n_tab))
+        return SOS_ERR_INVALID;
+    }
+  }
+  static_assert(sizeof(sos_ss_entry) == sizeof(sosss::Entry), "sos_ss_entry and sosss::Entry must match");
+  // one table: P0m [n_vec][K][N] | tab [n_tab] | wcos [n_az][K] | cos(phi) [n_az] | entries | rows (int)
+  const int N = g.N;
+  const size_t n_p0 = static_cast<size_t>(n_vec) * n_modes * N, n_w = static_cast<size_t>(n_az) * n_modes;
+  std::vector<double> tab(n_p0 + n_tab + n_w + n_az);
+  std::copy(P0m_h, P0m_h + n_p0, tab.begin());
+  if (n_tab) std::copy(tab_h, tab_h + n_tab, tab.begin() + n_p0);
+  double* w = tab.data() + n_p0 + n_tab;
+  double* cphi = w + n_w;
+  for (int q = 0; q < n_az; ++q) {
+    cphi[q] = std::cos(phi_h[q]);
+    for (int m = 0; m < n_modes; ++m) w[static_cast<size_t>(q) * n_modes + m] = m == 0 ? 1.0 : 2.0 * std::cos(m * phi_h[q]);
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  char* buf = nullptr;
+  const size_t dbytes = tab.size() * sizeof(double), ebytes = static_cast<size_t>(n) * sizeof(sos_ss_entry);
+  SOS_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&buf), dbytes + ebytes + n_rows * sizeof(int), st));
+  SOS_CUDA(cudaMemcpyAsync(buf, tab.data(), dbytes, cudaMemcpyHostToDevice, st));
+  SOS_CUDA(cudaMemcpyAsync(buf + dbytes, ent_h, ebytes, cudaMemcpyHostToDevice, st));
+  SOS_CUDA(cudaMemcpyAsync(buf + dbytes + ebytes, rows_h, n_rows * sizeof(int), cudaMemcpyHostToDevice, st));
+  const double* d = reinterpret_cast<const double*>(buf);
+  sosss::Tables t;
+  t.P0m = d;
+  t.tab = d + n_p0;
+  t.wcos = t.tab + n_tab;
+  t.cphi = t.wcos + n_w;
+  t.ent = reinterpret_cast<const sosss::Entry*>(buf + dbytes);
+  t.rows = reinterpret_cast<const int*>(buf + dbytes + ebytes);
+  const long long n_el = static_cast<long long>(n) * n_az * N;
+  sosss::single_scatter_kernel<<<static_cast<unsigned>((n_el + sosss::THREADS - 1) / sosss::THREADS), sosss::THREADS, 0, st>>>(
+      g, t, n, n_modes, n_rows, n_az, out_d);
+  const int r = launch_check(p, "single_scatter_kernel");
   SOS_CUDA(cudaFreeAsync(buf, st));
   return r;
 }

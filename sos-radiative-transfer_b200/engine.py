@@ -510,6 +510,30 @@ class SosEngine:
             torch.cuda.current_stream(self.device).synchronize()   # (the host tables are temporaries)
         return out
 
+    def single_scatter_correction(self, out: torch.Tensor, entries: np.ndarray, P0m: np.ndarray, tables: np.ndarray,
+                                  rows: Sequence[int], phi: np.ndarray):
+        """Exact single scattering of azimuth-resolved radiance (sos_single_scatter_correction): out (n_geo, n_rows, n_az, N) as
+        written by azimuth_synthesis at the layers `rows`; entries: _lib.SS_ENTRY_DTYPE records (plan scenario, geometry,
+        phase families, rows of P0m, table offsets, g, normalisations T, weights (alb_atm, f_atm, alb_aer, f_aer)); P0m
+        (n_vec, n_modes, N) the solar mode vectors the radiance was summed with; tables the tabulated phase functions
+        (abscissae then values at each entry's offset); phi (n_az,)."""
+        ent = np.ascontiguousarray(entries)
+        p0 = np.ascontiguousarray(P0m, dtype=np.float64)
+        tab = np.ascontiguousarray(tables, dtype=np.float64).reshape(-1)
+        rw = np.ascontiguousarray(rows, dtype=np.int32)
+        ph = np.ascontiguousarray(phi, dtype=np.float64)
+        n_geo, n_rows, n_az = out.shape[:3]
+        if (ent.dtype != _lib.SS_ENTRY_DTYPE or ent.ndim != 1 or p0.ndim != 3 or p0.shape[2] != self.N or rw.shape != (n_rows,)
+                or ph.shape != (n_az,) or out.shape[3] != self.N or out.dtype != torch.float64 or not out.is_contiguous()):
+            raise ValueError("single_scatter_correction: shapes do not match the plan")
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.sos_single_scatter_correction(self._plan, int(ent.size), ent.ctypes.data, p0.ctypes.data, p0.shape[0],
+                                                              p0.shape[1], tab.ctypes.data if tab.size else None, int(tab.size),
+                                                              rw.ctypes.data, n_rows, ph.ctypes.data, n_az, n_geo, out.data_ptr(),
+                                                              self._stream), "sos_single_scatter_correction")
+            torch.cuda.current_stream(self.device).synchronize()   # (the host tables are temporaries)
+        return out
+
     def azimuth_synthesis(self, I: torch.Tensor, geo: np.ndarray, weights: np.ndarray, n_geo: int, rows: Sequence[int],
                           out: torch.Tensor, accumulate: bool):
         """out[geo][r][p][:] (+)= sum over the members s of geo (ascending) of weights[s, p] * I[s, rows[r], :N]

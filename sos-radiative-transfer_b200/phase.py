@@ -156,6 +156,34 @@ def _mode_rings(f, cc, x, cm, phi):
     return np.stack(out)
 
 
+FAMILY_CODE = {"rayleigh": 0, "hg": 1, "fwc": 2, "mie_lognormal": 2}   # the device's phase families (csrc/phase.cuh)
+
+
+def exact_norm(name: str, mu: np.ndarray, mu0: float, g=0.5, n_quad: int = 25) -> float:
+    """T = trapz_mu(ring_0 / 4 pi): the mode-0 normalisation phase_modes divides the solar modes by at n_quad azimuth nodes
+    (at n_quad = 25 that of phase_P0), so that sum_m (2 - delta_m0) P0_m cos(m phi) -> p(cos Theta) / T as K -> infinity."""
+    name, g = resolve(name, g)
+    f = _kernel(name, g)
+    mu = np.asarray(mu, dtype=np.float64)
+    phi = np.linspace(0, np.pi, int(n_quad))
+    cc = (mu * mu0)[:, None]
+    x = (np.sqrt(1 - mu0 * mu0) * np.sqrt(1 - mu * mu))[:, None] * np.cos(0 - phi)[None, :]
+    return float(_trapz(_trapz(f(-(cc + x)) + f(-(cc - x)), phi) / (4 * np.pi), mu))
+
+
+def phase_exact(name: str, nb_angles: int, mu: np.ndarray, mu0: float, phi, g=0.5, n_quad: int = 25) -> np.ndarray:
+    """The solar phase vector at the azimuths phi, (n_phi, N): p(cos Theta(mu, mu0, phi)) / T with cos Theta = -mu0 mu +
+    sqrt(1 - mu0^2) sqrt(1 - mu^2) cos phi (the convention of phase_modes) and T = exact_norm(..., n_quad): the value the
+    series sum_m (2 - delta_m0) P0_m cos(m phi) of phase_modes(..., n_quad) converges to.  Isotropic: ones."""
+    name, g = resolve(name, g)
+    mu = np.asarray(mu, dtype=np.float64)
+    phi = np.atleast_1d(np.asarray(phi, dtype=np.float64))
+    if name == "iso":
+        return np.ones((phi.size, 2 * nb_angles))
+    c = -mu0 * mu[None, :] + np.sqrt(1 - mu0 * mu0) * np.sqrt(1 - mu * mu)[None, :] * np.cos(phi)[:, None]
+    return _kernel(name, g)(c) / exact_norm(name, mu, mu0, g, n_quad)
+
+
 def phase_modes(name: str, nb_angles: int, mu: np.ndarray, n_modes: int, g: float = 0.5, mu0=None, n_quad: int = 25,
                 want_P: bool = True):
     """Azimuthal Fourier modes m = 0 .. n_modes-1 of a phase function: (P0_m (K, N) or None without mu0, P_m (K, N, N) or
